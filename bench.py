@@ -2,7 +2,7 @@
 """bench.py -- learner transitions/sec (GAE + all PPO epochs) on synthetic stompy_pro-shaped
 trajectories (BASELINE.json metric; SURVEY.md section 8d).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is ONE learner update of the hot path (/root/reference/minppo/train.py:185-281): GAE
 over the [T x N] trajectory, E epochs x M minibatches of shuffle/gather + ActorCritic
@@ -146,7 +146,9 @@ def init_param_tree(hidden: int, num_layers: int, seed: int = 0, dims=None):
 
 def synth_shard(hp, rank: int, world: int, seed: int = 0, dims=None):
     """Synthetic shard [T, N/world, ...] in float32 NumPy.  Params from the init gains; value / log_prob
-    from a forward pass under those params (float32 torch CPU for speed); reward ~ N(0,1); done ~ B(0.01).
+    from a forward pass under those params; reward ~ N(0,1); done ~ B(0.01).  The same arguments give the same
+    bits in every run: the forward pass runs on one CPU thread (BLAS sums in an order that depends on how it splits
+    the work over threads, and it may choose that split anew in each run) and in float64, rounded once to float32.
     Input generation only: nothing here touches oracle/ or the product."""
     import torch
 
@@ -155,29 +157,55 @@ def synth_shard(hp, rank: int, world: int, seed: int = 0, dims=None):
     params = init_param_tree(hp.hidden_size, hp.num_layers, seed, dims=(obs_dim, act_dim))
     g = torch.Generator().manual_seed(1234 + rank)
     obs = torch.randn(T * Nl, obs_dim, generator=g)
-    pt = tree_map(params, lambda x: torch.from_numpy(x))["params"]
+    pt = tree_map(params, lambda x: torch.from_numpy(x).double())["params"]
 
     def mlp(m, x, tanh):
         for i in range(hp.num_layers):
-            x = x @ m[f"Dense_{i}"]["kernel"] + m[f"Dense_{i}"]["bias"]
-            x = torch.tanh(x) if tanh else torch.relu(x)
-        return x @ m[f"Dense_{hp.num_layers}"]["kernel"] + m[f"Dense_{hp.num_layers}"]["bias"]
+            x = torch.addmm(m[f"Dense_{i}"]["bias"], x, m[f"Dense_{i}"]["kernel"])
+            x = x.tanh_() if tanh else x.relu_()
+        return torch.addmm(m[f"Dense_{hp.num_layers}"]["bias"], x, m[f"Dense_{hp.num_layers}"]["kernel"])
 
-    with torch.no_grad():
-        mean = mlp(pt["MLP_0"], obs, hp.use_tanh)
-        value = mlp(pt["MLP_1"], obs, False)[:, 0]
-        scale = torch.exp(pt["log_std"])
-        action = mean + scale * torch.randn(mean.shape, generator=g)
-        z = (action - mean) / scale
-        log_prob = (-0.5 * z * z - 0.5 * np.log(2 * np.pi)).sum(-1) - torch.log(scale).sum()
-        last_val = mlp(pt["MLP_1"], torch.randn(Nl, obs_dim, generator=g), False)[:, 0]
+    threads = torch.get_num_threads()
+    torch.set_num_threads(1)
+    try:
+        with torch.no_grad():
+            obs64 = obs.double()
+            mean = mlp(pt["MLP_0"], obs64, hp.use_tanh)
+            value = mlp(pt["MLP_1"], obs64, False)[:, 0]
+            del obs64
+            scale = torch.exp(pt["log_std"])
+            action = mean + scale * torch.randn(mean.shape, generator=g).double()
+            z = (action - mean) / scale
+            log_prob = (-0.5 * z * z - 0.5 * np.log(2 * np.pi)).sum(-1) - torch.log(scale).sum()
+            last_val = mlp(pt["MLP_1"], torch.randn(Nl, obs_dim, generator=g).double(), False)[:, 0]
+    finally:
+        torch.set_num_threads(threads)
     traj = {
-        "obs": obs.reshape(T, Nl, obs_dim).numpy(), "action": action.reshape(T, Nl, act_dim).numpy(),
-        "value": value.reshape(T, Nl).numpy(), "log_prob": log_prob.reshape(T, Nl).numpy(),
+        "obs": obs.reshape(T, Nl, obs_dim).numpy(), "action": action.float().reshape(T, Nl, act_dim).numpy(),
+        "value": value.float().reshape(T, Nl).numpy(), "log_prob": log_prob.float().reshape(T, Nl).numpy(),
         "reward": torch.randn(T, Nl, generator=g).numpy(),
         "done": (torch.rand(T, Nl, generator=g) < 0.01).numpy(),
     }
-    return params, traj, last_val.numpy()
+    return params, traj, last_val.float().numpy()
+
+
+DUMP_LIMIT_BYTES = 63 << 20          # array data: with the .npy headers, a dump stays under 64 MB
+
+
+def dump_outputs(out_dir: str, arrays) -> None:
+    """Write each array as <out_dir>/<name>.npy: floating point as float32, integers as float64 (exact for 32-bit words).
+    If together they exceed DUMP_LIMIT_BYTES, each array larger than an equal share of the limit is replaced by the same
+    seeded sample of its flattened elements in every run, so that two builds can still be compared element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, np.float64 if np.issubdtype(np.asarray(v).dtype, np.integer) else np.float32)
+              for k, v in arrays.items()}
+    share = DUMP_LIMIT_BYTES // len(arrays)
+    over = sum(a.nbytes for a in arrays.values()) > DUMP_LIMIT_BYTES
+    for name, a in arrays.items():
+        if over and a.nbytes > share:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------
@@ -466,6 +494,11 @@ def run_ours(args):
     ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop() if sampler else None
     learner.check()
+    if args.dump_outputs and rank == 0:
+        # what Learner.update hands its caller after the last timed step (rank 0's copy when sharded)
+        dump_outputs(args.dump_outputs, {"params": ts.params.cpu().numpy(), "mu": ts.mu.cpu().numpy(),
+                                         "nu": ts.nu.cpu().numpy(), "step": ts.step.cpu().numpy(),
+                                         "rng_out": rng_out.cpu().numpy().view(np.uint32), "losses": losses.cpu().numpy()})
     tt = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -797,7 +830,15 @@ def main():
     ap.add_argument("--workload", default="auto", choices=["auto", "c4"],
                     help="auto: configs[1] per GPU (weak scaling); c4: configs[3] global batch (strong scaling)")
     ap.add_argument("--quick", action="store_true", help="device-resident timing only (development)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (params, mu, nu, step, rng_out, "
+                         "losses) as DIR/<name>.npy, under 64 MB in all (a seeded sample of larger outputs); "
+                         "--impl ours only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference(args)
     elif args.impl == "torch_gpu":

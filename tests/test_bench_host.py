@@ -3,8 +3,10 @@ synthetic parameter generator (which must stay the oracle's recipe so that the C
 problem).  bench.py's product arm must not import oracle/ (the oracle is the checker, never the thing measured)."""
 import ast
 import os
+import sys
 
 import numpy as np
+import pytest
 
 import bench
 from minppo_b200.config import to_c_config
@@ -43,6 +45,54 @@ def test_synthetic_parameters_are_the_oracles_recipe():
     b = P.flatten_params(P.init_params(bench.OBS_DIM, bench.ACT_DIM, 256, 2, 0, np.float32), 2)
     assert a.size == param_count(bench.OBS_DIM, bench.ACT_DIM, 256, 2) == 250133          # SURVEY.md 8a row 4
     assert np.array_equal(a, b)
+
+
+def test_synthetic_inputs_do_not_depend_on_the_thread_count():
+    """The benchmark's inputs are the same bits in every run, so that outputs of two builds can be compared exactly."""
+    import torch
+
+    hp = bench.BenchShape(num_envs=64, num_steps=16, num_minibatches=4, update_epochs=1)
+    threads = torch.get_num_threads()
+    shards = []
+    try:
+        for t in (1, 3):
+            torch.set_num_threads(t)
+            shards.append(bench.synth_shard(hp, 0, 1))
+            assert torch.get_num_threads() == t
+    finally:
+        torch.set_num_threads(threads)
+    (_, a, lva), (_, b, lvb) = shards
+    assert np.array_equal(lva, lvb) and lva.dtype == np.float32
+    for k in a:
+        assert np.array_equal(a[k], b[k]), k
+
+
+def test_dump_outputs_types_and_size_limit(tmp_path, monkeypatch):
+    """float32 / float64 files named after the outputs; over the limit, a large array becomes the same seeded sample of
+    its elements in every run, and the files stay within the limit."""
+    params = np.arange(1000, dtype=np.float32) / 7
+    arrays = {"params": params, "step": np.array([128], np.int32), "rng_out": np.array([0xFFFFFFFF, 7], np.uint32)}
+    bench.dump_outputs(str(tmp_path / "a"), arrays)
+    got = {k: np.load(tmp_path / "a" / f"{k}.npy") for k in arrays}
+    assert got["params"].dtype == np.float32 and np.array_equal(got["params"], params)
+    assert got["step"].dtype == np.float64 and got["step"].tolist() == [128.0]
+    assert got["rng_out"].dtype == np.float64 and got["rng_out"].tolist() == [4294967295.0, 7.0]
+
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 1200)
+    bench.dump_outputs(str(tmp_path / "b"), arrays)
+    bench.dump_outputs(str(tmp_path / "c"), arrays)
+    b, c = (np.load(tmp_path / d / "params.npy") for d in "bc")
+    assert np.array_equal(b, c) and b.size == 1200 // 3 // 4 and np.isin(b, params).all()
+    assert sum(os.path.getsize(tmp_path / "b" / f"{k}.npy") - 128 for k in arrays) <= 1200       # 128-byte .npy header
+    assert np.load(tmp_path / "b" / "step.npy").tolist() == [128.0]
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bench_rejects_bad_arguments(argv, monkeypatch):
+    monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
+    with pytest.raises(SystemExit) as e:
+        bench.main()
+    assert e.value.code == 2
 
 
 def test_product_arm_does_not_import_the_oracle():
