@@ -55,7 +55,7 @@ typedef struct minppo_config {
   int32_t update_epochs;     /* training.update_epochs -- E                           */
   int64_t total_timesteps;   /* training.total_timesteps (LR schedule, train.py:93)   */
   int32_t anneal_lr;         /* training.anneal_lr                                    */
-  int32_t hidden_size;       /* model.hidden_size  (multiple of 64, <= 256)           */
+  int32_t hidden_size;       /* model.hidden_size  (multiple of 64, <= 512; > 256: num_layers <= 2) */
   int32_t num_layers;        /* model.num_layers   (>= 1)                             */
   int32_t use_tanh;          /* model.use_tanh     (actor only; critic is relu, train.py:82) */
   int32_t obs_dim;           /* D                                                     */
@@ -65,7 +65,8 @@ typedef struct minppo_config {
   int32_t rank;              /* this rank owns envs [rank*N/G, (rank+1)*N/G)          */
   int32_t fast_tanh;         /* 1: tanh.approx.f32 (MUFU) in the GEMM epilogue        */
   int32_t dw_splits;         /* split-K factor of the weight-gradient GEMMs (0 = auto) */
-  int32_t disable_fused;     /* 1: always use the layer-wise kernels (default 0: fused step kernel when L == 2) */
+  int32_t disable_fused;     /* 1: always use the layer-wise kernels (default 0: fused step kernel when L == 2 and
+                                hidden_size <= 256; wider layers always run layer-wise) */
   double training_lr;        /* training.lr  (annealed path, train.py:101)            */
   double opt_lr;             /* opt.lr       (constant path, train.py:123)            */
   double max_grad_norm;      /* opt.max_grad_norm                                     */

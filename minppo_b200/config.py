@@ -60,7 +60,8 @@ class LearnerExtras:
                                          # activation); False = 1 - 2/(1+exp(2x)) through ex2/rcp (abs. err ~1e-7)
     use_graph: bool = True               # replay one CUDA graph per update
     dw_splits: int = 0                   # 0 = auto
-    fused: bool = True                   # fused forward+loss+backward kernel (2 hidden layers); False = layer-wise kernels
+    fused: bool = True                   # fused forward+loss+backward kernel when num_layers == 2 and hidden_size <= 256
+                                         # (wider layers always run layer-wise); False = layer-wise kernels
 
 
 @dataclass

@@ -218,9 +218,11 @@ size_t head_loss_smem_bytes(int H, int amax) {
 }
 
 int head_loss_init() {
-  cudaError_t e = cudaFuncSetAttribute(head_loss_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(head_loss_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(head_loss_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  // H = 512 with the 32-wide template: 212,416 bytes (above 200 KB, below the 227 KB a block may opt in to)
+  const int smax = static_cast<int>(head_loss_smem_bytes(MAX_HIDDEN, 32));
+  cudaError_t e = cudaFuncSetAttribute(head_loss_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(head_loss_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(head_loss_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
   return e == cudaSuccess ? 0 : MINPPO_ERR_CUDA;
 }
 

@@ -176,8 +176,14 @@ static int validate_config(const minppo_config& c) {
     set_error("non-positive size in minppo_config");
     return MINPPO_ERR_ARG;
   }
-  if (c.hidden_size % 64 != 0 || c.hidden_size > 256 || c.hidden_size <= 0) {
-    set_error("model.hidden_size=%d unsupported: must be a multiple of 64 and <= 256", c.hidden_size);
+  if (c.hidden_size % 64 != 0 || c.hidden_size > MAX_HIDDEN || c.hidden_size <= 0) {
+    set_error("model.hidden_size=%d unsupported: must be a multiple of 64 and <= %d", c.hidden_size, MAX_HIDDEN);
+    return MINPPO_ERR_UNSUPPORTED;
+  }
+  // wider than one GEMM tile: every hidden layer of both nets is two column groups of the weight-gradient launch
+  if (c.hidden_size > GEMM_MAXN && 2 * c.num_layers * 2 > GEMM_MAX_GROUPS) {
+    set_error("num_layers=%d unsupported at model.hidden_size=%d: hidden_size > %d allows num_layers <= %d", c.num_layers,
+              c.hidden_size, GEMM_MAXN, GEMM_MAX_GROUPS / 4);
     return MINPPO_ERR_UNSUPPORTED;
   }
   if (c.act_dim > 32) { set_error("act_dim=%d unsupported (<= 32)", c.act_dim); return MINPPO_ERR_UNSUPPORTED; }
@@ -220,7 +226,8 @@ struct NetBufs {
   std::vector<CUtensorMap> m_act_k, m_act_mn, m_dz_k, m_dz_mn, m_wn_mn, m_wn, m_dw;
   std::vector<CUtensorMap> m_wn_h;     // m_wn_h[l]: box {64 out, 32 in} -- half-k-block stages of the fused step kernel (MN-major B)
   CUtensorMap m_w1k_h;                 // wn[1]: box {64 out, H/2 in} -- (k-block, N half) stages of the fused kernel's dH1 GEMM (K-major B)
-  // m_wn_mn[l]: box {64 out, 64 in} -- MN-major B of the forward GEMMs;  m_wn[l] (l >= 1): box {64 out, H in} -- K-major B of dX
+  // m_wn_mn[l]: box {64 out, 64 in} -- MN-major B of the forward GEMMs;  m_wn[2 l + j] (l >= 1): box {64 out, N_j in} -- K-major
+  // B of dX for column group j (col_group)
 };
 
 struct UpdatePtrs {
@@ -241,8 +248,10 @@ struct minppo_ctx {
   int T, N, Nl, n0, M, E, L, H, D, Dp, A;
   long long B, Bl, P;
   int mb, cap, M_pad, m_tiles, tiles64, S;
-  int dw_nsplit;              // dW GEMM groups per (net, layer): 1 (128 x H tiles) or 2 (N halves: 128 x H/2 tiles, half the
-                              // split-K factor -- half the partial bytes stored and re-read per step; needs H % 128 == 0)
+  int dw_nsplit;              // dW GEMM groups per (net, layer): 1 (128 x H tiles) or 2 (column groups of col_group: half the
+                              // split-K factor -- half the partial bytes stored and re-read per step; H % 128 == 0 on the
+                              // fused path, always when H > GEMM_MAXN)
+  int hsplit;                 // column groups of the forward, dX and policy GEMMs: 1, or 2 when H > GEMM_MAXN (col_group)
   int maxu;                   // dwopt fast path: 4-element units of the hidden kernels per thread (1, 2 or 4)
   bool fused;                 // fused step kernel (L == 2; any obs_dim, act_dim <= 32, hidden_size <= 256)
   int head_parts;             // head partials per minibatch: m_tiles (fused) or tiles64
@@ -351,6 +360,14 @@ static const LeafInfo& find_leaf(const minppo_ctx* c, int net, int layer, int is
   for (const auto& l : c->leaves)
     if (l.net == net && l.layer == layer && l.is_kernel == is_kernel) return l;
   return c->leaves[0];
+}
+
+// Column range j of a hidden layer split into n groups: n == 1 is the whole of H; n == 2 puts H / 2 rounded up to a whole
+// 64-column panel first (512 -> 256 + 256, 448 -> 256 + 192, 320 -> 192 + 128): both widths are multiples of 64 and <= 256.
+static void col_group(int H, int n, int j, int* n_off, int* N) {
+  const int first = n == 1 ? H : (H / 2 + 63) / 64 * 64;
+  *n_off = j == 0 ? 0 : first;
+  *N = j == 0 ? first : H - first;
 }
 
 static int act_kind(const minppo_ctx* c, int net) {
@@ -505,7 +522,8 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
       g.k_count = nullptr;                                    // per step (counts[] below)
       g.tmC = nb.m_dw[l];
       g.colsum_out = c->fused ? nullptr : nb.dbias[l];      // fused path: the bias gradients come from the fused step kernel
-      g.N = H / c->dw_nsplit; g.n_off = nh * g.N;
+      col_group(H, c->dw_nsplit, nh, &g.n_off, &g.N);
+      g.ldc = H;
       g.m_tiles = (in_pad + 127) / 128; g.splits = c->S; g.m_store = in_l;
       cta += g.m_tiles * g.splits;
       }
@@ -549,11 +567,13 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
   for (int l = 0; l < L; ++l) {
     GemmParams p;
     memset(&p, 0, sizeof(p));
-    p.ngroups = 2;
-    for (int net = 0; net < 2; ++net) {
-      GemmGroup& g = p.g[net];
+    p.ngroups = 2 * c->hsplit;
+    for (int i = 0; i < p.ngroups; ++i) {
+      const int net = i / c->hsplit;
+      GemmGroup& g = p.g[i];
       NetBufs& nb = c->net[net];
-      g.cta_begin = net * c->m_tiles;
+      g.cta_begin = i * c->m_tiles;
+      col_group(H, c->hsplit, i % c->hsplit, &g.n_off, &g.N);
       g.bmode = B_TMA_MN;                 // kernel image as stored [in = k][out = n]
       g.tmB = nb.m_wn_mn[l];
       if (l == 0) {
@@ -564,10 +584,10 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
       g.out = nb.act[l + 1]; g.ldo = H;
       g.bias = u.params + find_leaf(c, net, l, 0).offset;
       g.act = act_kind(c, net);
-      g.N = H; g.m_tiles = c->m_tiles; g.splits = 1; g.m_store = c->M_pad;
+      g.m_tiles = c->m_tiles; g.splits = 1; g.m_store = c->M_pad;
     }
     PROF(PC_FWD_GEMM);
-    RET(launch_gemm<EPI_ACT>(p, 2 * c->m_tiles, stream));
+    RET(launch_gemm<EPI_ACT>(p, p.ngroups * c->m_tiles, stream));
     c->launches++;
   }
   // heads + loss + dz[L]
@@ -597,22 +617,24 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
   for (int l = L - 1; l >= 1; --l) {
     GemmParams p;
     memset(&p, 0, sizeof(p));
-    p.ngroups = 2;
-    for (int net = 0; net < 2; ++net) {
-      GemmGroup& g = p.g[net];
+    p.ngroups = 2 * c->hsplit;
+    for (int i = 0; i < p.ngroups; ++i) {
+      const int net = i / c->hsplit, j = i % c->hsplit;
+      GemmGroup& g = p.g[i];
       NetBufs& nb = c->net[net];
-      g.cta_begin = net * c->m_tiles;
+      g.cta_begin = i * c->m_tiles;
+      col_group(H, c->hsplit, j, &g.n_off, &g.N);
       g.amode = A_TMA_K; g.tmA = nb.m_dz_k[l + 1];
-      g.bmode = B_TMA_K; g.tmB = nb.m_wn[l];
+      g.bmode = B_TMA_K; g.tmB = nb.m_wn[2 * l + j];
       g.kb_total = H / 64;
       g.out = nb.dz[l]; g.ldo = H;
       g.hprev = nb.act[l]; g.ldh = H;
-      g.colsum = nb.colsum[l];
+      g.colsum = nb.colsum[l]; g.ldc = H;
       g.act = act_kind(c, net);
-      g.N = H; g.m_tiles = c->m_tiles; g.splits = 1; g.m_store = c->M_pad;
+      g.m_tiles = c->m_tiles; g.splits = 1; g.m_store = c->M_pad;
     }
     PROF(PC_BWD_GEMM);
-    RET(launch_gemm<EPI_DACT>(p, 2 * c->m_tiles, stream));
+    RET(launch_gemm<EPI_DACT>(p, p.ngroups * c->m_tiles, stream));
     c->launches++;
   }
   }  // !fused
@@ -915,7 +937,8 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   c->cap = c->M_pad;                                  // row lists are padded to whole GEMM tiles
   c->m_tiles = c->M_pad / 128;
   c->tiles64 = c->M_pad / 64;
-  c->fused = !cfg->disable_fused && c->L == 2;
+  c->fused = !cfg->disable_fused && c->L == 2 && c->H <= GEMM_MAXN;
+  c->hsplit = c->H > GEMM_MAXN ? 2 : 1;
   c->ap = c->A <= 16 ? 16 : 32;
   c->store_x = c->fused;        // the fused kernel's critic CTAs store the gathered X tile (any Dp: block by block from the slots)
   c->head_parts = c->fused ? c->m_tiles : c->tiles64;
@@ -924,8 +947,12 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   // split-K of the dW GEMMs: fill the SMs once
   {
     // N-halved dW tiles (fused path, H a multiple of 128): half the split-K factor for the same number of GEMM CTAs
-    // (only with TMA-fed A operands: groups that gather their rows by index would gather every row twice)
-    c->dw_nsplit = (c->fused && c->store_x && c->H % 128 == 0 && 2 * 2 * c->L <= GEMM_MAX_GROUPS &&
+    // (only with TMA-fed A operands: groups that gather their rows by index would gather every row twice).
+    // H > GEMM_MAXN needs the two column groups of col_group whatever the path; there the first layer's groups gather
+    // their observation rows by index (A_GATHER_MN), so every row is gathered once per column group: twice the
+    // observation-image reads of that layer's A operand.
+    c->dw_nsplit = c->H > GEMM_MAXN ? 2
+                 : (c->fused && c->store_x && c->H % 128 == 0 && 2 * 2 * c->L <= GEMM_MAX_GROUPS &&
                     !(getenv("MINPPO_DW_NSPLIT") && atoi(getenv("MINPPO_DW_NSPLIT")) == 1)) ? 2 : 1;
     int per_split = 0;
     for (int l = 0; l < c->L; ++l) per_split += 2 * c->dw_nsplit * (((l == 0 ? c->Dp : c->H) + 127) / 128);
@@ -1023,7 +1050,7 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
     nb.dw_part.assign(L, nullptr); nb.colsum.assign(L, nullptr); nb.dbias.assign(L, nullptr);
     ALLOC(nb.w2img, static_cast<size_t>(H) * FS_MAX_AP * 4);       // H/64 panels of [2 AP rows][128 B]
     nb.m_act_k.resize(L + 1); nb.m_act_mn.resize(L + 1); nb.m_dz_k.resize(L + 1); nb.m_dz_mn.resize(L + 1);
-    nb.m_wn_mn.resize(L); nb.m_wn.resize(L); nb.m_dw.resize(L); nb.m_wn_h.resize(L);
+    nb.m_wn_mn.resize(L); nb.m_wn.resize(2 * L); nb.m_dw.resize(L); nb.m_wn_h.resize(L);
     for (int l = 1; l <= L; ++l) {
       ALLOC(nb.act[l], static_cast<size_t>(c->M_pad) * H);
       ALLOC(nb.dz[l], static_cast<size_t>(c->M_pad) * H);
@@ -1040,7 +1067,11 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
       if ((rc = make_tmap(&nb.m_wn_h[l], nb.wn[l], H, kp, H, 64, 32))) return fail(rc);
       if (l == 1 && (rc = make_tmap(&nb.m_w1k_h, nb.wn[l], H, H, H, 64, H / 2))) return fail(rc);
       if (l >= 1) {
-        if ((rc = make_tmap(&nb.m_wn[l], nb.wn[l], H, H, H, 64, H))) return fail(rc);
+        for (int j = 0; j < c->hsplit; ++j) {
+          int n_off, n;
+          col_group(H, c->hsplit, j, &n_off, &n);
+          if ((rc = make_tmap(&nb.m_wn[2 * l + j], nb.wn[l], H, H, H, 64, n))) return fail(rc);
+        }
         ALLOC(nb.colsum[l], static_cast<size_t>(c->m_tiles) * H);
       }
       ALLOC(nb.dw_part[l], static_cast<size_t>(c->S) * in_l * H);
@@ -1190,10 +1221,12 @@ int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, con
     GemmParams p;
     memset(&p, 0, sizeof(p));
     int ng = 0;
-    for (int net = first; net < 2; ++net) {
+    for (int i = first * c->hsplit; i < 2 * c->hsplit; ++i) {
+      const int net = i / c->hsplit;
       GemmGroup& g = p.g[ng];
       g.cta_begin = ng * c->pol_tiles;
       ++ng;
+      col_group(H, c->hsplit, i % c->hsplit, &g.n_off, &g.N);
       g.bmode = B_TMA_MN; g.tmB = c->net[net].m_wn_mn[l];
       g.amode = A_TMA_K;
       if (l == 0) { g.tmA = c->m_pol_img_k; g.kb_total = c->Dp / 64; }
@@ -1201,7 +1234,7 @@ int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, con
       g.out = c->pol_act[net][l + 1]; g.ldo = H;
       g.bias = params + find_leaf(c, net, l, 0).offset;
       g.act = act_kind(c, net);
-      g.N = H; g.m_tiles = c->pol_tiles; g.splits = 1; g.m_store = c->pol_tiles * 128;
+      g.m_tiles = c->pol_tiles; g.splits = 1; g.m_store = c->pol_tiles * 128;
     }
     p.ngroups = ng;
     RET(launch_gemm<EPI_ACT>(p, ng * c->pol_tiles, stream));

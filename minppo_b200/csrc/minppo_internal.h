@@ -12,6 +12,9 @@ namespace minppo {
 
 enum : int { ACTK_TANH = 0, ACTK_RELU = 1, ACTK_TANH_FAST = 2 };   // == ACT_* in umma_gemm.cuh
 
+// widest model.hidden_size: hidden layers wider than one 256-column GEMM tile run as two column groups
+constexpr int MAX_HIDDEN = 512;
+
 // ---- gae.cu ------------------------------------------------------------------------------
 void gae_plan(int T, long long N, int sm_count, int* vec, int* chunks, int* seg_len);
 int gae_launch(const float* reward, const float* value, const uint8_t* done, const float* last_val, float* adv,

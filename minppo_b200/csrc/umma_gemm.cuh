@@ -6,6 +6,8 @@
 //   warps 2..5  : optional row-gather producer for A (cp.async by index, software swizzle),
 //                 then the epilogue (tcgen05.ld -> registers -> fused math -> global)
 // Operands are staged in a 4-deep shared-memory ring (mbarrier full/empty pairs).
+// A layer wider than 256 columns runs as several groups of one launch, each on its own column range (GemmGroup::n_off,
+// widths multiples of 64 and <= 256); B_TMA_K groups then carry a tensor map whose box is their own width.
 //
 // Operand modes (what the learner's layers need, /root/reference/minppo/train.py:56-83, 246):
 //   A_TMA_K     A[m][k] row-major in HBM (activations)            -> K-major tile
@@ -47,8 +49,8 @@ struct alignas(64) GemmGroup {
   void* out;                       // EPI_ACT/EPI_DACT: bf16 [M][ldo]
   const float* bias;               // EPI_ACT: fp32 [N]
   const __nv_bfloat16* hprev;      // EPI_DACT: layer output h (for f'(z) from h), bf16 [M][ldh]
-  float* colsum;                   // EPI_DACT: fp32 [m_tiles][N] per-tile column sums (bias grads)
-  float* colsum_out;               // EPI_PARTIAL + B_TMA_MN: fp32 [splits][N] column sums of B over this CTA's K range
+  float* colsum;                   // EPI_DACT: fp32 [m_tiles][ldc] per-tile column sums (bias grads)
+  float* colsum_out;               // EPI_PARTIAL + B_TMA_MN: fp32 [splits][ldc] column sums of B over this CTA's K range
                                    // (= bias gradient partials), computed on the tensor core as ones x B; or null
   int ldg, ldo, ldh;
   int amode, bmode;                // A_* / B_* operand modes
@@ -59,9 +61,14 @@ struct alignas(64) GemmGroup {
   int splits;                      // split-K factor (EPI_PARTIAL)
   int kb_total;                    // number of 64-wide k-blocks over the whole K
   int m_store;                     // EPI_PARTIAL: rows m < m_store are stored
-  int n_off;                       // B_TMA_MN / EPI_PARTIAL: first column of this group's N range inside B and C (N-split groups)
+  int n_off;                       // first column of this group's N range inside B, C, bias, out, hprev and the column sums
+                                   // (N-split groups: a layer wider than GEMM_MAXN runs as several groups of <= 256 columns)
+  int ldc;                         // row stride of colsum / colsum_out in floats (the full width of an N-split layer); 0 = N
   const int32_t* k_count;          // optional: number of valid K rows (device side); k-blocks beyond it are skipped
 };
+
+// 512 bytes: GEMM_MAX_GROUPS of them sit in every GEMM / dwopt parameter block
+static_assert(sizeof(GemmGroup) == 512, "GemmGroup grew: the kernel parameter blocks grow with it");
 
 struct alignas(64) GemmParams {
   int ngroups;                     // groups occupy consecutive blockIdx.x ranges starting at cta_begin
@@ -215,7 +222,7 @@ MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long l
           tma_load_2d(sa + 8192, &G.tmA, &full_bar[s], m_tile * GEMM_BM + 64, kb * GEMM_BK);
         }
         if (BMODE == B_TMA_K) {
-          tma_load_2d(sb, &G.tmB, &full_bar[s], kb * GEMM_BK, 0);                          // box {64 k, N}
+          tma_load_2d(sb, &G.tmB, &full_bar[s], kb * GEMM_BK, G.n_off);                    // box {64 k, N}
         } else {
           for (int c = 0; c < N / 64; ++c)
             tma_load_2d(sb + c * 8192, &G.tmB, &full_bar[s], G.n_off + c * 64, kb * GEMM_BK);   // box {64 n, 64 k}
@@ -323,6 +330,7 @@ MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long l
     }
     if (et == 0) GEMM_STAMP(10);                // accumulator complete
     const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16);
+    const int ldc = G.ldc ? G.ldc : N;
     for (int c0 = 32 * drain_idx; c0 < N; c0 += 32 * drain_members) {
       float v[32];
       if (nkb > 0) {
@@ -333,7 +341,7 @@ MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long l
         for (int j = 0; j < 32; ++j) v[j] = 0.f;
       }
       if (EPI == EPI_ACT) {
-        const float* bp = G.bias + c0;          // leaf offsets in the arena are only 4-byte aligned
+        const float* bp = G.bias + G.n_off + c0;   // leaf offsets in the arena are only 4-byte aligned
         uint32_t w[16];
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
@@ -349,11 +357,11 @@ MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long l
           w[2 * j] = pack_bf16x2(x0, x1);
           w[2 * j + 1] = pack_bf16x2(x2, x3);
         }
-        uint4* o = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(G.out) + static_cast<size_t>(row) * G.ldo + c0);
+        uint4* o = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(G.out) + static_cast<size_t>(row) * G.ldo + G.n_off + c0);
 #pragma unroll
         for (int j = 0; j < 4; ++j) o[j] = make_uint4(w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]);
       } else if (EPI == EPI_DACT) {
-        const uint4* h4 = reinterpret_cast<const uint4*>(G.hprev + static_cast<size_t>(row) * G.ldh + c0);
+        const uint4* h4 = reinterpret_cast<const uint4*>(G.hprev + static_cast<size_t>(row) * G.ldh + G.n_off + c0);
         uint32_t w[16];
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
@@ -372,7 +380,7 @@ MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long l
             v[e] = bf16_lo(w[4 * j + t]); v[e + 1] = bf16_hi(w[4 * j + t]);
           }
         }
-        uint4* o = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(G.out) + static_cast<size_t>(row) * G.ldo + c0);
+        uint4* o = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(G.out) + static_cast<size_t>(row) * G.ldo + G.n_off + c0);
 #pragma unroll
         for (int j = 0; j < 4; ++j) o[j] = make_uint4(w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]);
         const float cs = warp_colsum32(v);
@@ -404,14 +412,14 @@ MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long l
         float out = v[0];
 #pragma unroll
         for (int j = 1; j < 32; ++j) out = (static_cast<int>(lane_id()) == j) ? v[j] : out;
-        G.colsum_out[static_cast<size_t>(split) * N + cs_c0 + ch * 32 + lane_id()] = out;
+        G.colsum_out[static_cast<size_t>(split) * ldc + G.n_off + cs_c0 + ch * 32 + lane_id()] = out;
       }
     }
     if (EPI == EPI_DACT) {
       asm volatile("bar.sync 1, 128;" ::: "memory");
       for (int c = et; c < N; c += GEMM_EPI_THREADS) {
         const float s = (colsum_s[c] + colsum_s[GEMM_MAXN + c]) + (colsum_s[2 * GEMM_MAXN + c] + colsum_s[3 * GEMM_MAXN + c]);
-        G.colsum[static_cast<size_t>(m_tile) * N + c] = s;
+        G.colsum[static_cast<size_t>(m_tile) * ldc + G.n_off + c] = s;
       }
     }
   }
