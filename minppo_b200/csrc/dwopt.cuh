@@ -46,8 +46,6 @@ struct PeerXchg {
   int world, rank;
   int np;                        // floats per staging slot (multiple of 4)
   int two_phase;                 // 0: one-shot push to every rank; 1: reduce at rank (CTA index % W), result pushed back
-  int ablate;                    // debug (MINPPO_PX_ABLATE, TIMING ONLY, wrong results): 1 = push but never wait for the
-                                 // peers, 2 = neither push nor wait
 };
 MINPPO_DEVINL float* px_stage(const PeerXchg& x, int r, unsigned int par, int q) {
   return reinterpret_cast<float*>(x.base[r]) + (static_cast<size_t>(par) * x.world + q) * x.np;
@@ -112,7 +110,7 @@ struct alignas(64) DwOptParams {
   int prefetch;                  // 1: L2 prefetch of the next minibatch's observation rows by the GEMM CTAs' helper warps
   const __nv_bfloat16* obs_img;  // [Bl][obs_ld]
   int obs_ld;
-  int step;                      // dwopt_kernel: the minibatch step of this launch (the persistent kernel loops)
+  int step;                      // the minibatch step of this launch
 };
 
 template <int NTHREADS_MAX = 1024>
@@ -133,15 +131,14 @@ MINPPO_DEVINL float block_sum_dyn(float v, float* scratch /*[32]*/) {
 // MAXU = 4-element units of the hidden kernels a thread may own (fast path: reduced gradient and optimizer state stay in
 // registers across the second barrier).  MAXU = 1 covers P_late <= 4 * grid * 512 (303k parameters on 148 SMs: the
 // stand-in shape); larger observation widths take MAXU = 2 or 4.
-// The whole CTA calls this (any block size that is a multiple of 32 and >= GEMM_THREADS; all CTAs of the grid co-resident).
-// `ext_tmem`: TMEM base of a persistent caller (GEMM_NO_TMEM: the GEMM allocates and frees its own columns).
 template <int MAXU>
-MINPPO_DEVINL void dwopt_body(const DwOptParams& p, int step, uint8_t* smem_raw, uint32_t ext_tmem, bool build_tab = true) {
+__global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_constant__ DwOptParams p) {
+  extern __shared__ uint8_t smem_raw[];
   __shared__ float scratch[32];
   __shared__ float s_bcast[4];
   __shared__ LeafTab T;
   const OptArgs& a = p.opt;
-  const int P = a.P;
+  const int P = a.P, step = p.step;
   const int G = static_cast<int>(gridDim.x), NT = static_cast<int>(blockDim.x);
   const int32_t* row_count = p.padded ? p.counts + step : nullptr;          // rows of this minibatch on this rank
   const int32_t* next_ridx = (p.prefetch && step + 1 < p.EM) ? p.ridx_base + static_cast<size_t>(step + 1) * p.cap : nullptr;
@@ -162,10 +159,10 @@ MINPPO_DEVINL void dwopt_body(const DwOptParams& p, int step, uint8_t* smem_raw,
   }
   // The leaf table (kernel parameters -> shared memory: cold constant-bank misses, ~2k cycles at the head of a launch) is first
   // read in phase 2.  GEMM CTAs: the helper warps copy it while the GEMM is in flight (the CTA-wide barrier at the end of the GEMM
-  // body orders it); spare CTAs need it at once.  (A persistent caller builds the table once: it only depends on the launch.)
+  // body orders it); spare CTAs need it at once.
   const bool gemm_cta = b < p.gemm_ctas;
   if (!gemm_cta) {
-    if (build_tab) leaf_tab_build(T, a, t, NT);
+    leaf_tab_build(T, a, t, NT);
     __syncthreads();
   }
   DW_STAMP(14);
@@ -194,7 +191,7 @@ MINPPO_DEVINL void dwopt_body(const DwOptParams& p, int step, uint8_t* smem_raw,
     // update: no dependency on the preceding kernel).  Spread over all GEMM CTAs so that it never rides on the few
     // spare CTAs, whose number depends on the split-K factor.
     auto idle_work = [&]() {
-      if (build_tab) leaf_tab_build(T, a, t - GEMM_THREADS, NT - GEMM_THREADS);
+      leaf_tab_build(T, a, t - GEMM_THREADS, NT - GEMM_THREADS);
       scalars();
       if (next_ridx) {
         const int HELPERS = NT - GEMM_THREADS;
@@ -207,7 +204,7 @@ MINPPO_DEVINL void dwopt_body(const DwOptParams& p, int step, uint8_t* smem_raw,
         }
       }
     };
-    umma_gemm_body<EPI_PARTIAL>(p.gemm, smem_raw, p.trace ? p.trace + static_cast<size_t>(b) * 16 : nullptr, idle_work, ext_tmem,
+    umma_gemm_body<EPI_PARTIAL>(p.gemm, smem_raw, p.trace ? p.trace + static_cast<size_t>(b) * 16 : nullptr, idle_work,
                                 p.ridx_base + static_cast<size_t>(step) * p.cap, row_count);   // PDL wait / trigger inside
   } else {
     scalars();
@@ -275,11 +272,11 @@ MINPPO_DEVINL void dwopt_body(const DwOptParams& p, int step, uint8_t* smem_raw,
     // ---- one-shot all-reduce over NVLink peer memory (PeerXchg above; requires the fast path) -----------------
     const PeerXchg& X = p.px;
     const int R = X.rank;
-    const int W = X.ablate == 2 ? 1 : X.world;             // ablation: behave like a lone rank (slot R is never read)
+    const int W = X.world;
     // Once the error flag is up (a peer never delivered within the bound, or any earlier device-side guard fired) the
     // exchange stops waiting: the update is already lost (minppo_ctx_check reports it), and 128 steps x the spin bound
     // must not turn one dead peer into a quarter of an hour of hung GPUs.
-    const bool nowait = X.ablate != 0 || s_dead != 0;
+    const bool nowait = s_dead != 0;
     const unsigned int n = s_seq, par = n & 1u;
     const int n_late4 = 4 * n_units;
     // early element (or loss sum) of this thread: same job numbering as apply_adam_class<false>
@@ -519,12 +516,6 @@ MINPPO_DEVINL void dwopt_body(const DwOptParams& p, int step, uint8_t* smem_raw,
       if (gnorm_out) *gnorm_out = sc.gnorm;
     }
   }
-}
-
-template <int MAXU>
-__global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_constant__ DwOptParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  dwopt_body<MAXU>(p, p.step, smem_raw, GEMM_NO_TMEM);
 }
 
 // largest parameter count of the hidden kernels the register-resident fast path covers on a grid of `grid` CTAs

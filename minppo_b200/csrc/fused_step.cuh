@@ -111,7 +111,7 @@ struct alignas(64) FusedParams {
   int part_stride, po_logstd;
   int H, A, Dp, m_tiles, cap;
   int store_x;                   // 1: the critic CTAs store the gathered X tile for the dW GEMM (0: that GEMM gathers by index itself)
-  int step;                      // minibatch step e * M + k of this launch (fused_step_kernel; the persistent kernel loops)
+  int step;                      // minibatch step e * M + k of this launch
   float inv_mb, clip_eps, vf_coef;
   long long* trace;              // debug: [ctas][32] clock64 stamps (null = off)
 };
@@ -314,9 +314,8 @@ MINPPO_DEVINL void epilogue_dact(uint32_t tmem_acc, uint32_t h_base, uint32_t ds
 }
 
 // One (tile, net) unit of one minibatch step.  The whole CTA (FS_THREADS threads) calls this with the SAME arguments;
-// `sm` / `base` = the 1024-byte aligned dynamic shared memory, `tmem_base` = 512 allocated TMEM columns.  The mbarriers
-// are (re-)initialised on entry, so a persistent caller may run any number of units back to back.
-template <int AP, bool PERSISTENT>
+// `sm` / `base` = the 1024-byte aligned dynamic shared memory, `tmem_base` = 512 allocated TMEM columns.
+template <int AP>
 MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t* sm, uint32_t base, uint32_t tmem_base) {
   using LY = FsLayout<AP>;
   constexpr int NS = LY::NS, NS1 = LY::NS1, PG = LY::PG, RS = LY::RS;
@@ -375,7 +374,7 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
     if (threadIdx.x == 0) part[G.po_loss] = 0.f;
     return;
   }
-  __syncthreads();                       // persistent callers: the previous unit / phase is done with this memory
+  __syncthreads();
   if (threadIdx.x == FS_WORKERS) {
     FS_STAMP(16);
     // tensor maps into the descriptor cache first (weights: in front of the first L1 stage; stores: off any critical path)
@@ -407,7 +406,6 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
     // ===================== weight producer ======================================================================
     if (elect_one()) {
       griddep_wait();                 // the weight images are rewritten by the previous optimizer step
-      if (PERSISTENT) fence_proxy_async_global();   // ... published through a grid barrier (generic-proxy acquire)
       const uint32_t bytes = static_cast<uint32_t>(H) * 64u;
       // ---- L1: W0 half-k-blocks j = 0 .. 2 nk0 - 1 through NS1 stages (the ring + four stages parked in R0, which nothing
       //      touches before epilogue 1: for Dp <= 256 the whole L1 GEMM is fed up front)
@@ -913,13 +911,8 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
       tmem_ld_wait();
       if (sub * 128 + erow < H) part[G.po_db0 + sub * 128 + erow] = cs1;               // layer-0 bias gradient of this tile
     }
-    // The bulk stores must have READ shared memory before it is reused, and -- for a persistent caller, whose next phase
-    // reads H1 / dZ / X from other CTAs after a grid barrier, not after a kernel boundary -- their global writes must be
-    // complete and ordered before this thread's later (generic-proxy) barrier arrival.
-    if (wt == FS_STORE_THREAD || wt == 0) {                       // thread 0: the dW2 bulk copy (and, critic CTA, the X stores)
-      if (PERSISTENT) { tma_store_wait_all0(); fence_proxy_async_global(); }
-      else tma_store_wait_read0();                                 // one launch per step: the writes complete with the grid
-    }
+    // The bulk stores must have READ shared memory before the CTA exits; their global writes complete with the grid.
+    if (wt == FS_STORE_THREAD || wt == 0) tma_store_wait_read0();   // thread 0: the dW2 bulk copy (and, critic CTA, the X stores)
     if (wt == 0) FS_STAMP(12);
   }
 
@@ -948,10 +941,10 @@ __global__ void __launch_bounds__(FS_THREADS, 1) fused_step_kernel(const __grid_
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = tmem_slot;
-    fused_tile<AP, false>(p, unit, p.step, sm, base, tmem_base);
+    fused_tile<AP>(p, unit, p.step, sm, base, tmem_base);
     if (warp == FS_MMA_WARP) tmem_dealloc(tmem_base, 512);
   } else {
-    fused_tile<AP, false>(p, unit, p.step, sm, base, 0u);                // dead tile: zeroes its partials and returns
+    fused_tile<AP>(p, unit, p.step, sm, base, 0u);                // dead tile: zeroes its partials and returns
   }
 }
 

@@ -28,7 +28,6 @@
 #include "umma_gemm.cuh"
 #include "fused_step.cuh"
 #include "dwopt.cuh"
-#include "ppo_steps.cuh"
 #include "policy_fused.cuh"
 
 namespace minppo {
@@ -262,16 +261,10 @@ struct minppo_ctx {
   long long* trace;           // debug cycle stamps of the fused kernel [2*m_tiles][FS_TRACE_SLOTS]
   long long* trace2;          // debug cycle stamps of the dwopt kernel [sm_count][8]
   bool trace_on;
-  bool pdl;                   // programmatic dependent launch between step kernels (MINPPO_PDL=0 disables)
-  bool merged_opt;            // dW GEMM + reduction + Adam in one launch (MINPPO_SPLIT_OPT=1 disables)
-  bool persistent;            // all E x M minibatch steps in ONE persistent launch (ppo_steps.cuh; MINPPO_PERSISTENT=0 disables)
-  int steps_per_launch;       // development probe (MINPPO_STEPS_PER_LAUNCH): minibatch steps per persistent launch (0 = all)
-  int skip_mask;              // debug (MINPPO_SKIP): 1 = no fused step, 2 = no dW GEMM, 4 = no optimizer (timing ablation only)
   int32_t *perms, *rowidx, *counts;
   int32_t* perm_tmp;          // world_size > 1: the epochs THIS rank sorts ([ceil(E / W)][B]); broadcast into perms
-  bool padded;                // row lists sized for a worst-case row count (world_size > 1, or MINPPO_EMULATE_SHARD_PAD=W: timing probe
-                              // of the sharded shapes on one GPU): device-side row counts bound the per-minibatch work
-  bool share_perm;            // epoch e is sorted by rank e % W only and broadcast (MINPPO_SHARE_PERM=0: every rank sorts all)
+  bool padded;                // row lists sized for a worst-case row count (world_size > 1): device-side row counts bound
+                              // the per-minibatch work
   void* perm_ws;
   size_t perm_ws_bytes;
   __nv_bfloat16* obs_img;
@@ -387,7 +380,6 @@ static int init_kernel_attrs() {
   CK(cudaFuncSetAttribute(dwopt_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
   CK(cudaFuncSetAttribute(dwopt_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
   CK(cudaFuncSetAttribute(dwopt_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
-  CK(steps_init_attrs());
   CK(policy_fused_init_attrs());
   return 0;
 }
@@ -466,7 +458,7 @@ static int nccl_allreduce(minppo_ctx* c, float* buf, size_t n, cudaStream_t stre
   return 0;
 }
 
-// ---- parameter blocks of the per-minibatch kernels (shared by the per-step launches and the persistent kernel) ----
+// ---- parameter blocks of the per-minibatch kernels ----
 static void fill_fused_params(minppo_ctx* c, const UpdatePtrs& u, FusedParams* pp) {
   FusedParams& p = *pp;
   memset(&p, 0, sizeof(p));
@@ -514,7 +506,7 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
       g.cta_begin = cta;
       const int in_l = l == 0 ? c->D : H;
       const int in_pad = l == 0 ? c->Dp : H;
-      if (l == 0 && c->fused && c->store_x && !(c->skip_mask & 1)) { g.amode = A_TMA_MN; g.tmA = c->m_xg_mn; }   // rows gathered by the fused kernel
+      if (l == 0 && c->fused && c->store_x) { g.amode = A_TMA_MN; g.tmA = c->m_xg_mn; }   // rows gathered by the fused kernel
       else if (l == 0) { g.amode = A_GATHER_MN; g.rowidx = c->rowidx; g.gimage = c->obs_img; g.ldg = c->Dp; }      // row list: per step
       else { g.amode = A_TMA_MN; g.tmA = nb.m_act_mn[l]; }
       g.bmode = B_TMA_MN; g.tmB = nb.m_dz_mn[l + 1];
@@ -549,9 +541,8 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
   const int L = c->L, H = c->H;
   const int32_t* ridx = c->rowidx + static_cast<size_t>(s) * c->cap;
   // programmatic dependent launch between the per-minibatch kernels (fused path only; common.cuh)
-  const bool pdl = c->pdl && c->fused && !c->profiling;
-  if (c->fused && (c->skip_mask & 1)) {
-  } else if (c->fused) {
+  const bool pdl = c->fused && !c->profiling;
+  if (c->fused) {
     // forward + heads + loss + backward-to-dZ of both nets in one launch (fused_step.cuh)
     FusedParams p;
     fill_fused_params(c, u, &p);
@@ -639,19 +630,18 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
   }
   }  // !fused
   // weight gradients dW_l = act[l]^T dz[l+1] (split-K over minibatch rows), then the optimizer.
-  // Default: ONE launch (dwopt.cuh).  MINPPO_SPLIT_OPT=1, a grid that does not fit one CTA per SM or
-  // the timing ablation fall back to the two-launch sequence (GEMM kernel, opt_kernel).
+  // ONE launch (dwopt.cuh) when the GEMM grid fits one CTA per SM; otherwise the two-launch sequence (GEMM kernel,
+  // opt_kernel).
   DwOptParams dp;
   const int cta = fill_dwopt_params(c, u, &dp);
   dp.step = s;
   GemmParams& p = dp.gemm;
   OptArgs& o = dp.opt;
   const bool sharded = c->cfg.world_size > 1;
-  const bool merged = c->merged_opt && c->skip_mask == 0 && cta <= c->sm_count;
-  if (merged) {
+  if (cta <= c->sm_count) {
     // all-reduce fused into this launch (peer memory); needs the register-resident fast path of the kernel
     const bool px_on = sharded && c->peers_set && c->P <= dwopt_fast_capacity(c->sm_count, c->maxu);
-    if (px_on) { dp.px = c->px; dp.px.ablate = getenv("MINPPO_PX_ABLATE") ? atoi(getenv("MINPPO_PX_ABLATE")) : 0; }
+    if (px_on) dp.px = c->px;
     o.do_reduce = 1; o.do_apply = (sharded && !px_on) ? 0 : 1;
     {
       PROF(PC_DW_GEMM);
@@ -675,25 +665,23 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
   }
   o.losses_out = o.losses_out + static_cast<size_t>(s) * dp.losses_stride;
   o.gnorm_out = c->gnorms + s;
-  if (!(c->skip_mask & 2)) {
+  {
     PROF(PC_DW_GEMM);
     RET(launch_gemm<EPI_PARTIAL>(p, cta, stream, pdl));
     c->launches++;
   }
-  if (!(c->skip_mask & 4)) {
-    if (!sharded) {
-      o.do_reduce = 1; o.do_apply = 1;
-      PROF(PC_OPT);
-      RET(opt_launch(o, c->opt_blocks, stream, pdl));
-      c->launches++;
-    } else {
-      o.do_reduce = 1; o.do_apply = 0;
-      { PROF(PC_OPT); RET(opt_launch(o, c->opt_blocks, stream, pdl)); }
-      { PROF(PC_ALLREDUCE); RET(nccl_allreduce(c, c->gflat, static_cast<size_t>(c->P) + 2, stream)); }
-      o.do_reduce = 0; o.do_apply = 1;
-      { PROF(PC_OPT); RET(opt_launch(o, c->opt_blocks, stream, pdl)); }
-      c->launches += 3;
-    }
+  if (!sharded) {
+    o.do_reduce = 1; o.do_apply = 1;
+    PROF(PC_OPT);
+    RET(opt_launch(o, c->opt_blocks, stream, pdl));
+    c->launches++;
+  } else {
+    o.do_reduce = 1; o.do_apply = 0;
+    { PROF(PC_OPT); RET(opt_launch(o, c->opt_blocks, stream, pdl)); }
+    { PROF(PC_ALLREDUCE); RET(nccl_allreduce(c, c->gflat, static_cast<size_t>(c->P) + 2, stream)); }
+    o.do_reduce = 0; o.do_apply = 1;
+    { PROF(PC_OPT); RET(opt_launch(o, c->opt_blocks, stream, pdl)); }
+    c->launches += 3;
   }
   return 0;
 }
@@ -709,7 +697,7 @@ static int enqueue_update(minppo_ctx* c, const UpdatePtrs& u, cudaStream_t strea
   // parallel branch of the graph).  The permutation chain is 25+ tiny dependent launches, the observation image one
   // bandwidth-bound pass over the trajectory: side by side they cost the longer of the two.  Eager profiling runs keep
   // everything on one stream so that the per-class event times stay attributable.
-  const bool fork = !c->profiling && !(getenv("MINPPO_NO_FORK") && atoi(getenv("MINPPO_NO_FORK")) != 0);
+  const bool fork = !c->profiling;
   if (fork) {
     CK(cudaEventRecord(c->ev_fork, stream));
     CK(cudaStreamWaitEvent(c->side_stream, c->ev_fork, 0));
@@ -725,7 +713,7 @@ static int enqueue_update(minppo_ctx* c, const UpdatePtrs& u, cudaStream_t strea
     RET(gae_launch(u.reward, u.value, u.done, u.last_val, c->adv, c->tgt, c->T, c->Nl, gamma, gl, c->sm_count, 0, stream));
     c->launches++;
   }
-  if (c->share_perm) {
+  if (cfg.world_size > 1) {
     // The permutations depend only on the key chain, so the ranks split the sorting work by epoch (rank e % W sorts
     // epoch e) and broadcast: every rank still ends up with the same GLOBAL permutations, bit for bit.
     PROF(PC_PERM);
@@ -774,29 +762,6 @@ static int enqueue_update(minppo_ctx* c, const UpdatePtrs& u, cudaStream_t strea
       PROF(PC_WEIGHT_IMAGES);
       RET(weight_images_launch(o, stream));
       c->launches++;
-    }
-  }
-  // The E x M minibatch steps: ONE persistent launch (ppo_steps.cuh) when the fused path applies and the optimizer can
-  // run inside it (single GPU, or env-sharded ranks with the peer-memory exchange); otherwise two launches per step.
-  if (c->persistent && c->fused && c->merged_opt && c->skip_mask == 0 && !c->profiling) {
-    StepsParams sp;
-    memset(&sp, 0, sizeof(sp));
-    fill_fused_params(c, u, &sp.fs);
-    const int cta = fill_dwopt_params(c, u, &sp.dw);
-    const bool sharded = cfg.world_size > 1;
-    const bool px_on = sharded && c->peers_set && c->P <= dwopt_fast_capacity(c->sm_count, c->maxu);
-    if (cta <= c->sm_count && (!sharded || px_on)) {
-      if (px_on) { sp.dw.px = c->px; sp.dw.px.ablate = getenv("MINPPO_PX_ABLATE") ? atoi(getenv("MINPPO_PX_ABLATE")) : 0; }
-      sp.dw.opt.do_reduce = 1; sp.dw.opt.do_apply = 1;
-      sp.units = 2 * c->m_tiles;
-      const int chunk = c->steps_per_launch > 0 ? c->steps_per_launch : EM;
-      for (int s0 = 0; s0 < EM; s0 += chunk) {
-        sp.s0 = s0; sp.s1 = std::min(EM, s0 + chunk);
-        const cudaError_t e = steps_launch(sp, c->sm_count, stream, c->ap, c->maxu);
-        if (e != cudaSuccess) { set_error("ppo_steps launch failed: %s", cudaGetErrorString(e)); return MINPPO_ERR_CUDA; }
-        c->launches++;
-      }
-      return 0;
     }
   }
   for (int s = 0; s < EM; ++s) RET(enqueue_step(c, u, s, stream));
@@ -917,14 +882,11 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   c->D = cfg->obs_dim; c->Dp = (c->D + 63) / 64 * 64; c->A = cfg->act_dim;
   c->B = static_cast<long long>(c->T) * c->N; c->Bl = static_cast<long long>(c->T) * c->Nl;
   c->mb = static_cast<int>(c->B / c->M);
-  const int pad_emul = (cfg->world_size == 1 && getenv("MINPPO_EMULATE_SHARD_PAD")) ? atoi(getenv("MINPPO_EMULATE_SHARD_PAD")) : 0;
-  c->padded = cfg->world_size > 1 || pad_emul > 1;
+  c->padded = cfg->world_size > 1;
   if (!c->padded) c->cap = c->mb;
   else {
     long long cap = (3LL * c->mb / cfg->world_size + 1) / 2 + 256;    // 1.5 x mean + 256 rows
-    if (pad_emul == 3) cap = c->mb + 128;                             // probe: one spare tile only
-    else if (pad_emul > 1) cap = c->mb + c->mb / 2 + 256;                  // what a rank of a pad_emul-way job with this many rows would get
-    if (cap > c->mb && pad_emul <= 1) cap = c->mb;
+    if (cap > c->mb) cap = c->mb;
     if (cap > c->Bl) cap = c->Bl;
     c->cap = static_cast<int>(cap);
   }
@@ -952,21 +914,19 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
     // their observation rows by index (A_GATHER_MN), so every row is gathered once per column group: twice the
     // observation-image reads of that layer's A operand.
     c->dw_nsplit = c->H > GEMM_MAXN ? 2
-                 : (c->fused && c->store_x && c->H % 128 == 0 && 2 * 2 * c->L <= GEMM_MAX_GROUPS &&
-                    !(getenv("MINPPO_DW_NSPLIT") && atoi(getenv("MINPPO_DW_NSPLIT")) == 1)) ? 2 : 1;
+                 : (c->fused && c->store_x && c->H % 128 == 0 && 2 * 2 * c->L <= GEMM_MAX_GROUPS) ? 2 : 1;
     int per_split = 0;
     for (int l = 0; l < c->L; ++l) per_split += 2 * c->dw_nsplit * (((l == 0 ? c->Dp : c->H) + 127) / 128);
     // leave ~16 of the one-CTA-per-SM grid as spare CTAs: they sum the per-tile partials of the small leaves while the GEMM
     // runs (D = 415 / A = 20 with 4 spare CTAs: 6,441 elements x 64 partials on 2,048 threads outlasted the GEMM itself)
     const int gemm_budget = c->sm_count > 48 ? c->sm_count - 16 : c->sm_count;
     int S = cfg->dw_splits > 0 ? cfg->dw_splits : (gemm_budget / (per_split > 0 ? per_split : 1));
-    if (getenv("MINPPO_DW_SPLITS")) S = atoi(getenv("MINPPO_DW_SPLITS"));           // development probe
     // k-blocks (64 minibatch rows each) the splits share.  Padded row lists (env-sharded ranks): size the split for the
     // rows a minibatch is EXPECTED to have on this rank (mean + 3 sigma of the hypergeometric count), not for the
     // worst-case capacity -- the kernel splits the live k-blocks at run time, an over-sized S only removes spare CTAs.
     int kb_total = c->M_pad / 64;
     if (c->padded) {
-      const double mean = pad_emul > 1 ? c->mb : static_cast<double>(c->mb) / cfg->world_size;
+      const double mean = static_cast<double>(c->mb) / cfg->world_size;
       const long long rows = static_cast<long long>(mean + 3.0 * sqrt(mean)) + 1;
       kb_total = static_cast<int>(std::min<long long>(c->M_pad, rows + 63) / 64);
       if (kb_total < 1) kb_total = 1;
@@ -1022,18 +982,9 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   ALLOC(c->trace, static_cast<size_t>(2 * c->m_tiles) * FS_TRACE_SLOTS);
   ALLOC(c->trace2, static_cast<size_t>(c->sm_count) * 16);
   c->trace_on = getenv("MINPPO_TRACE") != nullptr;
-  c->pdl = !(getenv("MINPPO_PDL") && atoi(getenv("MINPPO_PDL")) == 0);
-  c->merged_opt = !(getenv("MINPPO_SPLIT_OPT") && atoi(getenv("MINPPO_SPLIT_OPT")) != 0);
-  c->skip_mask = getenv("MINPPO_SKIP") ? atoi(getenv("MINPPO_SKIP")) : 0;
-  // Measured (profiles/r02_persistent_vs_per_step.txt): the persistent kernel is 0.3 ms per update SLOWER at 1 GPU and 0.5 ms
-  // at 2 -- a grid barrier (release fence + atomic + acquire poll, ~2.2k cycles before skew) costs as much as a kernel boundary
-  // under programmatic dependent launch, and it needs four per step against two boundaries + two barriers.  Off by default.
-  c->persistent = getenv("MINPPO_PERSISTENT") && atoi(getenv("MINPPO_PERSISTENT")) != 0;
-  c->steps_per_launch = getenv("MINPPO_STEPS_PER_LAUNCH") ? atoi(getenv("MINPPO_STEPS_PER_LAUNCH")) : 0;
   ALLOC(c->perms, static_cast<size_t>(c->E) * c->B);
   c->perm_tmp = nullptr;
-  c->share_perm = cfg->world_size > 1 && !(getenv("MINPPO_SHARE_PERM") && atoi(getenv("MINPPO_SHARE_PERM")) == 0);
-  if (c->share_perm) ALLOC(c->perm_tmp, static_cast<size_t>((c->E + cfg->world_size - 1) / cfg->world_size) * c->B);
+  if (cfg->world_size > 1) ALLOC(c->perm_tmp, static_cast<size_t>((c->E + cfg->world_size - 1) / cfg->world_size) * c->B);
   ALLOC(c->rowidx, static_cast<size_t>(EM) * c->cap);
   ALLOC(c->counts, static_cast<size_t>(EM));
   c->perm_ws_bytes = perm_workspace_bytes(c->E, c->B);
@@ -1173,7 +1124,7 @@ int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, con
   if (!actor && !value) { set_error("minppo_policy_step: no output requested"); return MINPPO_ERR_ARG; }
   cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
   const int L = c->L, H = c->H;
-  if (c->fused && !(getenv("MINPPO_POLICY_LAYERWISE") && atoi(getenv("MINPPO_POLICY_LAYERWISE")) != 0)) {
+  if (c->fused) {
     // 2-hidden-layer nets: ONE launch (policy_fused.cuh) -- observation conversion, both hidden layers, heads, sampler
     if (!(flags & MINPPO_POLICY_WEIGHTS_CURRENT)) {
       UpdatePtrs u;

@@ -110,13 +110,11 @@ MINPPO_DEVINL float warp_colsum32(float (&v)[32]) {
 // in the two CTA-wide barriers.
 struct GemmNoIdle { MINPPO_DEVINL void operator()() const {} };
 // `idle` runs on the helper warps (warps >= 6, if the caller has any) while the GEMM is in flight.
-// Persistent callers (ppo_steps.cuh) pass the TMEM base they allocated once (`ext_tmem`; 0xFFFFFFFF = allocate and free
-// here), per-step overrides of the gather row list / valid-row count, and get the mbarriers re-initialised on every call.
-constexpr uint32_t GEMM_NO_TMEM = 0xFFFFFFFFu;
+// `step_rowidx` / `step_kcount` override the groups' gather row list / valid-row count (dwopt.cuh: the minibatch step's
+// entries of the per-update arrays, so that one parameter block serves every step).
 template <int EPI, typename IdleFn = GemmNoIdle>
 MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long long* trace = nullptr, IdleFn idle = IdleFn(),
-                                  uint32_t ext_tmem = GEMM_NO_TMEM, const int32_t* step_rowidx = nullptr,
-                                  const int32_t* step_kcount = nullptr) {
+                                  const int32_t* step_rowidx = nullptr, const int32_t* step_kcount = nullptr) {
 #define GEMM_STAMP(slot) do { if (trace) trace[(slot)] = clock64(); } while (0)
   const uint32_t raw = smem_u32(smem_raw);
   const uint32_t base = (raw + 1023u) & ~1023u;                      // SWIZZLE_128B: 1024-B aligned tiles
@@ -178,14 +176,14 @@ MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long l
     fence_mbar_init();
     GEMM_STAMP(15);
   }
-  if (warp == 1 && ext_tmem == GEMM_NO_TMEM) {
+  if (warp == 1) {
     tmem_alloc(tmem_slot, kTmemCols);
     tmem_relinquish();
   }
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  const uint32_t tmem_base = ext_tmem == GEMM_NO_TMEM ? *tmem_slot : ext_tmem;
+  const uint32_t tmem_base = *tmem_slot;
   if (threadIdx.x == 64) GEMM_STAMP(6);                 // prologue done
 
   // EPI_PARTIAL: warps beyond the six role warps (a caller running more warps per CTA, dwopt.cuh) help draining the
@@ -202,8 +200,6 @@ MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long l
     if (elect_one()) {
       griddep_wait();                  // PDL (common.cuh): operands are written by the preceding kernel
       griddep_launch();
-      if (ext_tmem != GEMM_NO_TMEM)    // persistent callers: the operands were published through a grid barrier (generic-proxy
-        fence_proxy_async_global();    // acquire) -- order the TMA (async-proxy) reads below after it
       GEMM_STAMP(7);                   // dependency wait passed
       const uint32_t a_bytes = kTmaA ? GEMM_A_BYTES : 0;
       const uint32_t b_bytes = static_cast<uint32_t>(N) * GEMM_BK * 2;
@@ -456,7 +452,7 @@ MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long l
 
   tc_fence_before();
   __syncthreads();
-  if (warp == 1 && ext_tmem == GEMM_NO_TMEM) tmem_dealloc(tmem_base, kTmemCols);
+  if (warp == 1) tmem_dealloc(tmem_base, kTmemCols);
 }
 
 template <int EPI>

@@ -1,10 +1,10 @@
 #!/bin/bash
-# One GPU session (single GPU): parity tests, smoke, PDL / ablation timings, fused-kernel cycle trace,
+# One GPU session (single GPU): parity tests, smoke, fused-kernel cycle trace,
 # full bench, ncu launch list and ncu --set full captures.  Everything lands in gpurun_out/.
-# Usage: bash scripts/gpu_call.sh [tests] [ablate] [trace] [bench] [ncu] [ncufull]   (default: all)
+# Usage: bash scripts/gpu_call.sh [tests] [trace] [bench] [ncu] [ncufull]   (default: all)
 cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
-WHAT="${*:-tests ablate trace bench ncu ncufull}"
+WHAT="${*:-tests trace bench ncu ncufull}"
 has() { [[ " $WHAT " == *" $1 "* ]]; }
 nvidia-smi > gpurun_out/nvidia_smi.txt 2>&1
 nproc > gpurun_out/nproc.txt
@@ -16,15 +16,6 @@ if has tests; then
   timeout 600 python -c "import __graft_entry__ as g; g.smoke()" > gpurun_out/smoke.log 2>&1
   echo "exit $?" >> gpurun_out/smoke.log
   tail -n 3 gpurun_out/pytest_*.log gpurun_out/smoke.log
-fi
-if has ablate; then
-  : > gpurun_out/ablate.log
-  for cfg in "MINPPO_PDL=1" "MINPPO_PDL=0" "MINPPO_PDL=1 MINPPO_SPLIT_OPT=1" "MINPPO_PDL=1 MINPPO_SKIP=6" \
-             "MINPPO_PDL=1 MINPPO_SKIP=5" "MINPPO_PDL=1 MINPPO_SKIP=3" $EXTRA_ABLATE; do
-    echo "## $cfg" >> gpurun_out/ablate.log
-    env $cfg timeout 600 python bench.py --quick --steps 10 --warmup 3 2>&1 | tail -n 2 >> gpurun_out/ablate.log
-  done
-  cat gpurun_out/ablate.log
 fi
 if has trace; then
   timeout 600 python scripts/trace_fused.py > gpurun_out/trace_fused.log 2>&1

@@ -17,7 +17,7 @@ for tp in 1 0; do
 done
 OUT=gpurun_out/multi_timing_g$N.log
 : > $OUT
-for cfg in "MINPPO_PX_TWO_PHASE=1" "MINPPO_PX_TWO_PHASE=0" "MINPPO_NCCL_ALLREDUCE=1" "MINPPO_PX_ABLATE=2" $EXTRA_ABLATE; do
+for cfg in "MINPPO_PX_TWO_PHASE=1" "MINPPO_PX_TWO_PHASE=0" "MINPPO_NCCL_ALLREDUCE=1" $EXTRA_ABLATE; do
   port=$((port + 1))
   echo "## $cfg" >> $OUT
   env $cfg timeout 300 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 \

@@ -10,7 +10,7 @@ echo "exit $?" >> gpurun_out/multigpu_parity_g${N}.log
 grep -E "^\[(small|wide)|MULTIGPU|^exit|MinppoError" gpurun_out/multigpu_parity_g${N}.log | cut -c1-400 | tail -n 4
 OUT=gpurun_out/multi_timing_g$N.log
 : > $OUT
-for cfg in $TIMING_CFGS; do   # e.g. TIMING_CFGS="MINPPO_PX_TWO_PHASE=0 MINPPO_PX_ABLATE=2"
+for cfg in $TIMING_CFGS; do   # e.g. TIMING_CFGS="MINPPO_PX_TWO_PHASE=0 MINPPO_NCCL_ALLREDUCE=1"
   port=$((port + 1))
   echo "## $cfg" >> $OUT
   env $cfg timeout 300 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 \

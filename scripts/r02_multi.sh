@@ -1,5 +1,5 @@
 #!/bin/bash
-# round 2 multi-GPU session (gpurun --gpus N): sharded parity (persistent kernel, per-step kernels), weak-scaling and
+# round 2 multi-GPU session (one box with N GPUs): sharded parity, weak-scaling and
 # configs[3] strong-scaling timings, full bench lines.  Usage: bash scripts/r02_multi.sh N [full]
 cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
@@ -10,7 +10,7 @@ timeout 200 python bench.py --quick --steps 10 --warmup 3 2>&1 | grep -E "quick|
 timeout 200 python bench.py --quick --steps 10 --warmup 3 --workload c4 2>&1 | grep -E "quick|rror" | cut -c1-100
 run() { port=$((port + 1)); env "${@:2}" timeout "$1" python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port $port "${CMD[@]}"; }
 CMD=(tests/multigpu/check_sharded_update.py)
-for cfg in "MINPPO_PERSISTENT=0" $PARITY_EXTRA; do
+for cfg in "X=default" $PARITY_EXTRA; do
   run 400 $cfg > gpurun_out/multigpu_parity_g${N}_${cfg#*=}.log 2>&1
   echo "exit $?" >> gpurun_out/multigpu_parity_g${N}_${cfg#*=}.log
   echo "## parity at $N GPUs, $cfg"
@@ -19,12 +19,12 @@ done
 OUT=gpurun_out/multi_timing_g$N.log
 : > $OUT
 CMD=(bench.py --gpus $N --quick --steps 10 --warmup 3)
-for cfg in "MINPPO_PERSISTENT=0" "MINPPO_PX_ABLATE=2" $EXTRA_ABLATE; do
+for cfg in "X=default" $EXTRA_ABLATE; do
   echo "## weak (configs[1] per GPU) $cfg" >> $OUT
   run 300 $cfg 2>&1 | grep -E "quick|rror" | cut -c1-140 >> $OUT
 done
 CMD=(bench.py --gpus $N --quick --steps 10 --warmup 3 --workload c4)
-for cfg in "MINPPO_PERSISTENT=0" $EXTRA_ABLATE; do
+for cfg in "X=default" $EXTRA_ABLATE; do
   echo "## strong (configs[3]: 16384 x 64 global) $cfg" >> $OUT
   run 300 $cfg 2>&1 | grep -E "quick|rror" | cut -c1-140 >> $OUT
 done

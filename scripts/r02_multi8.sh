@@ -1,5 +1,5 @@
 #!/bin/bash
-# short 8-GPU session (gpurun --gpus 8): 1-GPU reference, sharded parity, weak scaling (+ exchange ablated), configs[3] strong scaling
+# short 8-GPU session (one box with 8 GPUs): 1-GPU reference, sharded parity, weak scaling, configs[3] strong scaling
 cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
 N="${1:-8}"
@@ -15,10 +15,8 @@ echo "exit $?" >> gpurun_out/multigpu_parity_g${N}.log
 echo "## parity at $N GPUs" >> $OUT
 grep -E "^\[(small|wide)|MULTIGPU|^exit|MinppoError" gpurun_out/multigpu_parity_g${N}.log | cut -c1-400 | tail -n 4 >> $OUT
 CMD=(bench.py --gpus $N --quick --steps 10 --warmup 3)
-for cfg in "X=1" "MINPPO_PX_ABLATE=2"; do
-  echo "## weak (configs[1] per GPU) $cfg" >> $OUT
-  run 300 $cfg 2>&1 | grep -E "quick|rror" | cut -c1-140 >> $OUT
-done
+echo "## weak (configs[1] per GPU)" >> $OUT
+run 300 X=1 2>&1 | grep -E "quick|rror" | cut -c1-140 >> $OUT
 CMD=(bench.py --gpus $N --quick --steps 10 --warmup 3 --workload c4)
 echo "## strong (configs[3]: 16384 x 64 global)" >> $OUT
 run 300 X=1 2>&1 | grep -E "quick|rror" | cut -c1-140 >> $OUT

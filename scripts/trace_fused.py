@@ -1,7 +1,6 @@
 """Print the cycle timeline of the fused step kernel (MINPPO_TRACE=1) for a few CTAs of the last minibatch step."""
 import os, sys
 os.environ["MINPPO_TRACE"] = "1"
-os.environ.setdefault("MINPPO_PDL", "0")     # clean per-kernel timelines
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import ctypes as C
 import numpy as np, torch
@@ -52,14 +51,6 @@ for cta in (0, 1, n // 2, n - 1):
         st = tr[cta, 128 + 32 * e:128 + 32 * e + 16] - t0
         en = tr[cta, 128 + 32 * e + 16:128 + 32 * e + 32] - t0
         print(f"  {nm:18s} window {int(en.max() - st.min()):5d}  median warp {int(np.median(en - st)):5d}  start {int(st.min())}..{int(st.max())}  end per warp {[int(x) for x in en]}")
-if os.environ.get("MINPPO_PERSISTENT", "1") != "0":
-    # persistent kernel: cta_id of the tile body is net-major, the loop stamps are in row b = blockIdx.x
-    print("--- persistent loop, last step, cycles (mean over CTAs 0..127 | max): step start -> phase A done -> barrier 1 passed -> dwopt done -> barrier 2 passed")
-    seg = [(13, 14, "phase A (fused tile)"), (14, 15, "grid barrier 1"), (15, 20, "dwopt body (GEMM + 2 barriers + reduce + Adam)"), (20, 22, "grid barrier 2")]
-    for a_, b_, name in seg:
-        d = tr[:n, b_] - tr[:n, a_]
-        print(f"  {name:48s} mean {d.mean():9.0f} min {d.min():9.0f} max {d.max():9.0f}")
-    print(f"  whole step (13 -> 22)                            mean {(tr[:n, 22] - tr[:n, 13]).mean():9.0f}")
 for e, nm in enumerate(("epilogue 1 (H1)", "epilogue 2 (H2)", "dZ2 epilogue", "epilogue 3 (dZ1)")):
     st = tr[:, 128 + 32 * e:128 + 32 * e + 16] - tr[:, 16:17]
     en = tr[:, 128 + 32 * e + 16:128 + 32 * e + 32] - tr[:, 16:17]

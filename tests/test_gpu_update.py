@@ -67,6 +67,10 @@ CASES = {
                             hidden_size=64, ent_coef=0.01), D=100, A=24),
     # 16 k-blocks of D, P = 646k: four register-resident units per optimizer thread
     "d1000": dict(hp=dict(num_envs=32, num_steps=16, num_minibatches=2, update_epochs=1, anneal_lr=False), D=1000, A=10),
+    # the same with 4 dW splits: 4 x 40 GEMM CTAs do not fit one CTA per SM (148), so every step takes the two-launch
+    # sequence (stand-alone dW GEMM, then opt_kernel) instead of the merged dwopt launch
+    "d1000_two_launch": dict(hp=dict(num_envs=32, num_steps=16, num_minibatches=2, update_epochs=1, anneal_lr=False),
+                             D=1000, A=10, cfg=dict(dw_splits=4)),
 }
 FUSED_SHAPE_CASES = ["wide", "a32_h192", "a17_h128_d600", "a24_h64", "d1000"]
 
@@ -82,7 +86,7 @@ def test_update_parity(name, cuda_device):
     case = CASES[name]
     hp = P.Hyper(**case["hp"])
     pr = synth.make_problem(hp, case["D"], case["A"], seed=7, done_p=0.02)
-    got = run_gpu_update(hp, pr, cuda_device)
+    got = run_gpu_update(hp, pr, cuda_device, **case.get("cfg", {}))
 
     p64, o64, rng64, l64, aux64 = _oracle(hp, pr, np.float64, "exact")
     pbf, obf, _, lbf, auxbf = _oracle(hp, pr, np.float32, "bf16", perms=aux64["perms"])
@@ -354,26 +358,15 @@ def test_update_rejects_bad_arguments(cuda_device):
     lrn.close()
 
 
-@pytest.mark.parametrize("name", ["medium", "wide"])
-def test_persistent_all_steps_kernel_equals_per_step_launches(name, cuda_device, monkeypatch):
-    """The optional one-launch-for-all-steps kernel (MINPPO_PERSISTENT=1: fused tile -> grid barrier -> dW GEMM + optimizer
-    -> grid barrier, per step) runs the SAME tile and optimizer bodies as the per-step launches, on a different grid (hence
-    other split-K factors and fp32 summation orders: close, not bit-identical).  Both are separately held to the oracle by
-    test_update_parity (the persistent mode when the suite is run with MINPPO_PERSISTENT=1); this test keeps the optional
-    mode from rotting.  (It is not the default: measured slower, DESIGN.md 3.6.)"""
-    case = CASES[name]
+def test_dw_grid_past_one_wave_takes_the_two_launch_path(cuda_device):
+    """d1000_two_launch really runs the fallback: one more launch per minibatch step than the automatic split-K factor,
+    whose dW grid fits one CTA per SM (S = 2: 80 CTAs) and merges the GEMM and the optimizer into one launch."""
+    case = CASES["d1000_two_launch"]
     hp = P.Hyper(**case["hp"])
-    pr = synth.make_problem(hp, case["D"], case["A"], seed=11, done_p=0.02)
-    a = run_gpu_update(hp, pr, cuda_device)
-    monkeypatch.setenv("MINPPO_PERSISTENT", "1")                 # read when the context is created
-    b = run_gpu_update(hp, pr, cuda_device)
-    monkeypatch.delenv("MINPPO_PERSISTENT")
-    assert b["launches"] < a["launches"]
-    assert np.all(np.isfinite(b["losses"])) and np.all(np.isfinite(b["params"]))
-    assert rel_err(a["losses"], b["losses"]) < 1e-3
-    assert rel_err(a["grad_norms"], b["grad_norms"]) < 1e-2
-    lr = hp.opt_lr if not hp.anneal_lr else hp.training_lr
-    assert np.abs(a["params"] - b["params"]).max() < lr * (2.0 + 0.15 * hp.update_epochs * hp.num_minibatches)
+    pr = synth.make_problem(hp, case["D"], case["A"], seed=7, done_p=0.02)
+    auto = run_gpu_update(hp, pr, cuda_device)
+    two = run_gpu_update(hp, pr, cuda_device, **case["cfg"])
+    assert two["launches"] == auto["launches"] + hp.update_epochs * hp.num_minibatches
 
 
 def test_row_list_overflow_raises_the_device_flag_and_poisons_the_losses(cuda_device, monkeypatch):
