@@ -2,20 +2,25 @@
 // (replaces jax.value_and_grad's dW contractions, optax.chain(clip_by_global_norm, adam) and
 //  TrainState.apply_gradients: /root/reference/minppo/train.py:98-124, 246-248).
 //
-// Grid = one CTA per SM, all co-resident (two grid barriers):
+// Grid = one CTA per SM, all co-resident (one grid barrier):
 //   phase 1  CTAs [0, gemm_ctas): split-K tcgen05 GEMM dW_l = act_l^T dZ_{l+1} for every hidden layer of both
-//            nets (umma_gemm_body<EPI_PARTIAL>), fp32 partial tiles -> L2 by TMA store.
+//            nets (umma_gemm_body<EPI_PARTIAL>), fp32 partial tiles -> L2 by TMA store; then each CTA counts its
+//            output tile's completion counter up (S CTAs per tile).
 //            CTAs [gemm_ctas, grid): meanwhile sum the per-tile partials of the SMALL leaves (biases, output
-//            heads, log_std: one partial per 128-row tile of the fused step kernel) and the loss sums -> gflat.
-//   barrier
+//            heads, log_std: one partial per 128-row tile of the fused step kernel) and the loss sums -> gflat,
+//            then count the small-leaf counter up.
 //   phase 2  fixed-order sum of the split-K partials of the hidden kernels -> gflat (bitwise reproducible, no
 //            atomics; 16-byte loads, 16 partials in flight per thread), sum of squares -> per-block partial.
+//            Every thread first waits for the counter(s) of the tile(s) its units lie in: it depends on the S CTAs
+//            of that tile only, not on the whole grid.
 //   barrier
 //   phase 3  clip scale, Adam, params / mu / nu in place, bf16 weight images for the next step's GEMMs.
+// The counters are reset to zero after the barrier, when every wait of the launch has been satisfied; the next
+// launch's producers run behind this launch's end (griddepcontrol.wait), so the counters need no generations.
 // The phases are plain strided loops (no per-element unrolling): an earlier fully unrolled version was
 // 15k SASS instructions and spent a third of its time on instruction-cache misses.
-// With env-sharded ranks (do_apply == 0) the kernel stops after phase 2 with the local gradient SUM in gflat;
-// the all-reduce and opt_kernel (adam.cu, apply only) follow.
+// With env-sharded ranks (do_apply == 0) the kernel stops after phase 2 and the barrier (the counter reset needs it) with
+// the local gradient SUM in gflat; the all-reduce and opt_kernel (adam.cu, apply only) follow.
 #pragma once
 
 #include "opt_common.cuh"
@@ -70,6 +75,34 @@ MINPPO_DEVINL unsigned int ld_relaxed_sys_u32(const unsigned int* p) {
   asm volatile("ld.relaxed.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
   return v;
 }
+// Split-K completion counters (DwOptParams::done), one per 128-byte line: ~2k warps poll them in phase 2, and counters
+// sharing a line would put all of that on one L2 slice.
+constexpr int DWOPT_DONE_STRIDE = 32;
+MINPPO_DEVINL void red_release_add(unsigned int* p, unsigned int v) {
+  asm volatile("red.release.gpu.global.add.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+// wait until *p >= target; bounded like grid_barrier: past the bound the error flag goes up instead of a hang
+MINPPO_DEVINL void wait_count(const unsigned int* p, unsigned int target, int* err_flag) {
+  const long long t0 = clock64();
+  for (;;) {
+    unsigned int v;
+    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    if (v >= target) break;
+    if (clock64() - t0 > 4000000000LL) { atomicExch(err_flag, MINPPO_ERR_BARRIER); break; }
+  }
+}
+// Wait until the split-K partials of the 4-element unit at element e of late leaf L are complete: the counter of the dW
+// GEMM tile that wrote them reaches S (the layer-wise path's bias leaves: every tile of the layer, each writes some columns).
+MINPPO_DEVINL void wait_late_unit(const unsigned int* done, const OptLeaf& L, int e, unsigned int S, int* err_flag) {
+  int k = L.tile0, n = L.tile_n;
+  if (L.tile_split) {                                    // hidden kernel [in][out]: column group, then 128-row m-tile
+    const int i = e / L.cols, j = e - i * L.cols;
+    k += (j >= L.tile_split ? n >> 1 : 0) + (i >> 7);
+    n = 1;
+  }
+  for (const int end = k + n; k < end; ++k) wait_count(done + k * DWOPT_DONE_STRIDE, S, err_flag);
+}
+
 // four consecutive fp32 of an arena (L2-coherent: ld.cg / plain st), by the widest access the address allows
 MINPPO_DEVINL void ld_unit(const float* p, float (&v)[4]) {
   const uintptr_t a = reinterpret_cast<uintptr_t>(p);
@@ -97,6 +130,8 @@ struct alignas(64) DwOptParams {
   OptArgs opt;                   // losses_out / gnorm_out: bases of the per-step arrays (losses_stride floats apart / 1 apart)
   int gemm_ctas;                 // CTAs [0, gemm_ctas) run the GEMM; the others pre-reduce the small leaves
   long long* trace;              // debug: [grid][16] clock64 stamps (null = off)
+  unsigned int* done;            // [1 + gemm_ctas / S][DWOPT_DONE_STRIDE] completion counters (zero at launch, reset at its end):
+                                 // [0] small-leaf CTAs done, [1 + b / S] split-K tile of GEMM CTA b: S partials stored
   // Gradient exchange over NVLink peer memory (env-sharded ranks; world == 0: not configured).  Every rank exports
   // one allocation [stage | pad | result] (PeerXchg above); base[r] is rank r's copy as mapped HERE.
   PeerXchg px;
@@ -129,7 +164,7 @@ MINPPO_DEVINL float block_sum_dyn(float v, float* scratch /*[32]*/) {
 }
 
 // MAXU = 4-element units of the hidden kernels a thread may own (fast path: reduced gradient and optimizer state stay in
-// registers across the second barrier).  MAXU = 1 covers P_late <= 4 * grid * 512 (303k parameters on 148 SMs: the
+// registers across the grid barrier).  MAXU = 1 covers P_late <= 4 * grid * 512 (303k parameters on 148 SMs: the
 // stand-in shape); larger observation widths take MAXU = 2 or 4.
 template <int MAXU>
 __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_constant__ DwOptParams p) {
@@ -152,7 +187,9 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
   DW_STAMP(0);
   __shared__ unsigned int s_seq;
   __shared__ int s_dead;                                  // error flag already up when this launch started
+  __shared__ unsigned long long s_waited;                 // trace: when this CTA's last counter wait was satisfied (clock64)
   const bool px_on = p.px.world > 1;                     // gradient exchange over peer memory fused into this launch
+  if (p.trace && t == 0) s_waited = 0ull;
   if (px_on && t == 0) {
     s_seq = __ldcg(p.px.seq) + 1u;                       // number of this exchange
     s_dead = __ldcg(a.err_flag) != 0;
@@ -168,7 +205,7 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
   DW_STAMP(14);
 
   // Per-step scalars (two powf, A exp/log): computed by the last thread, whose warp has no GEMM role, while the
-  // GEMM is in flight (GEMM CTAs) or up front (spare CTAs) -- never between the barriers, never in front of the
+  // GEMM is in flight (GEMM CTAs) or up front (spare CTAs) -- never in phase 2, never in front of the
   // CTA-wide barrier of the GEMM prologue.
   const bool scal_thread = t == NT - 1;
   int count = 0;
@@ -178,7 +215,7 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
       count = __ldcg(a.count);                           // Adam step count BEFORE this step
       step_scalars(a, count, s_bcast[1], s_bcast[2], s_bcast[3]);
       if (b == 0 && losses_out) {
-        // train.py:240 -- evaluated with the PRE-update log_std (nothing is updated before the second barrier)
+        // train.py:240 -- evaluated with the PRE-update log_std (nothing is updated before the grid barrier)
         for (int j = 0; j < a.A; ++j) ent += logf(fabsf(expf(__ldcg(a.params + a.off_logstd + j))));
       }
     }
@@ -214,13 +251,25 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
     const int live_tiles = row_count ? (max(__ldcg(row_count), 0) + p.part_rows - 1) / p.part_rows : 0x7fffffff;
     ss = reduce_leaves<false>(a, T, e * NT + t, ne * NT, live_tiles);
   }
+  // Publish this CTA's phase-1 output: one count on its tile's counter (GEMM CTAs) or on the small-leaf counter.  The GEMM's
+  // partial tile is an async-proxy (TMA) write that phase 2 reads with generic loads: the storing thread waited for it with
+  // cp.async.bulk.wait_group 0 (the writes done, not only the shared-memory reads that .read waits for) and then issued
+  // fence.proxy.async.global, which orders those writes before its later generic operations.  This CTA barrier carries them,
+  // and every other thread's plain stores (small-leaf gflat, the layer-wise path's bias column sums), to thread 0, whose
+  // release add makes all of it visible to a consumer's acquire load of the counter.  (The barrier also keeps the phase-2
+  // set-up from being scheduled into phase 1: without it the kernel spills at MAXU = 2 and 4.)
+  const unsigned int S = static_cast<unsigned int>(p.gemm.g[0].splits);
+  __syncthreads();
+  if (t == 0) red_release_add(p.done + (gemm_cta ? (1 + b / S) * DWOPT_DONE_STRIDE : 0), 1u);
   DW_STAMP(1);
-  grid_barrier(a.barrier, a.err_flag);
-  DW_STAMP(2);
+  auto wait_unit = [&](const OptLeaf& L, int e) {
+    wait_late_unit(p.done, L, e, S, a.err_flag);
+    if (p.trace) atomicMax(&s_waited, static_cast<unsigned long long>(clock64()));
+  };
 
   // ---- phase 2 ----------------------------------------------------------------------------------
   // Fast path: at most MAXU 4-element units of a hidden kernel per thread, so the reduced gradient and the optimizer
-  // state of those elements stay in registers across the second barrier and only the small leaves go through gflat.
+  // state of those elements stay in registers across the grid barrier and only the small leaves go through gflat.
   int n_units = 0;
   for (int l = 0; l < T.nleaves; ++l)
     if (T.leaf[l].late) n_units += T.size[l] >> 2;
@@ -228,7 +277,7 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
   const bool fast = n_units <= GT_ * MAXU;
   // job number of this thread for the per-element work on the SMALL leaves (reduction, exchange, Adam).  (Dealing the jobs
   // round-robin over the CTAs instead -- t * G + b -- was measured: every CTA's Adam phase then carries one more dependent
-  // load -> divide chain, 6.5k -> 12.5k cycles; concentrated on the first CTAs the chain hides behind the second barrier.)
+  // load -> divide chain, 6.5k -> 12.5k cycles; concentrated on the first CTAs the chain hides behind the grid barrier.)
   const int gtid = b * NT + t;
   float4 g4[MAXU];
   float pv[MAXU][4], mv[MAXU][4], nv[MAXU][4];
@@ -253,10 +302,12 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
         const OptLeaf& L = T.leaf[l];
         ul[u] = l; ui[u] = L.offset + 4 * x;
         if (a.do_apply) {
-          // the arena offset of a leaf is only 4-byte aligned in general (act_dim is arbitrary): widest aligned access
+          // the arena offset of a leaf is only 4-byte aligned in general (act_dim is arbitrary): widest aligned access.
+          // Issued before the counter wait: phase 1 does not write them.
           ld_unit(a.params + ui[u], pv[u]); ld_unit(a.mu + ui[u], mv[u]); ld_unit(a.nu + ui[u], nv[u]);
         }
-        g4[u] = sum_partials16_v4(L.grad_src + L.src_offset + 4 * x, L.nparts, L.part_stride);
+        wait_unit(L, 4 * x);
+        g4[u] = sum_partials16_v4<8>(L.grad_src + L.src_offset + 4 * x, L.nparts, L.part_stride);
         if (!px_on) {
           if (!a.do_apply || a.keep_gflat) { const float gq[4] = {g4[u].x, g4[u].y, g4[u].z, g4[u].w}; st_unit(a.gflat + ui[u], gq); }
           ss = fmaf(g4[u].x, g4[u].x, ss); ss = fmaf(g4[u].y, g4[u].y, ss); ss = fmaf(g4[u].z, g4[u].z, ss); ss = fmaf(g4[u].w, g4[u].w, ss);
@@ -264,9 +315,8 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
       }
     }
   } else {
-    ss += reduce_leaves<true>(a, T, gtid, GT_);
+    ss += reduce_leaves<true>(a, T, gtid, GT_, 0x7fffffff, wait_unit);
   }
-  if (!a.do_apply) return;                               // NCCL fallback: gflat = the local gradient sum; opt_kernel applies
 
   if (px_on) {
     // ---- one-shot all-reduce over NVLink peer memory (PeerXchg above; requires the fast path) -----------------
@@ -306,7 +356,14 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
     };
     const float4 sent4 = make_float4(-0.f, -0.f, -0.f, -0.f);
     float gl = 0.f;
-    if (eidx >= 0) gl = canon(__ldcg(a.gflat + eidx));
+    if (eidx >= 0) {
+      // written by the small-leaf CTAs (or, without them, by this thread in phase 2)
+      if (has_extra) {
+        wait_count(p.done, static_cast<unsigned int>(G - p.gemm_ctas), a.err_flag);
+        if (p.trace) atomicMax(&s_waited, static_cast<unsigned long long>(clock64()));
+      }
+      gl = canon(__ldcg(a.gflat + eidx));
+    }
     // TWO-PHASE (X.two_phase, used for W >= 4): the units of warp w of CTA b are reduced by rank (b + w) % W only (dealt per warp,
     // not per CTA: the owner's W - 1 polls and W - 1 result pushes per unit then spread over all SMs).  A non-owner pushes its
     // unit to the owner (one store instead of W - 1) and polls the result slot; the owner polls the W - 1 contributions,
@@ -439,11 +496,16 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
     DW_STAMP(15);
     if (b == 0 && scal_thread) *X.seq = n;
   }
-  const float bs = block_sum_dyn(ss, scratch);
+  const float bs = block_sum_dyn(ss, scratch);           // (its CTA barriers also order the s_waited updates)
   if (t == 0) a.block_ss[b] = bs;
+  // trace slot 2: this CTA's last counter wait satisfied (the end of phase 1 if it had none)
+  if (p.trace && t == 0) p.trace[static_cast<size_t>(b) * 16 + 2] = max(static_cast<long long>(s_waited), p.trace[static_cast<size_t>(b) * 16 + 1]);
   DW_STAMP(3);
   grid_barrier(a.barrier, a.err_flag);
   DW_STAMP(4);
+  // every counter wait of this launch is behind the barrier: back to zero for the next launch
+  if (b == 0 && t <= p.gemm_ctas / static_cast<int>(S)) p.done[t * DWOPT_DONE_STRIDE] = 0u;
+  if (!a.do_apply) return;                               // NCCL fallback: gflat = the local gradient sum; opt_kernel applies
 
   // ---- phase 3 ----------------------------------------------------------------------------------
   // This thread's element of the SMALL leaves (at most one when they fit one sweep of the grid): gradient and optimizer state

@@ -271,6 +271,7 @@ struct minppo_ctx {
   __nv_bfloat16* xg;           // gathered observation rows of the current minibatch [M_pad][Dp] (fused path)
   CUtensorMap m_xg_k, m_xg_mn;
   unsigned long long* barrier;
+  unsigned int* dw_done;      // dwopt_kernel's split-K tile completion counters [sm_count + 2][DWOPT_DONE_STRIDE]
   int* err_flag;
   NetBufs net[2];
   int head_stride, po_w3a, po_b3a, po_w3c, po_b3c, po_logstd, po_bh_a, po_bh_c, po_loss;
@@ -404,8 +405,7 @@ static void fill_opt_args(const minppo_ctx* c, const UpdatePtrs& u, OptArgs* o) 
     ol.offset = static_cast<int>(lf.offset);
     ol.cols = static_cast<int>(lf.cols);
     ol.grad_bias = 0.f;
-    ol.img_t = nullptr; ol.img_n = nullptr; ol.ld_t = 0; ol.ld_n = 0; ol.img_w2 = nullptr; ol.late = 0; ol.ap = 16;
-    if (lf.net == 2) {                         // log_std
+    ol.img_t = nullptr; ol.img_n = nullptr; ol.ld_t = 0; ol.ld_n = 0; ol.img_w2 = nullptr; ol.late = 0; ol.ap = 16;    if (lf.net == 2) {                         // log_std
       ol.grad_src = c->head_part; ol.src_offset = c->po_logstd; ol.nparts = c->head_parts; ol.part_stride = c->head_stride;
       ol.grad_bias = cfg.rank == 0 ? -static_cast<float>(cfg.ent_coef) : 0.f;
     } else if (lf.layer == L) {                // output heads
@@ -498,9 +498,12 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
   const int L = c->L, H = c->H;
   GemmParams& p = dp.gemm;
   int cta = 0, ng = 0;
+  int tile_first[2][4], tile_count[2][4], tile_split[2][4];   // split-K output tiles of each (net, layer): dwopt.cuh counters
   for (int net = 0; net < 2; ++net) {
     NetBufs& nb = c->net[net];
     for (int l = 0; l < L; ++l) {
+      tile_first[net][l] = cta / c->S;
+      tile_count[net][l] = 0;
       for (int nh = 0; nh < c->dw_nsplit; ++nh) {
       GemmGroup& g = p.g[ng++];
       g.cta_begin = cta;
@@ -518,12 +521,23 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
       g.ldc = H;
       g.m_tiles = (in_pad + 127) / 128; g.splits = c->S; g.m_store = in_l;
       cta += g.m_tiles * g.splits;
+      tile_count[net][l] += g.m_tiles;
+      if (nh == 0) tile_split[net][l] = g.N;
       }
     }
   }
   p.ngroups = ng;
   gemm_finalize(p);
   fill_opt_args(c, u, &dp.opt);
+  for (size_t i = 0; i < c->leaves.size(); ++i) {
+    OptLeaf& ol = dp.opt.leaf[i];
+    const LeafInfo& lf = c->leaves[i];
+    if (!ol.late) continue;                                  // hidden kernels (and, layer-wise path, hidden biases)
+    ol.tile0 = 1 + tile_first[lf.net][lf.layer];             // counter 0: the small-leaf pre-reducers
+    ol.tile_n = tile_count[lf.net][lf.layer];
+    ol.tile_split = lf.is_kernel ? tile_split[lf.net][lf.layer] : 0;
+  }
+  dp.done = c->dw_done;
   dp.opt.losses_out = u.losses_out ? u.losses_out : c->losses_scratch;
   dp.losses_stride = u.losses_out ? 4 : 0;
   dp.opt.gnorm_out = c->gnorms;
@@ -994,6 +1008,7 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   if ((rc = make_tmap(&c->m_xg_k, c->xg, c->Dp, c->M_pad, c->Dp, 64, 128))) return fail(rc);
   if ((rc = make_tmap(&c->m_xg_mn, c->xg, c->Dp, c->M_pad, c->Dp, 64, 64))) return fail(rc);
   ALLOC(c->barrier, 1);
+  ALLOC(c->dw_done, static_cast<size_t>(c->sm_count + 2) * DWOPT_DONE_STRIDE);   // zeroed: dwopt_kernel expects 0 at launch
   ALLOC(c->err_flag, 1);
   for (int net = 0; net < 2; ++net) {
     NetBufs& nb = c->net[net];

@@ -105,6 +105,10 @@ struct OptLeaf {
   int late;                      // 1: partials are written by the dW GEMM of the same launch (hidden kernels)
   int size;                      // elements of this leaf (host-computed: the kernels never walk the table serially)
   int ap;                        // img_w2: padded head width of the image (16 or 32 rows per hi / lo half)
+  // late leaves in dwopt.cuh: the completion counters of the dW GEMM tiles that write this leaf's partials
+  int tile0;                     // counter of the layer's first tile (column group 0, m-tile 0); tiles run m-tile fastest
+  int tile_n;                    // tiles of the layer (column groups x 128-row m-tiles)
+  int tile_split;                // hidden kernels: columns of column group 0; 0 (biases): an element needs every tile
 };
 struct OptArgs {
   OptLeaf leaf[MINPPO_MAX_LEAVES];

@@ -147,7 +147,10 @@ MINPPO_DEVINL float4 ld_partial_v4(const float* p) {
   asm volatile("ld.global.L1::no_allocate.L2::256B.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p) : "memory");
   return v;
 }
-// same, four consecutive elements at once (16-byte loads; src 16-byte aligned, stride % 4 == 0)
+// same, four consecutive elements at once (16-byte loads; src 16-byte aligned, stride % 4 == 0).  Below 16 partials the loads
+// go out in batches of REM (4, or 8 where the registers allow it: dwopt's S = 8 partials in one L2 round trip instead of two);
+// the summation order is the same for every REM.
+template <int REM = 4>
 MINPPO_DEVINL float4 sum_partials16_v4(const float* __restrict__ src, int nparts, size_t stride) {
   float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
   int p = 0;
@@ -158,6 +161,14 @@ MINPPO_DEVINL float4 sum_partials16_v4(const float* __restrict__ src, int nparts
     for (int u = 0; u < 16; ++u) v[u] = ld_partial_v4(src + static_cast<size_t>(p + u) * stride);
 #pragma unroll
     for (int u = 0; u < 16; ++u) { acc.x += v[u].x; acc.y += v[u].y; acc.z += v[u].z; acc.w += v[u].w; }
+  }
+#pragma unroll 1
+  for (; REM > 4 && p + REM <= nparts; p += REM) {
+    float4 v[REM];
+#pragma unroll
+    for (int u = 0; u < REM; ++u) v[u] = ld_partial_v4(src + static_cast<size_t>(p + u) * stride);
+#pragma unroll
+    for (int u = 0; u < REM; ++u) { acc.x += v[u].x; acc.y += v[u].y; acc.z += v[u].z; acc.w += v[u].w; }
   }
 #pragma unroll 1
   for (; p + 4 <= nparts; p += 4) {                      // remainders in batches of 4 loads in flight (same summation order)
@@ -182,8 +193,11 @@ MINPPO_DEVINL float4 sum_partials16_v4(const float* __restrict__ src, int nparts
 //                  elements per job (sizes and partial strides are multiples of 4, partial buffers 16-byte
 //                  aligned; gflat itself is only 4-byte aligned at a leaf offset).
 // Jobs are dealt round-robin (job = first + k * stride); the leaf walk is monotonic in k.
-template <bool LATE>
-MINPPO_DEVINL float reduce_leaves(const OptArgs& a, const LeafTab& T, int first, int stride, int max_parts = 0x7fffffff) {
+// `ready(leaf, element)` runs before the partials of a LATE job are read (dwopt.cuh: waits for the dW GEMM tile).
+struct NoWait { MINPPO_DEVINL void operator()(const OptLeaf&, int) const {} };
+template <bool LATE, typename ReadyFn = NoWait>
+MINPPO_DEVINL float reduce_leaves(const OptArgs& a, const LeafTab& T, int first, int stride, int max_parts = 0x7fffffff,
+                                  ReadyFn ready = ReadyFn()) {
   const int nl = T.nleaves;
   int l = -1, base = 0, n = 0;
   float ss = 0.f;
@@ -203,6 +217,7 @@ MINPPO_DEVINL float reduce_leaves(const OptArgs& a, const LeafTab& T, int first,
     const OptLeaf& L = T.leaf[l];
     const int x = j - base;
     if (LATE) {
+      ready(L, 4 * x);
       const float4 g = sum_partials16_v4(L.grad_src + L.src_offset + 4 * x, L.nparts, L.part_stride);
       float* dst = a.gflat + L.offset + 4 * x;
       dst[0] = g.x; dst[1] = g.y; dst[2] = g.z; dst[3] = g.w;

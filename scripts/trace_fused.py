@@ -61,15 +61,15 @@ for e, nm in enumerate(("epilogue 1 (H1)", "epilogue 2 (H2)", "dZ2 epilogue", "e
 tot = tr[:, 12] - tr[:, 16]
 print("total cycles per CTA: actor mean", tot[:n // 2].mean(), "critic mean", tot[n // 2:].mean(), "max", tot.max())
 
-# ---- dwopt kernel phases (last minibatch step): stamps 0 start, 1 phase-1 done, 2 barrier-1 passed, 3 phase-2 done,
-# 4 barrier-2 passed, 5 end
+# ---- dwopt kernel phases (last minibatch step): stamps 0 start, 1 phase-1 done, 2 the CTA's last split-K counter wait
+# satisfied (= 1 if it had none), 3 phase-2 done, 4 grid barrier passed, 5 end
 nsm = torch.cuda.get_device_properties(dev).multi_processor_count
 o2 = torch.empty((nsm, 16), dtype=torch.int64, device=dev)
 _lib.check(learner.lib.minppo_ctx_read(learner._h, 8, o2.data_ptr(), o2.numel() * 8, torch.cuda.current_stream(dev).cuda_stream))
 torch.cuda.synchronize()
 t2 = o2.cpu().numpy()
 d = t2[:, 1:6] - t2[:, 0:5]
-lab = ["phase1 (GEMM / small leaves)", "barrier 1 wait", "phase 2 (reduce)", "barrier 2 wait", "phase 3 (Adam)"]
+lab = ["phase1 (GEMM / small leaves)", "counter waits (to last)", "phase 2 (after last wait)", "grid barrier wait", "phase 3 (Adam)"]
 print("--- dwopt kernel, cycles per CTA (globaltimer-free: per-SM clock64 deltas)")
 for k in range(5):
     print(f"  {lab[k]:30s} gemm CTAs: mean {d[:128, k].mean():8.0f} min {d[:128, k].min():8.0f} max {d[:128, k].max():8.0f}"
