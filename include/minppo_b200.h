@@ -59,14 +59,14 @@ typedef struct minppo_config {
   int32_t num_layers;        /* model.num_layers   (>= 1)                             */
   int32_t use_tanh;          /* model.use_tanh     (actor only; critic is relu, train.py:82) */
   int32_t obs_dim;           /* D                                                     */
-  int32_t act_dim;           /* A (<= 32)                                             */
+  int32_t act_dim;           /* A (<= 64; > 32: layer-wise kernels)                   */
   int32_t prng_mode;         /* MINPPO_PRNG_*                                         */
   int32_t world_size;        /* G: env-sharded ranks (1 = single GPU)                 */
   int32_t rank;              /* this rank owns envs [rank*N/G, (rank+1)*N/G)          */
   int32_t fast_tanh;         /* 1: tanh.approx.f32 (MUFU) in the GEMM epilogue        */
   int32_t dw_splits;         /* split-K factor of the weight-gradient GEMMs (0 = auto) */
-  int32_t disable_fused;     /* 1: always use the layer-wise kernels (default 0: fused step kernel when L == 2 and
-                                hidden_size <= 256; wider layers always run layer-wise) */
+  int32_t disable_fused;     /* 1: always use the layer-wise kernels (default 0: fused step kernel when L == 2,
+                                hidden_size <= 256 and act_dim <= 32; wider layers or heads always run layer-wise) */
   double training_lr;        /* training.lr  (annealed path, train.py:101)            */
   double opt_lr;             /* opt.lr       (constant path, train.py:123)            */
   double max_grad_norm;      /* opt.max_grad_norm                                     */

@@ -12,6 +12,10 @@
 //
 // Rows >= count (padding of the last 128-row GEMM tile, or rows another GPU owns) produce
 // exact zeros everywhere.
+//
+// AMAX = 64 (act_dim 33..64): the whole fp32 head kernel W3a (H x 65 floats) does not fit beside the two activation
+// tiles at H > 384, so phase 1 stages it HL_KCHUNK rows at a time, and phase 3 reads each thread's row of it from the
+// arena.  Every thread accumulates the same terms in the same order as with the whole kernel resident.
 #include "common.cuh"
 #include "minppo_internal.h"
 
@@ -19,21 +23,33 @@ namespace minppo {
 
 constexpr int HL_ROWS = 64;
 constexpr int HL_THREADS = 256;
+constexpr int HL_KCHUNK = 256;          // rows of W3a per phase-1 stage (AMAX > 32)
+static_assert(HL_KCHUNK % 8 == 0, "phase 1 steps k by 8 across a quad");
 
 MINPPO_DEVINL float dclip(float x, float lo, float hi) {
   // d/dx min(max(x, lo), hi) with the 0.5/0.5 tie split of jnp.minimum / jnp.maximum
   return (x > lo && x < hi) ? 1.f : ((x == lo || x == hi) ? 0.5f : 0.f);
 }
 
+// rows [k0, k0 + rows) of the head kernel W3a -> w3a[rows][AMAX + 1], columns >= A zero
+template <int AMAX>
+MINPPO_DEVINL void hl_stage_w3a(float* w3a, const float* P, int off_w3a, int A, int k0, int rows, int tid) {
+  for (int i = tid; i < rows * AMAX; i += HL_THREADS) {
+    const int k = i / AMAX, j = i % AMAX;
+    w3a[k * (AMAX + 1) + j] = j < A ? P[off_w3a + (k0 + k) * A + j] : 0.f;
+  }
+}
+
 template <int AMAX>
 __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArgs a) {
   extern __shared__ __align__(16) uint8_t hl_smem[];
+  constexpr bool CHUNKED = AMAX > 32;
   const int H = a.H, A = a.A;
   const int HS = H + 8;                        // padded bf16 row stride
   __nv_bfloat16* hA = reinterpret_cast<__nv_bfloat16*>(hl_smem);
   __nv_bfloat16* hC = hA + HL_ROWS * HS;
-  float* w3a = reinterpret_cast<float*>(hC + HL_ROWS * HS);       // [H][AMAX+1]
-  float* w3c = w3a + H * (AMAX + 1);                              // [H]
+  float* w3a = reinterpret_cast<float*>(hC + HL_ROWS * HS);       // [H][AMAX+1]  (AMAX > 32: [HL_KCHUNK][AMAX+1])
+  float* w3c = w3a + (CHUNKED ? HL_KCHUNK : H) * (AMAX + 1);       // [H]
   float* gm = w3c + H;                                            // [64][AMAX]  g_mean
   float* gv = gm + HL_ROWS * AMAX;                                // [64]
   float* red = gv + HL_ROWS;                                      // [8][AMAX + 4] warp partials
@@ -45,9 +61,15 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
   const float* P = a.params;
 
   // ---- stage weights and the two activation tiles --------------------------------------
-  for (int i = tid; i < H * AMAX; i += HL_THREADS) {
-    const int k = i / AMAX, j = i % AMAX;
-    w3a[k * (AMAX + 1) + j] = j < A ? P[a.off_w3a + k * A + j] : 0.f;
+  // (the AMAX <= 32 loops are kept as they are rather than shared with the chunked ones: sharing them changes the
+  // compiled code of the instances every act_dim <= 32 runs)
+  if constexpr (CHUNKED) {
+    hl_stage_w3a<AMAX>(w3a, P, a.off_w3a, A, 0, min(H, HL_KCHUNK), tid);
+  } else {
+    for (int i = tid; i < H * AMAX; i += HL_THREADS) {
+      const int k = i / AMAX, j = i % AMAX;
+      w3a[k * (AMAX + 1) + j] = j < A ? P[a.off_w3a + k * A + j] : 0.f;
+    }
   }
   for (int i = tid; i < H; i += HL_THREADS) w3c[i] = P[a.off_w3c + i];
   {
@@ -68,15 +90,35 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
   float accv = 0.f;
 #pragma unroll
   for (int j = 0; j < AMAX; ++j) acc[j] = 0.f;
-  for (int k0 = part * 2; k0 < H; k0 += 8) {
-    const uint32_t wa = *reinterpret_cast<const uint32_t*>(hA + r * HS + k0);
-    const uint32_t wc = *reinterpret_cast<const uint32_t*>(hC + r * HS + k0);
-    const float a0 = bf16_lo(wa), a1 = bf16_hi(wa);
-    const float* w0 = w3a + k0 * (AMAX + 1);
-    const float* w1 = w0 + (AMAX + 1);
+  if constexpr (CHUNKED) {
+    for (int kc = 0; kc < H; kc += HL_KCHUNK) {              // the same k sequence per thread, one stage at a time
+      if (kc > 0) {
+        __syncthreads();
+        hl_stage_w3a<AMAX>(w3a, P, a.off_w3a, A, kc, min(H - kc, HL_KCHUNK), tid);
+        __syncthreads();
+      }
+      for (int k0 = kc + part * 2; k0 < min(H, kc + HL_KCHUNK); k0 += 8) {
+        const uint32_t wa = *reinterpret_cast<const uint32_t*>(hA + r * HS + k0);
+        const uint32_t wc = *reinterpret_cast<const uint32_t*>(hC + r * HS + k0);
+        const float a0 = bf16_lo(wa), a1 = bf16_hi(wa);
+        const float* w0 = w3a + (k0 - kc) * (AMAX + 1);
+        const float* w1 = w0 + (AMAX + 1);
 #pragma unroll
-    for (int j = 0; j < AMAX; ++j) acc[j] = fmaf(a1, w1[j], fmaf(a0, w0[j], acc[j]));
-    accv = fmaf(bf16_hi(wc), w3c[k0 + 1], fmaf(bf16_lo(wc), w3c[k0], accv));
+        for (int j = 0; j < AMAX; ++j) acc[j] = fmaf(a1, w1[j], fmaf(a0, w0[j], acc[j]));
+        accv = fmaf(bf16_hi(wc), w3c[k0 + 1], fmaf(bf16_lo(wc), w3c[k0], accv));
+      }
+    }
+  } else {
+    for (int k0 = part * 2; k0 < H; k0 += 8) {
+      const uint32_t wa = *reinterpret_cast<const uint32_t*>(hA + r * HS + k0);
+      const uint32_t wc = *reinterpret_cast<const uint32_t*>(hC + r * HS + k0);
+      const float a0 = bf16_lo(wa), a1 = bf16_hi(wa);
+      const float* w0 = w3a + k0 * (AMAX + 1);
+      const float* w1 = w0 + (AMAX + 1);
+#pragma unroll
+      for (int j = 0; j < AMAX; ++j) acc[j] = fmaf(a1, w1[j], fmaf(a0, w0[j], acc[j]));
+      accv = fmaf(bf16_hi(wc), w3c[k0 + 1], fmaf(bf16_lo(wc), w3c[k0], accv));
+    }
   }
 #pragma unroll
   for (int j = 0; j < AMAX; ++j) {
@@ -176,10 +218,15 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
   }
 
   // ---- phase 3: thread = hidden column c.  dZ tiles, dW3, bias grads of the last hidden layer
+  // (AMAX > 32: row c of W3a read from the arena, which stays in L2; shared memory holds only a k-chunk of it)
   for (int c = tid; c < H; c += HL_THREADS) {
     float w[AMAX], dw[AMAX];
 #pragma unroll
-    for (int j = 0; j < AMAX; ++j) { w[j] = w3a[c * (AMAX + 1) + j]; dw[j] = 0.f; }
+    for (int j = 0; j < AMAX; ++j) {
+      if constexpr (CHUNKED) w[j] = j < A ? __ldg(P + a.off_w3a + c * A + j) : 0.f;
+      else w[j] = w3a[c * (AMAX + 1) + j];
+      dw[j] = 0.f;
+    }
     const float wc = w3c[c];
     float dwc = 0.f, dba = 0.f, dbc = 0.f;
     for (int rr = 0; rr < HL_ROWS; ++rr) {
@@ -212,27 +259,36 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
   }
 }
 
-size_t head_loss_smem_bytes(int H, int amax) {
-  return static_cast<size_t>(2) * HL_ROWS * (H + 8) * 2 + static_cast<size_t>(H) * (amax + 1) * 4 + H * 4 +
+constexpr size_t head_loss_smem_bytes(int H, int amax) {
+  return static_cast<size_t>(2) * HL_ROWS * (H + 8) * 2 +
+         static_cast<size_t>(amax > 32 ? HL_KCHUNK : H) * (amax + 1) * 4 + H * 4 +
          HL_ROWS * amax * 4 + HL_ROWS * 4 + 8 * (amax + 4) * 4 + 64;
 }
+// H = 512: 212,416 bytes with the 32-wide template, 220,608 with the 64-wide one (its W3a staged in 256-row chunks):
+// above 200 KB, within the 227 KB a block may opt in to
+constexpr int HL_SMEM_OPTIN = 227 * 1024;
+static_assert(head_loss_smem_bytes(MAX_HIDDEN, 32) <= HL_SMEM_OPTIN, "head_loss_kernel<32> shared memory at H = 512");
+static_assert(head_loss_smem_bytes(MAX_HIDDEN, 64) <= HL_SMEM_OPTIN, "head_loss_kernel<64> shared memory at H = 512");
 
 int head_loss_init() {
-  // H = 512 with the 32-wide template: 212,416 bytes (above 200 KB, below the 227 KB a block may opt in to)
   const int smax = static_cast<int>(head_loss_smem_bytes(MAX_HIDDEN, 32));
   cudaError_t e = cudaFuncSetAttribute(head_loss_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(head_loss_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(head_loss_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, smax);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(head_loss_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             static_cast<int>(head_loss_smem_bytes(MAX_HIDDEN, 64)));
   return e == cudaSuccess ? 0 : MINPPO_ERR_CUDA;
 }
 
 int head_loss_launch(const HeadLossArgs& a, int tiles, cudaStream_t stream) {
-  if (a.A > 32) return MINPPO_ERR_ARG;
-  const int amax = a.A <= 8 ? 8 : (a.A <= 16 ? 16 : 32);
+  if (a.A > MAX_ACT_DIM) return MINPPO_ERR_ARG;
+  const int amax = a.A <= 8 ? 8 : (a.A <= 16 ? 16 : (a.A <= 32 ? 32 : 64));
   const size_t smem = head_loss_smem_bytes(a.H, amax);
   if (amax == 8) head_loss_kernel<8><<<tiles, HL_THREADS, smem, stream>>>(a);
   else if (amax == 16) head_loss_kernel<16><<<tiles, HL_THREADS, smem, stream>>>(a);
-  else head_loss_kernel<32><<<tiles, HL_THREADS, smem, stream>>>(a);
+  else if (amax == 32) head_loss_kernel<32><<<tiles, HL_THREADS, smem, stream>>>(a);
+  else head_loss_kernel<64><<<tiles, HL_THREADS, smem, stream>>>(a);
   return cudaGetLastError() == cudaSuccess ? 0 : MINPPO_ERR_CUDA;
 }
 

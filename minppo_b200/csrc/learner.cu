@@ -185,7 +185,10 @@ static int validate_config(const minppo_config& c) {
               c.hidden_size, GEMM_MAXN, GEMM_MAX_GROUPS / 4);
     return MINPPO_ERR_UNSUPPORTED;
   }
-  if (c.act_dim > 32) { set_error("act_dim=%d unsupported (<= 32)", c.act_dim); return MINPPO_ERR_UNSUPPORTED; }
+  if (c.act_dim > MAX_ACT_DIM) {
+    set_error("act_dim=%d unsupported (<= %d)", c.act_dim, MAX_ACT_DIM);
+    return MINPPO_ERR_UNSUPPORTED;
+  }
   if (2 * (c.num_layers + 1) * 2 + 1 > OPT_TAB_LEAVES) { set_error("too many layers"); return MINPPO_ERR_UNSUPPORTED; }
   if (2 * c.num_layers > 6) { set_error("num_layers=%d unsupported (<= 3)", c.num_layers); return MINPPO_ERR_UNSUPPORTED; }
   const long long B = static_cast<long long>(c.num_envs) * c.num_steps;
@@ -252,7 +255,7 @@ struct minppo_ctx {
                               // fused path, always when H > GEMM_MAXN)
   int hsplit;                 // column groups of the forward, dX and policy GEMMs: 1, or 2 when H > GEMM_MAXN (col_group)
   int maxu;                   // dwopt fast path: 4-element units of the hidden kernels per thread (1, 2 or 4)
-  bool fused;                 // fused step kernel (L == 2; any obs_dim, act_dim <= 32, hidden_size <= 256)
+  bool fused;                 // fused step kernel (L == 2; any obs_dim, act_dim <= FS_MAX_AP, hidden_size <= 256)
   int head_parts;             // head partials per minibatch: m_tiles (fused) or tiles64
   std::vector<LeafInfo> leaves;
   // device buffers
@@ -913,7 +916,8 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   c->cap = c->M_pad;                                  // row lists are padded to whole GEMM tiles
   c->m_tiles = c->M_pad / 128;
   c->tiles64 = c->M_pad / 64;
-  c->fused = !cfg->disable_fused && c->L == 2 && c->H <= GEMM_MAXN;
+  // wider hidden layers or heads than the fused step kernel holds run layer-wise, whatever learner.fused says
+  c->fused = !cfg->disable_fused && c->L == 2 && c->H <= GEMM_MAXN && c->A <= FS_MAX_AP;
   c->hsplit = c->H > GEMM_MAXN ? 2 : 1;
   c->ap = c->A <= 16 ? 16 : 32;
   c->store_x = c->fused;        // the fused kernel's critic CTAs store the gathered X tile (any Dp: block by block from the slots)

@@ -14,6 +14,8 @@ enum : int { ACTK_TANH = 0, ACTK_RELU = 1, ACTK_TANH_FAST = 2 };   // == ACT_* i
 
 // widest model.hidden_size: hidden layers wider than one 256-column GEMM tile run as two column groups
 constexpr int MAX_HIDDEN = 512;
+// widest act_dim: above 32 (FS_MAX_AP) the heads run on the layer-wise kernels' 64-wide templates
+constexpr int MAX_ACT_DIM = 64;
 
 // ---- gae.cu ------------------------------------------------------------------------------
 void gae_plan(int T, long long N, int sm_count, int* vec, int* chunks, int* seg_len);

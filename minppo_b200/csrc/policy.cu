@@ -116,23 +116,27 @@ __global__ void __launch_bounds__(PH_THREADS) policy_head_kernel(const PolicyHea
   if (a.log_prob) a.log_prob[row] = quad - logdet;
 }
 
-static size_t policy_head_smem(int H, int amax) { return (static_cast<size_t>(H) * (amax + 1) + H) * 4; }
+static constexpr size_t policy_head_smem(int H, int amax) { return (static_cast<size_t>(H) * (amax + 1) + H) * 4; }
+// H = 512 with the 64-wide template: 135,168 bytes
+static_assert(policy_head_smem(MAX_HIDDEN, 64) <= 200 * 1024, "policy_head_kernel<64> shared memory at H = 512");
 
 int policy_head_launch(const PolicyHeadArgs& a, cudaStream_t stream) {
-  if (a.A > 32 || a.H % 8 != 0 || a.rows <= 0) { set_error("policy head: unsupported shape"); return MINPPO_ERR_ARG; }
+  if (a.A > MAX_ACT_DIM || a.H % 8 != 0 || a.rows <= 0) { set_error("policy head: unsupported shape"); return MINPPO_ERR_ARG; }
   static bool attr_done = false;
   if (!attr_done) {
     cudaFuncSetAttribute(policy_head_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     cudaFuncSetAttribute(policy_head_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     cudaFuncSetAttribute(policy_head_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+    cudaFuncSetAttribute(policy_head_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     attr_done = true;
   }
-  const int amax = a.A <= 8 ? 8 : (a.A <= 16 ? 16 : 32);
+  const int amax = a.A <= 8 ? 8 : (a.A <= 16 ? 16 : (a.A <= 32 ? 32 : 64));
   const size_t smem = policy_head_smem(a.H, amax);
   const int blocks = (a.rows + PH_ROWS - 1) / PH_ROWS;
   if (amax == 8) policy_head_kernel<8><<<blocks, PH_THREADS, smem, stream>>>(a);
   else if (amax == 16) policy_head_kernel<16><<<blocks, PH_THREADS, smem, stream>>>(a);
-  else policy_head_kernel<32><<<blocks, PH_THREADS, smem, stream>>>(a);
+  else if (amax == 32) policy_head_kernel<32><<<blocks, PH_THREADS, smem, stream>>>(a);
+  else policy_head_kernel<64><<<blocks, PH_THREADS, smem, stream>>>(a);
   const cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { set_error("policy_head launch failed: %s", cudaGetErrorString(e)); return MINPPO_ERR_CUDA; }
   return 0;
