@@ -142,7 +142,6 @@ struct alignas(64) DwOptParams {
   int padded;                    // 1: row lists are sized for a worst case, counts[] bound the per-minibatch work
   int losses_stride;             // floats between the losses of consecutive steps (4; 0 = every step writes the scratch slot)
   int part_rows;                 // minibatch rows per early-leaf partial (128: fused step kernel, 64: head_loss kernel)
-  int prefetch;                  // 1: L2 prefetch of the next minibatch's observation rows by the GEMM CTAs' helper warps
   const __nv_bfloat16* obs_img;  // [Bl][obs_ld]
   int obs_ld;
   int step;                      // the minibatch step of this launch
@@ -176,7 +175,7 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
   const int P = a.P, step = p.step;
   const int G = static_cast<int>(gridDim.x), NT = static_cast<int>(blockDim.x);
   const int32_t* row_count = p.padded ? p.counts + step : nullptr;          // rows of this minibatch on this rank
-  const int32_t* next_ridx = (p.prefetch && step + 1 < p.EM) ? p.ridx_base + static_cast<size_t>(step + 1) * p.cap : nullptr;
+  const int32_t* next_ridx = step + 1 < p.EM ? p.ridx_base + static_cast<size_t>(step + 1) * p.cap : nullptr;
   const int32_t* next_count = p.padded ? p.counts + step + 1 : nullptr;
   float* losses_out = a.losses_out ? a.losses_out + static_cast<size_t>(step) * p.losses_stride : nullptr;
   float* gnorm_out = a.gnorm_out ? a.gnorm_out + step : nullptr;
@@ -309,7 +308,8 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
         wait_unit(L, 4 * x);
         g4[u] = sum_partials16_v4<8>(L.grad_src + L.src_offset + 4 * x, L.nparts, L.part_stride);
         if (!px_on) {
-          if (!a.do_apply || a.keep_gflat) { const float gq[4] = {g4[u].x, g4[u].y, g4[u].z, g4[u].w}; st_unit(a.gflat + ui[u], gq); }
+          const float gq[4] = {g4[u].x, g4[u].y, g4[u].z, g4[u].w};
+          st_unit(a.gflat + ui[u], gq);
           ss = fmaf(g4[u].x, g4[u].x, ss); ss = fmaf(g4[u].y, g4[u].y, ss); ss = fmaf(g4[u].z, g4[u].z, ss); ss = fmaf(g4[u].w, g4[u].w, ss);
         }
       }
@@ -446,7 +446,8 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
         g4[u] = v;
         st_sys_v4(src, sent4);
       }
-      if (a.keep_gflat) { const float gq[4] = {g4[u].x, g4[u].y, g4[u].z, g4[u].w}; st_unit(a.gflat + ui[u], gq); }
+      const float gq[4] = {g4[u].x, g4[u].y, g4[u].z, g4[u].w};
+      st_unit(a.gflat + ui[u], gq);
       ss = fmaf(g4[u].x, g4[u].x, ss); ss = fmaf(g4[u].y, g4[u].y, ss); ss = fmaf(g4[u].z, g4[u].z, ss); ss = fmaf(g4[u].w, g4[u].w, ss);
     }
     if (eidx >= 0) {

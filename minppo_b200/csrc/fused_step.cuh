@@ -95,7 +95,7 @@ struct alignas(64) FusedNet {
 struct alignas(64) FusedParams {
   FusedNet net[2];
   CUtensorMap tm_xg;             // gathered observation rows [M_pad][Dp], box {64, 128}: TMA store by the critic CTAs,
-                                 // the A operand of both nets' first-layer weight-gradient GEMM (store_x only)
+                                 // the A operand of both nets' first-layer weight-gradient GEMM
   const int32_t* rowidx;         // [E*M][cap] row lists of ALL minibatch steps of the update
   const __nv_bfloat16* obs_img;  // [Bl][Dp]
   const int32_t* count;          // [E*M]
@@ -110,7 +110,6 @@ struct alignas(64) FusedParams {
   float* part;                   // per-tile partials [m_tiles][part_stride]
   int part_stride, po_logstd;
   int H, A, Dp, m_tiles, cap;
-  int store_x;                   // 1: the critic CTAs store the gathered X tile for the dW GEMM (0: that GEMM gathers by index itself)
   int step;                      // minibatch step e * M + k of this launch
   float inv_mb, clip_eps, vf_coef;
   long long* trace;              // debug: [ctas][32] clock64 stamps (null = off)
@@ -380,7 +379,7 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
     // tensor maps into the descriptor cache first (weights: in front of the first L1 stage; stores: off any critical path)
     tma_prefetch_desc(&G.tm_w0); tma_prefetch_desc(&G.tm_w1); tma_prefetch_desc(&G.tm_w1k);
     tma_prefetch_desc(&G.tm_h1); tma_prefetch_desc(&G.tm_dz2); tma_prefetch_desc(&G.tm_dz1);
-    if (p.store_x && net == 1) tma_prefetch_desc(&p.tm_xg);
+    if (net == 1) tma_prefetch_desc(&p.tm_xg);
     for (int s = 0; s < 8; ++s) { mbar_init(&l1_full[s], 1); mbar_init(&l1_empty[s], 1); }
     for (int s = 0; s < 4; ++s) {
       mbar_init(&x_full[s], FS_NWW); mbar_init(&x_empty[s], 1); mbar_init(&x_stored[s], 1);
@@ -653,7 +652,7 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
     // for Dp > 256 the slots are refilled as the MMAs release them
     // The critic CTA (relu epilogues: the shorter chain) also TMA-stores every X k-block for the first-layer dW GEMM, straight
     // from its slot as soon as the block is complete; a slot is refilled only after that store has read it (x_stored).
-    const bool x_store_cta = p.store_x && net == 1;
+    const bool x_store_cta = net == 1;
     const bool x_store = x_store_cta && wt == 0;
     {
       int issued = nb0 + 1;                                      // cp.async groups committed so far (X blocks, then W2T)

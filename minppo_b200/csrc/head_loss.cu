@@ -7,7 +7,7 @@
 //   logp, ratio, clipped surrogate, clipped value loss              (train.py:223-239)
 //   g_mean = dL/dmean, g_v = dL/dv, dL/dlog_std                      (hand-derived; oracle/ppo_numpy.py)
 //   dZ_a = (g_mean W3a^T) * f'(h_a), dZ_c = (g_v W3c^T) * f'(h_c)   -> bf16, feeds the tcgen05 GEMMs
-//   per-tile partial sums of dW3, db3, db of the last hidden layer, dlog_std and the loss terms
+//   per-tile partial sums of dW3, db3, dlog_std and the loss terms
 // Partials are written per tile (no atomics) and reduced in fixed order by the optimizer kernel.
 //
 // Rows >= count (padding of the last 128-row GEMM tile, or rows another GPU owns) produce
@@ -64,14 +64,14 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
   // (the AMAX <= 32 loops are kept as they are rather than shared with the chunked ones: sharing them changes the
   // compiled code of the instances every act_dim <= 32 runs)
   if constexpr (CHUNKED) {
-    hl_stage_w3a<AMAX>(w3a, P, a.off_w3a, A, 0, min(H, HL_KCHUNK), tid);
+    hl_stage_w3a<AMAX>(w3a, P, a.off.w3a, A, 0, min(H, HL_KCHUNK), tid);
   } else {
     for (int i = tid; i < H * AMAX; i += HL_THREADS) {
       const int k = i / AMAX, j = i % AMAX;
-      w3a[k * (AMAX + 1) + j] = j < A ? P[a.off_w3a + k * A + j] : 0.f;
+      w3a[k * (AMAX + 1) + j] = j < A ? P[a.off.w3a + k * A + j] : 0.f;
     }
   }
-  for (int i = tid; i < H; i += HL_THREADS) w3c[i] = P[a.off_w3c + i];
+  for (int i = tid; i < H; i += HL_THREADS) w3c[i] = P[a.off.w3c + i];
   {
     const int chunks = H / 8;                                      // 16-byte chunks per row
     for (int i = tid; i < HL_ROWS * chunks; i += HL_THREADS) {
@@ -94,7 +94,7 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
     for (int kc = 0; kc < H; kc += HL_KCHUNK) {              // the same k sequence per thread, one stage at a time
       if (kc > 0) {
         __syncthreads();
-        hl_stage_w3a<AMAX>(w3a, P, a.off_w3a, A, kc, min(H - kc, HL_KCHUNK), tid);
+        hl_stage_w3a<AMAX>(w3a, P, a.off.w3a, A, kc, min(H - kc, HL_KCHUNK), tid);
         __syncthreads();
       }
       for (int k0 = kc + part * 2; k0 < min(H, kc + HL_KCHUNK); k0 += 8) {
@@ -149,9 +149,9 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
 #pragma unroll
       for (int j = 0; j < AMAX; ++j) {
         if (j < A) {
-          const float scale = expf(P[a.off_logstd + j]);
+          const float scale = expf(P[a.off.logstd + j]);
           inv_s[j] = 1.f / scale;
-          const float mean = acc[j] + P[a.off_b3a + j];
+          const float mean = acc[j] + P[a.off.b3a + j];
           z[j] = (a.action[static_cast<size_t>(src) * A + j] - mean) * inv_s[j];
           quad += -0.5f * z[j] * z[j] - 0.91893853320467274178f;
           logdet += logf(fabsf(scale));
@@ -175,7 +175,7 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
         dls[j] = g_logp * (z[j] * z[j] - 1.f);
       }
       // value loss, train.py:226-231
-      const float v = accv + P[a.off_b3c];
+      const float v = accv + P[a.off.b3c];
       const float v_old = a.v_old[src], tgt = a.tgt[src];
       const float dvv = v - v_old;
       const float v_clip = v_old + fminf(fmaxf(dvv, -a.clip_eps), a.clip_eps);
@@ -217,18 +217,18 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
     else { for (int rr = 0; rr < HL_ROWS; ++rr) s += gv[rr]; part_out[a.po_b3c] = s; }
   }
 
-  // ---- phase 3: thread = hidden column c.  dZ tiles, dW3, bias grads of the last hidden layer
+  // ---- phase 3: thread = hidden column c.  dZ tiles, dW3
   // (AMAX > 32: row c of W3a read from the arena, which stays in L2; shared memory holds only a k-chunk of it)
   for (int c = tid; c < H; c += HL_THREADS) {
     float w[AMAX], dw[AMAX];
 #pragma unroll
     for (int j = 0; j < AMAX; ++j) {
-      if constexpr (CHUNKED) w[j] = j < A ? __ldg(P + a.off_w3a + c * A + j) : 0.f;
+      if constexpr (CHUNKED) w[j] = j < A ? __ldg(P + a.off.w3a + c * A + j) : 0.f;
       else w[j] = w3a[c * (AMAX + 1) + j];
       dw[j] = 0.f;
     }
     const float wc = w3c[c];
-    float dwc = 0.f, dba = 0.f, dbc = 0.f;
+    float dwc = 0.f;
     for (int rr = 0; rr < HL_ROWS; ++rr) {
       const float ha = __bfloat162float(hA[rr * HS + c]);
       const float hc = __bfloat162float(hC[rr * HS + c]);
@@ -247,15 +247,11 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
       const __nv_bfloat16 zc = __float2bfloat16_rn(g_v * wc * fc);
       a.dz_a[static_cast<size_t>(row0 + rr) * a.ldh + c] = za;
       a.dz_c[static_cast<size_t>(row0 + rr) * a.ldh + c] = zc;
-      dba += __bfloat162float(za);
-      dbc += __bfloat162float(zc);
     }
 #pragma unroll
     for (int j = 0; j < AMAX; ++j)
       if (j < A) part_out[a.po_w3a + c * A + j] = dw[j];
     part_out[a.po_w3c + c] = dwc;
-    part_out[a.po_bh_a + c] = dba;
-    part_out[a.po_bh_c + c] = dbc;
   }
 }
 

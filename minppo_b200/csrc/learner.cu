@@ -7,8 +7,8 @@
 //     fwd  layer 0      tcgen05 GEMM, A rows gathered by index, bias+activation epilogue
 //     fwd  layer 1..L-1 tcgen05 GEMM (TMA both operands)
 //     heads + PPO loss + dZ of the last hidden layer (SIMT fp32)
-//     bwd  layer L-1..1 tcgen05 GEMM dA = dZ W^T, f' epilogue, bias-grad column sums
-//     dW   all layers   tcgen05 split-K GEMM act^T dZ -> per-split partials
+//     bwd  layer L-1..1 tcgen05 GEMM dA = dZ W^T, f' epilogue
+//     dW   all layers   tcgen05 split-K GEMM act^T dZ (+ bias-gradient column sums ones x dZ) -> per-split partials
 //     optimizer         partial reduction [+ NCCL all-reduce] + global-norm clip + Adam + bf16 images
 // The whole sequence is captured into one CUDA graph per pointer set.
 #include <cuda.h>
@@ -224,7 +224,6 @@ struct NetBufs {
   std::vector<float*> dw_part;         // dw_part[l], l = 0..L-1 [S][in_l][H]
   uint8_t* w2img;                      // head kernel^T bf16 hi / lo image (16 KB, fused path)
   std::vector<float*> dbias;           // dbias[l], l = 0..L-1 [S][H]: bias-gradient partials from the dW GEMM (ones x dz[l+1])
-  std::vector<float*> colsum;          // colsum[l],  l = 1..L-1 [m_tiles][H]  -> bias grad of layer l-1
   std::vector<CUtensorMap> m_act_k, m_act_mn, m_dz_k, m_dz_mn, m_wn_mn, m_wn, m_dw;
   std::vector<CUtensorMap> m_wn_h;     // m_wn_h[l]: box {64 out, 32 in} -- half-k-block stages of the fused step kernel (MN-major B)
   CUtensorMap m_w1k_h;                 // wn[1]: box {64 out, H/2 in} -- (k-block, N half) stages of the fused kernel's dH1 GEMM (K-major B)
@@ -277,10 +276,10 @@ struct minppo_ctx {
   unsigned int* dw_done;      // dwopt_kernel's split-K tile completion counters [sm_count + 2][DWOPT_DONE_STRIDE]
   int* err_flag;
   NetBufs net[2];
-  int head_stride, po_w3a, po_b3a, po_w3c, po_b3c, po_logstd, po_bh_a, po_bh_c, po_loss;
+  int head_stride, po_w3a, po_b3a, po_w3c, po_b3c, po_logstd, po_loss;
   int po_db[2][2];            // fused path: [net][layer] hidden-bias gradient partials (column sums of dZ), H floats each
   int ap;                     // padded head width of the fused step kernel: 16 (A <= 16) or 32
-  bool store_x;               // fused path: the fused kernel stores the gathered X tile for the first-layer dW GEMM
+  HeadOffsets head;           // arena offsets of the output-head leaves
   int opt_blocks;
   // graph cache
   cudaStream_t cap_stream;
@@ -379,6 +378,7 @@ static int init_kernel_attrs() {
   CK(cudaFuncSetAttribute(umma_gemm_kernel<EPI_DACT>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
   CK(cudaFuncSetAttribute(umma_gemm_kernel<EPI_PARTIAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
   if (head_loss_init()) { set_error("head_loss_init failed"); return MINPPO_ERR_CUDA; }
+  if (policy_head_init()) { set_error("policy_head_init failed"); return MINPPO_ERR_CUDA; }
   CK(cudaFuncSetAttribute(fused_step_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, FsLayout<16>::BYTES));
   CK(cudaFuncSetAttribute(fused_step_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, FsLayout<32>::BYTES));
   CK(cudaFuncSetAttribute(dwopt_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, GEMM_SMEM_BYTES));
@@ -407,8 +407,7 @@ static void fill_opt_args(const minppo_ctx* c, const UpdatePtrs& u, OptArgs* o) 
     OptLeaf& ol = o->leaf[n++];
     ol.offset = static_cast<int>(lf.offset);
     ol.cols = static_cast<int>(lf.cols);
-    ol.grad_bias = 0.f;
-    ol.img_t = nullptr; ol.img_n = nullptr; ol.ld_t = 0; ol.ld_n = 0; ol.img_w2 = nullptr; ol.late = 0; ol.ap = 16;    if (lf.net == 2) {                         // log_std
+    if (lf.net == 2) {                         // log_std
       ol.grad_src = c->head_part; ol.src_offset = c->po_logstd; ol.nparts = c->head_parts; ol.part_stride = c->head_stride;
       ol.grad_bias = cfg.rank == 0 ? -static_cast<float>(cfg.ent_coef) : 0.f;
     } else if (lf.layer == L) {                // output heads
@@ -418,7 +417,7 @@ static void fill_opt_args(const minppo_ctx* c, const UpdatePtrs& u, OptArgs* o) 
     } else if (lf.is_kernel) {                 // hidden kernels: split-K partials of the dW GEMM
       const int in_l = lf.layer == 0 ? c->D : H;
       ol.grad_src = c->net[lf.net].dw_part[lf.layer]; ol.src_offset = 0; ol.nparts = c->S; ol.part_stride = in_l * H; ol.late = 1;
-      ol.img_n = c->net[lf.net].wn[lf.layer]; ol.ld_n = H;
+      ol.img_n = c->net[lf.net].wn[lf.layer];
     } else if (c->fused) {                     // hidden biases, fused path: per-tile column sums of dz[l+1] from the fused step kernel
       ol.grad_src = c->head_part; ol.src_offset = c->po_db[lf.net][lf.layer]; ol.nparts = c->head_parts; ol.part_stride = c->head_stride;
     } else {                                   // hidden biases: column sums of dz[l+1], computed by the dW GEMM (ones x dz)
@@ -432,14 +431,13 @@ static void fill_opt_args(const minppo_ctx* c, const UpdatePtrs& u, OptArgs* o) 
     o->leaf[i].size = (i + 1 < n ? o->leaf[i + 1].offset : static_cast<int>(c->P)) - o->leaf[i].offset;
     if (!o->leaf[i].late) o->n_early += o->leaf[i].size;
   }
-  o->keep_gflat = 1;                         // minppo_ctx_read(what=3) returns the last reduced gradient
   o->P = static_cast<int>(c->P);
   o->A = c->A;
   o->gflat = c->gflat;
   o->loss_src = c->head_part; o->loss_src_offset = c->po_loss; o->loss_nparts = c->head_parts; o->loss_part_stride = c->head_stride;
   o->params = u.params; o->mu = u.mu; o->nu = u.nu; o->count = u.count;
   o->block_ss = c->block_ss; o->barrier = c->barrier; o->err_flag = c->err_flag;
-  o->off_logstd = static_cast<int>(c->leaves.back().offset);
+  o->off_logstd = c->head.logstd;
   o->anneal = cfg.anneal_lr ? 1 : 0;
   o->anneal_div = c->mb * c->E;                                                     // train.py:100
   const long long nu = cfg.total_timesteps / cfg.num_steps / cfg.num_envs;          // train.py:93
@@ -474,7 +472,7 @@ static void fill_fused_params(minppo_ctx* c, const UpdatePtrs& u, FusedParams* p
     g.b0 = u.params + find_leaf(c, net, 0, 0).offset;
     g.b1 = u.params + find_leaf(c, net, 1, 0).offset;
     g.w2img = reinterpret_cast<const uint4*>(nb.w2img);
-    g.b2 = u.params + find_leaf(c, net, 2, 0).offset;
+    g.b2 = u.params + (net == 0 ? c->head.b3a : c->head.b3c);
     g.act = act_kind(c, net);
     g.aout = net == 0 ? c->A : 1;
     g.po_w2 = net == 0 ? c->po_w3a : c->po_w3c;
@@ -483,10 +481,10 @@ static void fill_fused_params(minppo_ctx* c, const UpdatePtrs& u, FusedParams* p
     g.po_db0 = c->po_db[net][0]; g.po_db1 = c->po_db[net][1];
   }
   p.rowidx = c->rowidx; p.obs_img = c->obs_img; p.count = c->counts; p.step = 0;
-  p.tm_xg = c->m_xg_k; p.store_x = c->store_x ? 1 : 0;
+  p.tm_xg = c->m_xg_k;
   p.adv_sum = c->stats; p.adv_sq = c->stats + c->E * c->M;
   p.action = u.action; p.v_old = u.value; p.logp_old = u.log_prob; p.adv = c->adv; p.tgt = c->tgt;
-  p.log_std = u.params + c->leaves.back().offset;
+  p.log_std = u.params + c->head.logstd;
   p.part = c->head_part; p.part_stride = c->head_stride; p.po_logstd = c->po_logstd;
   p.H = H; p.A = c->A; p.Dp = c->Dp; p.m_tiles = c->m_tiles; p.cap = c->cap;
   p.inv_mb = static_cast<float>(1.0 / c->mb);
@@ -512,7 +510,7 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
       g.cta_begin = cta;
       const int in_l = l == 0 ? c->D : H;
       const int in_pad = l == 0 ? c->Dp : H;
-      if (l == 0 && c->fused && c->store_x) { g.amode = A_TMA_MN; g.tmA = c->m_xg_mn; }   // rows gathered by the fused kernel
+      if (l == 0 && c->fused) { g.amode = A_TMA_MN; g.tmA = c->m_xg_mn; }   // rows gathered by the fused kernel
       else if (l == 0) { g.amode = A_GATHER_MN; g.rowidx = c->rowidx; g.gimage = c->obs_img; g.ldg = c->Dp; }      // row list: per step
       else { g.amode = A_TMA_MN; g.tmA = nb.m_act_mn[l]; }
       g.bmode = B_TMA_MN; g.tmB = nb.m_dz_mn[l + 1];
@@ -548,9 +546,51 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
   dp.ridx_base = c->rowidx; dp.counts = c->counts; dp.cap = c->cap; dp.EM = c->E * c->M;
   dp.padded = c->padded ? 1 : 0;
   dp.part_rows = c->fused ? 128 : 64;
-  dp.prefetch = 1; dp.obs_img = c->obs_img; dp.obs_ld = c->Dp;
+  dp.obs_img = c->obs_img; dp.obs_ld = c->Dp;
   dp.trace = c->trace_on ? c->trace2 : nullptr;
   return cta;
+}
+
+// One net's operands in the forward GEMM of one hidden layer
+struct FwdOperands {
+  const int32_t* rowidx;        // A gathered by index from the observation image (layer 0 of a minibatch), or null:
+  const CUtensorMap* a_map;     //   A through this K-major map [rows][in]
+  __nv_bfloat16* out;           // [m_tiles * 128][H]
+};
+// Forward GEMM of hidden layer l, out = f(A W_l + b_l), for nets first_net..1 (the critic-only bootstrap value starts at
+// net 1): one group per (net, column group) over m_tiles 128-row tiles.
+static void fill_forward_gemm(const minppo_ctx* c, int l, const float* params, int first_net, int m_tiles,
+                              const FwdOperands (&op)[2], GemmParams* pp) {
+  GemmParams& p = *pp;
+  memset(&p, 0, sizeof(p));
+  const int H = c->H;
+  int ng = 0;
+  for (int i = first_net * c->hsplit; i < 2 * c->hsplit; ++i, ++ng) {
+    const int net = i / c->hsplit;
+    GemmGroup& g = p.g[ng];
+    g.cta_begin = ng * m_tiles;
+    col_group(H, c->hsplit, i % c->hsplit, &g.n_off, &g.N);
+    g.bmode = B_TMA_MN;                   // kernel image as stored [in = k][out = n]
+    g.tmB = c->net[net].m_wn_mn[l];
+    if (op[net].rowidx) { g.amode = A_GATHER_K; g.rowidx = op[net].rowidx; g.gimage = c->obs_img; g.ldg = c->Dp; }
+    else { g.amode = A_TMA_K; g.tmA = *op[net].a_map; }
+    g.kb_total = (l == 0 ? c->Dp : H) / 64;
+    g.out = op[net].out; g.ldo = H;
+    g.bias = params + find_leaf(c, net, l, 0).offset;
+    g.act = act_kind(c, net);
+    g.m_tiles = m_tiles; g.splits = 1; g.m_store = m_tiles * 128;
+  }
+  p.ngroups = ng;
+}
+
+// bf16 weight images of the fp32 arena `params` (what the GEMMs and the fused kernels read)
+static int enqueue_weight_images(const minppo_ctx* c, const float* params, cudaStream_t stream) {
+  UpdatePtrs u;
+  memset(&u, 0, sizeof(u));
+  u.params = const_cast<float*>(params);               // weight_images only reads the arena
+  OptArgs o;
+  fill_opt_args(c, u, &o);
+  return weight_images_launch(o, stream);
 }
 
 // ---- one minibatch step --------------------------------------------------------------------
@@ -573,27 +613,11 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
   } else {
   // forward
   for (int l = 0; l < L; ++l) {
+    FwdOperands op[2];
+    for (int net = 0; net < 2; ++net)
+      op[net] = {l == 0 ? ridx : nullptr, &c->net[net].m_act_k[l], c->net[net].act[l + 1]};
     GemmParams p;
-    memset(&p, 0, sizeof(p));
-    p.ngroups = 2 * c->hsplit;
-    for (int i = 0; i < p.ngroups; ++i) {
-      const int net = i / c->hsplit;
-      GemmGroup& g = p.g[i];
-      NetBufs& nb = c->net[net];
-      g.cta_begin = i * c->m_tiles;
-      col_group(H, c->hsplit, i % c->hsplit, &g.n_off, &g.N);
-      g.bmode = B_TMA_MN;                 // kernel image as stored [in = k][out = n]
-      g.tmB = nb.m_wn_mn[l];
-      if (l == 0) {
-        g.amode = A_GATHER_K; g.rowidx = ridx; g.gimage = c->obs_img; g.ldg = c->Dp; g.kb_total = c->Dp / 64;
-      } else {
-        g.amode = A_TMA_K; g.tmA = nb.m_act_k[l]; g.kb_total = H / 64;
-      }
-      g.out = nb.act[l + 1]; g.ldo = H;
-      g.bias = u.params + find_leaf(c, net, l, 0).offset;
-      g.act = act_kind(c, net);
-      g.m_tiles = c->m_tiles; g.splits = 1; g.m_store = c->M_pad;
-    }
+    fill_forward_gemm(c, l, u.params, 0, c->m_tiles, op, &p);
     PROF(PC_FWD_GEMM);
     RET(launch_gemm<EPI_ACT>(p, p.ngroups * c->m_tiles, stream));
     c->launches++;
@@ -609,10 +633,8 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
     a.action = u.action; a.v_old = u.value; a.logp_old = u.log_prob; a.adv = c->adv; a.tgt = c->tgt;
     a.partials = c->head_part; a.partial_stride = c->head_stride;
     a.po_w3a = c->po_w3a; a.po_b3a = c->po_b3a; a.po_w3c = c->po_w3c; a.po_b3c = c->po_b3c;
-    a.po_logstd = c->po_logstd; a.po_bh_a = c->po_bh_a; a.po_bh_c = c->po_bh_c; a.po_loss = c->po_loss;
-    a.off_w3a = static_cast<int>(find_leaf(c, 0, L, 1).offset); a.off_b3a = static_cast<int>(find_leaf(c, 0, L, 0).offset);
-    a.off_w3c = static_cast<int>(find_leaf(c, 1, L, 1).offset); a.off_b3c = static_cast<int>(find_leaf(c, 1, L, 0).offset);
-    a.off_logstd = static_cast<int>(c->leaves.back().offset);
+    a.po_logstd = c->po_logstd; a.po_loss = c->po_loss;
+    a.off = c->head;
     a.H = H; a.A = c->A; a.ldh = H; a.cap = c->cap;
     a.act_a = act_kind(c, 0) == ACT_RELU ? ACTK_RELU : ACTK_TANH; a.act_c = ACTK_RELU;
     a.inv_mb = static_cast<float>(1.0 / c->mb);
@@ -637,7 +659,6 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
       g.kb_total = H / 64;
       g.out = nb.dz[l]; g.ldo = H;
       g.hprev = nb.act[l]; g.ldh = H;
-      g.colsum = nb.colsum[l]; g.ldc = H;
       g.act = act_kind(c, net);
       g.m_tiles = c->m_tiles; g.splits = 1; g.m_store = c->M_pad;
     }
@@ -719,9 +740,7 @@ static int enqueue_update(minppo_ctx* c, const UpdatePtrs& u, cudaStream_t strea
     CK(cudaEventRecord(c->ev_fork, stream));
     CK(cudaStreamWaitEvent(c->side_stream, c->ev_fork, 0));
     RET(obs_image_launch(u.obs, c->obs_img, c->Bl, c->D, c->Dp, c->side_stream));
-    OptArgs o;
-    fill_opt_args(c, u, &o);
-    RET(weight_images_launch(o, c->side_stream));
+    RET(enqueue_weight_images(c, u.params, c->side_stream));
     CK(cudaEventRecord(c->ev_join, c->side_stream));
     c->launches += 2;
   }
@@ -774,10 +793,8 @@ static int enqueue_update(minppo_ctx* c, const UpdatePtrs& u, cudaStream_t strea
     }
     // the weight images must match the caller's params at entry (they may have been replaced)
     {
-      OptArgs o;
-      fill_opt_args(c, u, &o);
       PROF(PC_WEIGHT_IMAGES);
-      RET(weight_images_launch(o, stream));
+      RET(enqueue_weight_images(c, u.params, stream));
       c->launches++;
     }
   }
@@ -920,9 +937,13 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   c->fused = !cfg->disable_fused && c->L == 2 && c->H <= GEMM_MAXN && c->A <= FS_MAX_AP;
   c->hsplit = c->H > GEMM_MAXN ? 2 : 1;
   c->ap = c->A <= 16 ? 16 : 32;
-  c->store_x = c->fused;        // the fused kernel's critic CTAs store the gathered X tile (any Dp: block by block from the slots)
   c->head_parts = c->fused ? c->m_tiles : c->tiles64;
   c->P = build_layout(*cfg, &c->leaves);
+  c->head.w3a = static_cast<int>(find_leaf(c, 0, c->L, 1).offset);
+  c->head.b3a = static_cast<int>(find_leaf(c, 0, c->L, 0).offset);
+  c->head.w3c = static_cast<int>(find_leaf(c, 1, c->L, 1).offset);
+  c->head.b3c = static_cast<int>(find_leaf(c, 1, c->L, 0).offset);
+  c->head.logstd = static_cast<int>(c->leaves.back().offset);
   c->maxu = c->P <= dwopt_fast_capacity(c->sm_count, 1) ? 1 : (c->P <= dwopt_fast_capacity(c->sm_count, 2) ? 2 : 4);
   // split-K of the dW GEMMs: fill the SMs once
   {
@@ -932,7 +953,7 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
     // their observation rows by index (A_GATHER_MN), so every row is gathered once per column group: twice the
     // observation-image reads of that layer's A operand.
     c->dw_nsplit = c->H > GEMM_MAXN ? 2
-                 : (c->fused && c->store_x && c->H % 128 == 0 && 2 * 2 * c->L <= GEMM_MAX_GROUPS) ? 2 : 1;
+                 : (c->fused && c->H % 128 == 0 && 2 * 2 * c->L <= GEMM_MAX_GROUPS) ? 2 : 1;
     int per_split = 0;
     for (int l = 0; l < c->L; ++l) per_split += 2 * c->dw_nsplit * (((l == 0 ? c->Dp : c->H) + 127) / 128);
     // leave ~16 of the one-CTA-per-SM grid as spare CTAs: they sum the per-tile partials of the small leaves while the GEMM
@@ -968,8 +989,6 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
     c->po_w3c = o; o += H;
     c->po_b3c = o; o += 1;
     c->po_logstd = o; o += A;
-    c->po_bh_a = o; o += H;
-    c->po_bh_c = o; o += H;
     for (int net = 0; net < 2; ++net)
       for (int l = 0; l < 2; ++l) { c->po_db[net][l] = o; o += H; }
     c->po_loss = o; o += 2;
@@ -1017,7 +1036,7 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   for (int net = 0; net < 2; ++net) {
     NetBufs& nb = c->net[net];
     nb.act.assign(L + 1, nullptr); nb.dz.assign(L + 1, nullptr); nb.wn.assign(L, nullptr);
-    nb.dw_part.assign(L, nullptr); nb.colsum.assign(L, nullptr); nb.dbias.assign(L, nullptr);
+    nb.dw_part.assign(L, nullptr); nb.dbias.assign(L, nullptr);
     ALLOC(nb.w2img, static_cast<size_t>(H) * FS_MAX_AP * 4);       // H/64 panels of [2 AP rows][128 B]
     nb.m_act_k.resize(L + 1); nb.m_act_mn.resize(L + 1); nb.m_dz_k.resize(L + 1); nb.m_dz_mn.resize(L + 1);
     nb.m_wn_mn.resize(L); nb.m_wn.resize(2 * L); nb.m_dw.resize(L); nb.m_wn_h.resize(L);
@@ -1042,7 +1061,6 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
           col_group(H, c->hsplit, j, &n_off, &n);
           if ((rc = make_tmap(&nb.m_wn[2 * l + j], nb.wn[l], H, H, H, 64, n))) return fail(rc);
         }
-        ALLOC(nb.colsum[l], static_cast<size_t>(c->m_tiles) * H);
       }
       ALLOC(nb.dw_part[l], static_cast<size_t>(c->S) * in_l * H);
       ALLOC(nb.dbias[l], static_cast<size_t>(c->S) * H);
@@ -1143,16 +1161,9 @@ int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, con
   if (!actor && !value) { set_error("minppo_policy_step: no output requested"); return MINPPO_ERR_ARG; }
   cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
   const int L = c->L, H = c->H;
+  if (!(flags & MINPPO_POLICY_WEIGHTS_CURRENT)) RET(enqueue_weight_images(c, params, stream));
   if (c->fused) {
     // 2-hidden-layer nets: ONE launch (policy_fused.cuh) -- observation conversion, both hidden layers, heads, sampler
-    if (!(flags & MINPPO_POLICY_WEIGHTS_CURRENT)) {
-      UpdatePtrs u;
-      memset(&u, 0, sizeof(u));
-      u.params = const_cast<float*>(params);               // weight_images only reads the arena
-      OptArgs o;
-      fill_opt_args(c, u, &o);
-      RET(weight_images_launch(o, stream));
-    }
     PolicyParams pp;
     memset(&pp, 0, sizeof(pp));
     for (int net = 0; net < 2; ++net) {
@@ -1162,11 +1173,11 @@ int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, con
       g.b0 = params + find_leaf(c, net, 0, 0).offset;
       g.b1 = params + find_leaf(c, net, 1, 0).offset;
       g.w2img = reinterpret_cast<const uint4*>(nb.w2img);
-      g.b2 = params + find_leaf(c, net, 2, 0).offset;
+      g.b2 = params + (net == 0 ? c->head.b3a : c->head.b3c);
       g.act = act_kind(c, net);
       g.aout = net == 0 ? c->A : 1;
     }
-    pp.obs = obs; pp.log_std = params + c->leaves.back().offset;
+    pp.obs = obs; pp.log_std = params + c->head.logstd;
     pp.key_in = actor ? key_in : nullptr; pp.key_out = actor ? key_out : nullptr;
     pp.action = action; pp.log_prob = log_prob; pp.value = value; pp.mean_out = mean;
     pp.n0 = c->n0; pp.n_total = static_cast<long long>(c->N) * c->A;
@@ -1178,45 +1189,21 @@ int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, con
   }
   // bf16 image of last_obs, zero padded to Dp columns (rows >= Nl of the image stay zero from allocation)
   RET(obs_image_launch(obs, c->pol_img, c->Nl, c->D, c->Dp, stream));
-  if (!(flags & MINPPO_POLICY_WEIGHTS_CURRENT)) {
-    UpdatePtrs u;
-    memset(&u, 0, sizeof(u));
-    u.params = const_cast<float*>(params);               // weight_images only reads the arena
-    OptArgs o;
-    fill_opt_args(c, u, &o);
-    RET(weight_images_launch(o, stream));
-  }
   const int first = actor ? 0 : 1;                        // critic only: the bootstrap value (train.py:182-183)
   for (int l = 0; l < L; ++l) {
+    FwdOperands op[2];
+    for (int net = 0; net < 2; ++net)
+      op[net] = {nullptr, l == 0 ? &c->m_pol_img_k : &c->m_pol_act_k[net][l], c->pol_act[net][l + 1]};
     GemmParams p;
-    memset(&p, 0, sizeof(p));
-    int ng = 0;
-    for (int i = first * c->hsplit; i < 2 * c->hsplit; ++i) {
-      const int net = i / c->hsplit;
-      GemmGroup& g = p.g[ng];
-      g.cta_begin = ng * c->pol_tiles;
-      ++ng;
-      col_group(H, c->hsplit, i % c->hsplit, &g.n_off, &g.N);
-      g.bmode = B_TMA_MN; g.tmB = c->net[net].m_wn_mn[l];
-      g.amode = A_TMA_K;
-      if (l == 0) { g.tmA = c->m_pol_img_k; g.kb_total = c->Dp / 64; }
-      else { g.tmA = c->m_pol_act_k[net][l]; g.kb_total = H / 64; }
-      g.out = c->pol_act[net][l + 1]; g.ldo = H;
-      g.bias = params + find_leaf(c, net, l, 0).offset;
-      g.act = act_kind(c, net);
-      g.m_tiles = c->pol_tiles; g.splits = 1; g.m_store = c->pol_tiles * 128;
-    }
-    p.ngroups = ng;
-    RET(launch_gemm<EPI_ACT>(p, ng * c->pol_tiles, stream));
+    fill_forward_gemm(c, l, params, first, c->pol_tiles, op, &p);
+    RET(launch_gemm<EPI_ACT>(p, p.ngroups * c->pol_tiles, stream));
   }
   PolicyHeadArgs a;
   memset(&a, 0, sizeof(a));
   a.h_a = actor ? c->pol_act[0][L] : nullptr;
   a.h_c = c->pol_act[1][L];
   a.params = params;
-  a.off_w3a = static_cast<int>(find_leaf(c, 0, L, 1).offset); a.off_b3a = static_cast<int>(find_leaf(c, 0, L, 0).offset);
-  a.off_w3c = static_cast<int>(find_leaf(c, 1, L, 1).offset); a.off_b3c = static_cast<int>(find_leaf(c, 1, L, 0).offset);
-  a.off_logstd = static_cast<int>(c->leaves.back().offset);
+  a.off = c->head;
   a.H = H; a.A = c->A; a.ldh = H; a.rows = c->Nl;
   a.n0 = c->n0; a.n_total = static_cast<long long>(c->N) * c->A;
   a.key_in = actor ? key_in : nullptr; a.key_out = actor ? key_out : nullptr; a.mode = c->cfg.prng_mode;

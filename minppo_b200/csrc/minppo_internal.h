@@ -42,6 +42,11 @@ int compact_rows_launch(const int32_t* perms, int32_t* rowidx, int32_t* counts, 
 int adv_stats_launch(const float* adv, const int32_t* rowidx, const int32_t* counts, float* stats, int EM, int cap,
                      int mb, int pass, cudaStream_t stream);
 
+// arena offsets of the output-head leaves (kernel and bias of each net's head, log_std)
+struct HeadOffsets {
+  int w3a, b3a, w3c, b3c, logstd;
+};
+
 // ---- head_loss.cu ------------------------------------------------------------------------
 struct HeadLossArgs {
   const __nv_bfloat16* h_a;      // last hidden activation, actor  [M_pad][ldh]
@@ -60,8 +65,8 @@ struct HeadLossArgs {
   const float* tgt;              // [Bl]
   float* partials;               // [tiles][partial_stride]
   int partial_stride;
-  int po_w3a, po_b3a, po_w3c, po_b3c, po_logstd, po_bh_a, po_bh_c, po_loss;   // offsets inside a partial
-  int off_w3a, off_b3a, off_w3c, off_b3c, off_logstd;                          // offsets inside the arena
+  int po_w3a, po_b3a, po_w3c, po_b3c, po_logstd, po_loss;   // offsets inside a partial
+  HeadOffsets off;                                            // offsets inside the arena
   int H, A, ldh, cap;
   int act_a, act_c;              // ACTK_* of the hidden layers
   float inv_mb, clip_eps, vf_coef;
@@ -74,7 +79,7 @@ struct PolicyHeadArgs {
   const __nv_bfloat16* h_a;      // last hidden activation, actor  [rows_pad][ldh]; null = critic only (bootstrap value)
   const __nv_bfloat16* h_c;      // last hidden activation, critic [rows_pad][ldh]
   const float* params;           // fp32 arena
-  int off_w3a, off_b3a, off_w3c, off_b3c, off_logstd;
+  HeadOffsets off;
   int H, A, ldh;
   int rows;                      // env rows of this rank
   long long n0;                  // first GLOBAL env index of this rank
@@ -87,6 +92,7 @@ struct PolicyHeadArgs {
   float* value;                  // [rows] or null
   float* mean_out;               // [rows][A] or null
 };
+int policy_head_init();
 int policy_head_launch(const PolicyHeadArgs& a, cudaStream_t stream);
 
 // ---- adam.cu -----------------------------------------------------------------------------
@@ -98,10 +104,8 @@ struct OptLeaf {
   int nparts;                    // partials to sum (fixed order)
   int part_stride;               // floats between consecutive partials
   float grad_bias;               // constant added to every element (-ent_coef for log_std)
-  __nv_bfloat16* img_t;          // unused (was: transposed image); kept null
-  __nv_bfloat16* img_n;          // bf16 image [in][ld_n] of a hidden kernel, ld_n == cols (the B operand of the
-                                 // forward GEMMs as MN-major and of the dX GEMMs as K-major), or null
-  int ld_t, ld_n;
+  __nv_bfloat16* img_n;          // bf16 image [in][cols] of a hidden kernel (the B operand of the forward GEMMs as MN-major
+                                 // and of the dX GEMMs as K-major), or null
   uint8_t* img_w2;               // output-head kernels: 16 KB bf16 hi / lo image of kernel^T in the fused kernel's
                                  // shared-memory layout (fused_step.cuh FS_W2T), or null
   int late;                      // 1: partials are written by the dW GEMM of the same launch (hidden kernels)
@@ -117,8 +121,7 @@ struct OptArgs {
   int nleaves, P, A;
   int n_early;                   // elements of the leaves with late == 0
   int do_reduce, do_apply;
-  int keep_gflat;                // also store the reduced gradient when reduce+apply are fused (tests)
-  float* gflat;                  // [P + 4]
+  float* gflat;                  // [P + 4] reduced gradient (minppo_ctx_read buffer 3 returns the last one), then the loss sums
   const float* loss_src;         // loss partial sums (2 per partial)
   int loss_src_offset, loss_nparts, loss_part_stride;
   float* params; float* mu; float* nu;

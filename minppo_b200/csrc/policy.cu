@@ -37,10 +37,10 @@ __global__ void __launch_bounds__(PH_THREADS) policy_head_kernel(const PolicyHea
   if (actor) {
     for (int i = tid; i < H * AMAX; i += PH_THREADS) {
       const int k = i / AMAX, j = i % AMAX;
-      w3a[k * (AMAX + 1) + j] = j < A ? P[a.off_w3a + k * A + j] : 0.f;
+      w3a[k * (AMAX + 1) + j] = j < A ? P[a.off.w3a + k * A + j] : 0.f;
     }
   }
-  for (int i = tid; i < H; i += PH_THREADS) w3c[i] = P[a.off_w3c + i];
+  for (int i = tid; i < H; i += PH_THREADS) w3c[i] = P[a.off.w3c + i];
   if (tid == 0 && a.key_in) {
     const uint32_t k[2] = {a.key_in[0], a.key_in[1]};
     uint32_t r[2], s[2];
@@ -91,7 +91,7 @@ __global__ void __launch_bounds__(PH_THREADS) policy_head_kernel(const PolicyHea
   accv += __shfl_xor_sync(0xffffffffu, accv, 2);
   if (!live || part != 0) return;
 
-  if (a.value) a.value[row] = accv + P[a.off_b3c];
+  if (a.value) a.value[row] = accv + P[a.off.b3c];
   if (!actor) return;
   const uint32_t akey[2] = {s_key[2], s_key[3]};
   const uint32_t gbase = static_cast<uint32_t>((a.n0 + row) * A);           // flat index of eps[n][0] in the global draw
@@ -99,10 +99,10 @@ __global__ void __launch_bounds__(PH_THREADS) policy_head_kernel(const PolicyHea
 #pragma unroll
   for (int j = 0; j < AMAX; ++j) {
     if (j < A) {
-      const float mean = acc[j] + P[a.off_b3a + j];
+      const float mean = acc[j] + P[a.off.b3a + j];
       float act = mean;
       if (a.mean_out) a.mean_out[static_cast<size_t>(row) * A + j] = mean;
-      const float scale = expf(P[a.off_logstd + j]);
+      const float scale = expf(P[a.off.logstd + j]);
       if (a.key_in) {
         const float eps = normal_from_bits(random_bits_at(akey, a.mode, gbase + j, static_cast<uint32_t>(a.n_total)));
         act = __fadd_rn(mean, __fmul_rn(scale, eps));
@@ -118,18 +118,19 @@ __global__ void __launch_bounds__(PH_THREADS) policy_head_kernel(const PolicyHea
 
 static constexpr size_t policy_head_smem(int H, int amax) { return (static_cast<size_t>(H) * (amax + 1) + H) * 4; }
 // H = 512 with the 64-wide template: 135,168 bytes
-static_assert(policy_head_smem(MAX_HIDDEN, 64) <= 200 * 1024, "policy_head_kernel<64> shared memory at H = 512");
+constexpr int PH_SMEM_OPTIN = 200 * 1024;
+static_assert(policy_head_smem(MAX_HIDDEN, 64) <= PH_SMEM_OPTIN, "policy_head_kernel<64> shared memory at H = 512");
+
+int policy_head_init() {
+  cudaError_t e = cudaFuncSetAttribute(policy_head_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, PH_SMEM_OPTIN);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_head_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, PH_SMEM_OPTIN);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_head_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, PH_SMEM_OPTIN);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_head_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, PH_SMEM_OPTIN);
+  return e == cudaSuccess ? 0 : MINPPO_ERR_CUDA;
+}
 
 int policy_head_launch(const PolicyHeadArgs& a, cudaStream_t stream) {
   if (a.A > MAX_ACT_DIM || a.H % 8 != 0 || a.rows <= 0) { set_error("policy head: unsupported shape"); return MINPPO_ERR_ARG; }
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaFuncSetAttribute(policy_head_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(policy_head_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(policy_head_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    cudaFuncSetAttribute(policy_head_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-    attr_done = true;
-  }
   const int amax = a.A <= 8 ? 8 : (a.A <= 16 ? 16 : (a.A <= 32 ? 32 : 64));
   const size_t smem = policy_head_smem(a.H, amax);
   const int blocks = (a.rows + PH_ROWS - 1) / PH_ROWS;

@@ -32,7 +32,7 @@ constexpr int GEMM_STAGE_BYTES = GEMM_A_BYTES + GEMM_B_BYTES;
 constexpr int GEMM_THREADS = 192;
 constexpr int GEMM_EPI_THREADS = 128;
 constexpr int GEMM_ONES_BYTES = 16384;                   // all-ones bf16 [128][64] tile: A operand of the bias-gradient MMAs
-constexpr int GEMM_SMEM_BYTES = GEMM_STAGES * GEMM_STAGE_BYTES + GEMM_ONES_BYTES + 1024 /*align*/ + 4 * GEMM_MAXN * 4 /*colsum*/ + 256;
+constexpr int GEMM_SMEM_BYTES = GEMM_STAGES * GEMM_STAGE_BYTES + GEMM_ONES_BYTES + 1024 /*align*/ + 256;
 constexpr int GEMM_MAX_GROUPS = 8;
 
 enum : int { A_TMA_K = 0, A_GATHER_K = 1, A_TMA_MN = 2, A_GATHER_MN = 3 };
@@ -49,7 +49,6 @@ struct alignas(64) GemmGroup {
   void* out;                       // EPI_ACT/EPI_DACT: bf16 [M][ldo]
   const float* bias;               // EPI_ACT: fp32 [N]
   const __nv_bfloat16* hprev;      // EPI_DACT: layer output h (for f'(z) from h), bf16 [M][ldh]
-  float* colsum;                   // EPI_DACT: fp32 [m_tiles][ldc] per-tile column sums (bias grads)
   float* colsum_out;               // EPI_PARTIAL + B_TMA_MN: fp32 [splits][ldc] column sums of B over this CTA's K range
                                    // (= bias gradient partials), computed on the tensor core as ones x B; or null
   int ldg, ldo, ldh;
@@ -63,7 +62,7 @@ struct alignas(64) GemmGroup {
   int m_store;                     // EPI_PARTIAL: rows m < m_store are stored
   int n_off;                       // first column of this group's N range inside B, C, bias, out, hprev and the column sums
                                    // (N-split groups: a layer wider than GEMM_MAXN runs as several groups of <= 256 columns)
-  int ldc;                         // row stride of colsum / colsum_out in floats (the full width of an N-split layer); 0 = N
+  int ldc;                         // row stride of colsum_out in floats (the full width of an N-split layer); 0 = N
   const int32_t* k_count;          // optional: number of valid K rows (device side); k-blocks beyond it are skipped
 };
 
@@ -88,23 +87,6 @@ MINPPO_DEVINL void gather_line(uint32_t tile_base, int line, const __nv_bfloat16
   for (int j = 0; j < 8; ++j) cp_async_16(dst + ((j ^ sw) << 4), reinterpret_cast<const char*>(src) + j * 16);
 }
 
-// ---- 32x32 transpose-reduce: lane j ends with the sum over lanes of v[j] --------------------
-MINPPO_DEVINL float warp_colsum32(float (&v)[32]) {
-  const uint32_t lane = lane_id();
-#pragma unroll
-  for (int half = 16; half >= 1; half >>= 1) {
-    const bool upper = (lane & half) != 0;
-#pragma unroll
-    for (int i = 0; i < half; ++i) {
-      // keep the half of the columns selected by this lane's bit, send the other half
-      float keep = upper ? v[i + half] : v[i];
-      float send = upper ? v[i] : v[i + half];
-      v[i] = keep + __shfl_xor_sync(0xffffffffu, send, half);
-    }
-  }
-  return v[0];   // column index == lane (bit b of lane selected the upper half at step b)
-}
-
 // The whole CTA (GEMM_THREADS threads) calls this; it returns after the TMEM columns are released.
 // Warps 0..5 carry the roles; a caller may run with more warps per CTA (dwopt.cuh): they only take part
 // in the two CTA-wide barriers.
@@ -120,8 +102,7 @@ MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long l
   const uint32_t base = (raw + 1023u) & ~1023u;                      // SWIZZLE_128B: 1024-B aligned tiles
   uint8_t* aligned = smem_raw + (base - raw);
   const uint32_t ones = base + GEMM_STAGES * GEMM_STAGE_BYTES;                             // 1024-byte aligned
-  float* colsum_s = reinterpret_cast<float*>(aligned + GEMM_STAGES * GEMM_STAGE_BYTES + GEMM_ONES_BYTES);   // [4][MAXN]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(aligned + GEMM_STAGES * GEMM_STAGE_BYTES + GEMM_ONES_BYTES + 4 * GEMM_MAXN * 4);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(aligned + GEMM_STAGES * GEMM_STAGE_BYTES + GEMM_ONES_BYTES);
   uint64_t* full_bar = bars;                       // [STAGES]
   uint64_t* empty_bar = bars + GEMM_STAGES;        // [STAGES]
   uint64_t* tmem_full_bar = bars + 2 * GEMM_STAGES;
@@ -372,15 +353,11 @@ MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long l
             const int e = 8 * j + 2 * t;
             v[e] *= d0; v[e + 1] *= d1;
             w[4 * j + t] = pack_bf16x2(v[e], v[e + 1]);
-            // bias gradient sums what the dW GEMM will see: the bf16-rounded dZ
-            v[e] = bf16_lo(w[4 * j + t]); v[e + 1] = bf16_hi(w[4 * j + t]);
           }
         }
         uint4* o = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(G.out) + static_cast<size_t>(row) * G.ldo + G.n_off + c0);
 #pragma unroll
         for (int j = 0; j < 4; ++j) o[j] = make_uint4(w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]);
-        const float cs = warp_colsum32(v);
-        colsum_s[q * GEMM_MAXN + c0 + lane_id()] = cs;
       } else {  // EPI_PARTIAL: stage the fp32 tile in the (now idle) operand ring, SW128, then TMA-store it
         const int r = q * 32 + static_cast<int>(lane_id());
         const uint32_t dst = base + (c0 >> 5) * 16384 + r * 128;      // chunk tile: [128 rows][32 floats]
@@ -409,13 +386,6 @@ MINPPO_DEVINL void umma_gemm_body(const GemmParams& p, uint8_t* smem_raw, long l
 #pragma unroll
         for (int j = 1; j < 32; ++j) out = (static_cast<int>(lane_id()) == j) ? v[j] : out;
         G.colsum_out[static_cast<size_t>(split) * ldc + G.n_off + cs_c0 + ch * 32 + lane_id()] = out;
-      }
-    }
-    if (EPI == EPI_DACT) {
-      asm volatile("bar.sync 1, 128;" ::: "memory");
-      for (int c = et; c < N; c += GEMM_EPI_THREADS) {
-        const float s = (colsum_s[c] + colsum_s[GEMM_MAXN + c]) + (colsum_s[2 * GEMM_MAXN + c] + colsum_s[3 * GEMM_MAXN + c]);
-        G.colsum[static_cast<size_t>(m_tile) * ldc + G.n_off + c] = s;
       }
     }
   }
