@@ -1,85 +1,11 @@
-// minppo_b200 -- gradient reduction + global-norm clip + Adam, one multi-tensor kernel
-// (replaces optax.chain(clip_by_global_norm, adam) and TrainState.apply_gradients,
-//  /root/reference/minppo/train.py:98-101, 114-124, 248).
-//
-// The whole parameter set lives in one contiguous fp32 arena (leaf order = JAX's sorted
-// flatten order of the pickle tree, SURVEY.md section 5); mu / nu are arenas of the same shape.
-//
-// Phase R (reduce): every gradient element is the fixed-order sum of the per-tile / per-split
-//   partials the backward kernels wrote (no atomics -> bitwise reproducible), written to gflat;
-//   the minibatch loss sums ride along at gflat[P .. P+4).
-// Phase A (apply): sum of squares -> grid barrier -> clip scale -> Adam -> params, mu, nu and the
-//   bf16 weight images the tcgen05 GEMMs read (transposed [out][in] for forward, [in][out] for dX).
-// Single GPU runs R+A in one launch; with env-sharded ranks R, NCCL all-reduce(gflat), A.
+// minppo_b200 -- bf16 operand images: the observation image of an update, and the weight images the tcgen05 GEMMs and
+// the fused kernels read, from the fp32 parameter arena (at the start of an update and of a rollout policy step).  The
+// optimizer, which also rewrites the weight images after every minibatch step, is dwopt_kernel (dwopt.cuh).
 #include "common.cuh"
 #include "minppo_internal.h"
 #include "opt_common.cuh"
 
 namespace minppo {
-
-// Stand-alone optimizer launch: used when the merged dW + optimizer kernel (dwopt.cuh) does not apply --
-// env-sharded ranks (apply only, after the all-reduce of gflat) and the two-launch fallback.
-// Plain strided loops: the gradient lives in gflat between the phases.
-__global__ void __launch_bounds__(OPT_THREADS, 2) opt_kernel(const OptArgs a) {
-  __shared__ float scratch[32];
-  __shared__ float s_bcast[4];
-  __shared__ LeafTab T;
-  const int P = a.P;
-  const int G = gridDim.x;
-  leaf_tab_build(T, a, threadIdx.x, OPT_THREADS);
-  __syncthreads();
-  const int first = static_cast<int>(blockIdx.x) * OPT_THREADS + static_cast<int>(threadIdx.x);
-  const int stride = G * OPT_THREADS;
-
-  const int count = a.do_apply ? __ldcg(a.count) : 0;      // Adam step count BEFORE this step
-  float ent = a.entropy_const;                             // A * (0.5 + 0.5 log 2pi) + sum log|scale|
-  if (a.do_apply && blockIdx.x == 0 && threadIdx.x == 0 && a.losses_out) {
-    // train.py:240 -- evaluated with the PRE-update log_std (nothing is updated before the barrier)
-    for (int j = 0; j < a.A; ++j) ent += logf(fabsf(expf(__ldcg(a.params + a.off_logstd + j))));
-  }
-  griddep_wait();
-  if (threadIdx.x == 0) griddep_launch();
-  float ss = 0.f;
-  if (a.do_reduce) {
-    ss = reduce_leaves<false>(a, T, first, stride);
-    ss += reduce_leaves<true>(a, T, first, stride);
-  } else {
-#pragma unroll 1
-    for (int i = first; i < P; i += stride) { const float g = __ldcg(a.gflat + i); ss = fmaf(g, g, ss); }
-  }
-  if (!a.do_apply) return;
-
-  const float bs = block_sum<OPT_THREADS>(ss, scratch);
-  if (threadIdx.x == 0) a.block_ss[blockIdx.x] = bs;
-  grid_barrier(a.barrier, a.err_flag);
-  {
-    const float v = static_cast<int>(threadIdx.x) < G ? __ldcg(a.block_ss + threadIdx.x) : 0.f;   // G <= OPT_THREADS
-    const float tot = block_sum<OPT_THREADS>(v, scratch);
-    if (threadIdx.x == 0) s_bcast[0] = sqrtf(tot);
-  }
-  if (threadIdx.x == 32) step_scalars(a, count, s_bcast[1], s_bcast[2], s_bcast[3]);
-  __syncthreads();
-  AdamScalars sc;
-  sc.gnorm = s_bcast[0]; sc.lr = s_bcast[1]; sc.c1 = s_bcast[2]; sc.c2 = s_bcast[3];
-  sc.trigger = sc.gnorm < a.max_norm;                      // optax.clip_by_global_norm
-  apply_adam(a, T, sc, first, stride);
-  if (blockIdx.x == 0 && threadIdx.x == 0) {
-    *a.count = count + 1;
-    if (a.losses_out) {
-      // gflat[P] = sum max(vl, vlc), gflat[P+1] = sum min(l1, l2) over the global minibatch
-      const float value_loss = 0.5f * __ldcg(a.gflat + P) * a.inv_mb;
-      const float actor_loss = -__ldcg(a.gflat + P + 1) * a.inv_mb;
-      // a raised device-side error flag (row-list overflow, barrier / exchange timeout) poisons the reported losses:
-      // the failure surfaces in the update's own result without a host round trip (minppo_ctx_check names the cause)
-      const float poison = __ldcg(a.err_flag) != 0 ? __int_as_float(0x7fc00000) : 0.f;
-      a.losses_out[0] = actor_loss + a.vf_coef * value_loss - a.ent_coef * ent + poison;
-      a.losses_out[1] = value_loss + poison;
-      a.losses_out[2] = actor_loss + poison;
-      a.losses_out[3] = ent + poison;
-      if (a.gnorm_out) *a.gnorm_out = sc.gnorm;
-    }
-  }
-}
 
 // fp32 [rows][cols] -> bf16 [rows][ld] (zero padded); used for the observation image and
 // for the initial weight images.
@@ -110,13 +36,6 @@ __global__ void weight_images_kernel(const OptArgs a) {
     while (l + 1 < a.nleaves && i >= a.leaf[l + 1].offset) ++l;
     write_images(a.leaf[l], i, a.params[i]);
   }
-}
-
-int opt_max_params(int) { return 0x7fffffff - 2; }      // strided loops: no per-launch limit
-
-int opt_launch(const OptArgs& a, int blocks, cudaStream_t stream, bool pdl) {
-  const cudaError_t e = launch_kernel(opt_kernel, blocks, OPT_THREADS, 0, stream, pdl, a);
-  return e == cudaSuccess ? 0 : MINPPO_ERR_CUDA;
 }
 
 int weight_images_launch(const OptArgs& a, cudaStream_t stream) {

@@ -19,8 +19,11 @@
 // launch's producers run behind this launch's end (griddepcontrol.wait), so the counters need no generations.
 // The phases are plain strided loops (no per-element unrolling): an earlier fully unrolled version was
 // 15k SASS instructions and spent a third of its time on instruction-cache misses.
-// With env-sharded ranks (do_apply == 0) the kernel stops after phase 2 and the barrier (the counter reset needs it) with
-// the local gradient SUM in gflat; the all-reduce and opt_kernel (adam.cu, apply only) follow.
+// Launched without GEMM CTAs (gemm_ctas == 0), every CTA is a spare CTA: after a stand-alone dW GEMM launch when the GEMM
+// grid does not fit one CTA per SM, and to apply an all-reduced gradient (learner.cu fill_apply_only).
+// With env-sharded ranks that do not exchange over peer memory (do_apply == 0) the kernel stops after phase 2 and the
+// barrier (the counter reset needs it) with the local gradient SUM in gflat; the NCCL all-reduce and that apply-only
+// launch follow.
 #pragma once
 
 #include "opt_common.cuh"
@@ -128,7 +131,8 @@ MINPPO_DEVINL void st_unit(float* p, const float (&v)[4]) {
 struct alignas(64) DwOptParams {
   GemmParams gemm;               // the per-step row list / valid-row count of the groups come from the arrays below
   OptArgs opt;                   // losses_out / gnorm_out: bases of the per-step arrays (losses_stride floats apart / 1 apart)
-  int gemm_ctas;                 // CTAs [0, gemm_ctas) run the GEMM; the others pre-reduce the small leaves
+  int gemm_ctas;                 // CTAs [0, gemm_ctas) run the GEMM; the others pre-reduce the small leaves (gemm.g[0].splits
+                                 // >= 1 also at 0: the counter reset divides by it)
   long long* trace;              // debug: [grid][16] clock64 stamps (null = off)
   unsigned int* done;            // [1 + gemm_ctas / S][DWOPT_DONE_STRIDE] completion counters (zero at launch, reset at its end):
                                  // [0] small-leaf CTAs done, [1 + b / S] split-K tile of GEMM CTA b: S partials stored
@@ -506,7 +510,7 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
   DW_STAMP(4);
   // every counter wait of this launch is behind the barrier: back to zero for the next launch
   if (b == 0 && t <= p.gemm_ctas / static_cast<int>(S)) p.done[t * DWOPT_DONE_STRIDE] = 0u;
-  if (!a.do_apply) return;                               // NCCL fallback: gflat = the local gradient sum; opt_kernel applies
+  if (!a.do_apply) return;                               // NCCL fallback: gflat = the local gradient sum; applied by a later launch
 
   // ---- phase 3 ----------------------------------------------------------------------------------
   // This thread's element of the SMALL leaves (at most one when they fit one sweep of the grid): gradient and optimizer state

@@ -280,7 +280,6 @@ struct minppo_ctx {
   int po_db[2][2];            // fused path: [net][layer] hidden-bias gradient partials (column sums of dZ), H floats each
   int ap;                     // padded head width of the fused step kernel: 16 (A <= 16) or 32
   HeadOffsets head;           // arena offsets of the output-head leaves
-  int opt_blocks;
   // graph cache
   cudaStream_t cap_stream;
   cudaStream_t side_stream;    // fork/join branch of an update: operand staging (observation + weight images) runs beside
@@ -530,7 +529,10 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
   p.ngroups = ng;
   gemm_finalize(p);
   fill_opt_args(c, u, &dp.opt);
-  for (size_t i = 0; i < c->leaves.size(); ++i) {
+  // A GEMM grid past one CTA per SM runs as a launch of its own in front of dwopt (enqueue_step): dwopt then has no GEMM
+  // CTAs, and its late leaves wait for no counter (tile fields 0), since their partials are complete when it starts.
+  dp.gemm_ctas = cta <= c->sm_count ? cta : 0;
+  for (size_t i = 0; i < c->leaves.size() && dp.gemm_ctas; ++i) {
     OptLeaf& ol = dp.opt.leaf[i];
     const LeafInfo& lf = c->leaves[i];
     if (!ol.late) continue;                                  // hidden kernels (and, layer-wise path, hidden biases)
@@ -542,13 +544,32 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
   dp.opt.losses_out = u.losses_out ? u.losses_out : c->losses_scratch;
   dp.losses_stride = u.losses_out ? 4 : 0;
   dp.opt.gnorm_out = c->gnorms;
-  dp.gemm_ctas = cta;
   dp.ridx_base = c->rowidx; dp.counts = c->counts; dp.cap = c->cap; dp.EM = c->E * c->M;
   dp.padded = c->padded ? 1 : 0;
   dp.part_rows = c->fused ? 128 : 64;
   dp.obs_img = c->obs_img; dp.obs_ld = c->Dp;
   dp.trace = c->trace_on ? c->trace2 : nullptr;
   return cta;
+}
+
+// The NCCL fallback's second dwopt launch, which only applies the all-reduced gradient: gflat holds it (P floats, then the
+// two loss sums), and it becomes the single partial of every leaf and of the loss sums.  The reduction phase then copies
+// gflat onto itself and forms the global norm; phase 3 runs clip + Adam and writes the weight images as usual.  Every leaf
+// is "early": the late path issues 16-byte loads, and gflat + a leaf offset is only 4-byte aligned.  grad_bias is 0
+// because rank 0 added -ent_coef to the log_std gradient before the all-reduce, and padded is 0 because the live-tile
+// cap counts per-tile partials, which gflat is not.
+static void fill_apply_only(const minppo_ctx* c, DwOptParams* dpp) {
+  DwOptParams& dp = *dpp;
+  OptArgs& o = dp.opt;
+  for (int i = 0; i < o.nleaves; ++i) {
+    OptLeaf& ol = o.leaf[i];
+    ol.late = 0; ol.grad_src = c->gflat; ol.src_offset = ol.offset; ol.nparts = 1; ol.grad_bias = 0.f;
+  }
+  o.n_early = o.P;
+  o.loss_src = c->gflat; o.loss_src_offset = o.P; o.loss_nparts = 1;
+  o.do_apply = 1;
+  dp.gemm_ctas = 0;
+  dp.padded = 0;
 }
 
 // One net's operands in the forward GEMM of one hidden layer
@@ -667,59 +688,44 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
     c->launches++;
   }
   }  // !fused
-  // weight gradients dW_l = act[l]^T dz[l+1] (split-K over minibatch rows), then the optimizer.
-  // ONE launch (dwopt.cuh) when the GEMM grid fits one CTA per SM; otherwise the two-launch sequence (GEMM kernel,
-  // opt_kernel).
+  // weight gradients dW_l = act[l]^T dz[l+1] (split-K over minibatch rows), then the optimizer: ONE dwopt launch
+  // (dwopt.cuh) when the GEMM grid fits one CTA per SM; otherwise the stand-alone GEMM kernel, then dwopt without GEMM
+  // CTAs.  Env-sharded ranks without the peer-memory exchange then all-reduce the gradient sums over NCCL and apply them
+  // with a second dwopt launch.
   DwOptParams dp;
   const int cta = fill_dwopt_params(c, u, &dp);
   dp.step = s;
-  GemmParams& p = dp.gemm;
-  OptArgs& o = dp.opt;
+  const bool two_launch = cta > c->sm_count;
   const bool sharded = c->cfg.world_size > 1;
-  if (cta <= c->sm_count) {
-    // all-reduce fused into this launch (peer memory); needs the register-resident fast path of the kernel
-    const bool px_on = sharded && c->peers_set && c->P <= dwopt_fast_capacity(c->sm_count, c->maxu);
-    if (px_on) dp.px = c->px;
-    o.do_reduce = 1; o.do_apply = (sharded && !px_on) ? 0 : 1;
-    {
-      PROF(PC_DW_GEMM);
-      const cudaError_t e = dwopt_launch(dp, c->sm_count, stream, pdl, c->maxu);
-      if (e != cudaSuccess) { set_error("dwopt launch failed: %s", cudaGetErrorString(e)); return MINPPO_ERR_CUDA; }
-      c->launches++;
-    }
-    if (sharded && !px_on) {
-      { PROF(PC_ALLREDUCE); RET(nccl_allreduce(c, c->gflat, static_cast<size_t>(c->P) + 2, stream)); }
-      o.losses_out = o.losses_out + static_cast<size_t>(s) * dp.losses_stride; o.gnorm_out = c->gnorms + s;   // opt_kernel: direct pointers
-      o.do_reduce = 0; o.do_apply = 1;
-      { PROF(PC_OPT); RET(opt_launch(o, c->opt_blocks, stream, pdl)); }
-      c->launches += 2;
-    }
+  // all-reduce fused into the dwopt launch (peer memory); needs the register-resident fast path of the kernel, and the
+  // GEMM in the same launch
+  const bool px_on = sharded && c->peers_set && c->P <= dwopt_fast_capacity(c->sm_count, c->maxu) && !two_launch;
+  const bool nccl = sharded && !px_on;
+  if (px_on) dp.px = c->px;
+  dp.opt.do_apply = nccl ? 0 : 1;
+  auto launch_dwopt = [&]() -> int {
+    PROF(dp.gemm_ctas ? PC_DW_GEMM : PC_OPT);
+    const cudaError_t e = dwopt_launch(dp, c->sm_count, stream, pdl, c->maxu);
+    if (e != cudaSuccess) { set_error("dwopt launch failed: %s", cudaGetErrorString(e)); return MINPPO_ERR_CUDA; }
+    c->launches++;
     return 0;
-  }
-  // two-launch fallback (stand-alone GEMM kernel + opt_kernel): per-step pointers go into the blocks directly
-  for (int i = 0; i < p.ngroups; ++i) {
-    if (p.g[i].rowidx) p.g[i].rowidx = ridx;
-    p.g[i].k_count = c->padded ? c->counts + s : nullptr;
-  }
-  o.losses_out = o.losses_out + static_cast<size_t>(s) * dp.losses_stride;
-  o.gnorm_out = c->gnorms + s;
-  {
+  };
+  if (two_launch) {
+    GemmParams p = dp.gemm;                                  // this step's row list and row count go into the groups
+    for (int i = 0; i < p.ngroups; ++i) {
+      if (p.g[i].rowidx) p.g[i].rowidx = ridx;
+      p.g[i].k_count = c->padded ? c->counts + s : nullptr;
+    }
     PROF(PC_DW_GEMM);
     RET(launch_gemm<EPI_PARTIAL>(p, cta, stream, pdl));
     c->launches++;
   }
-  if (!sharded) {
-    o.do_reduce = 1; o.do_apply = 1;
-    PROF(PC_OPT);
-    RET(opt_launch(o, c->opt_blocks, stream, pdl));
-    c->launches++;
-  } else {
-    o.do_reduce = 1; o.do_apply = 0;
-    { PROF(PC_OPT); RET(opt_launch(o, c->opt_blocks, stream, pdl)); }
+  RET(launch_dwopt());
+  if (nccl) {
     { PROF(PC_ALLREDUCE); RET(nccl_allreduce(c, c->gflat, static_cast<size_t>(c->P) + 2, stream)); }
-    o.do_reduce = 0; o.do_apply = 1;
-    { PROF(PC_OPT); RET(opt_launch(o, c->opt_blocks, stream, pdl)); }
-    c->launches += 3;
+    c->launches++;
+    fill_apply_only(c, &dp);
+    RET(launch_dwopt());
   }
   return 0;
 }
@@ -977,8 +983,6 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
     while (S > 1 && ((kb_total + S - 1) / S) * (S - 1) >= kb_total) --S;
     c->S = S;
   }
-  c->opt_blocks = c->sm_count;
-  if (c->P > opt_max_params(c->opt_blocks)) { set_error("parameter count %lld exceeds the single-sweep optimizer kernel (%d)", c->P, opt_max_params(c->opt_blocks)); return fail(MINPPO_ERR_UNSUPPORTED); }
   const int H = c->H, L = c->L, A = c->A;
   // head partial layout
   {
@@ -1012,7 +1016,7 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
     c->px.np = np; c->px.world = 0; c->px.rank = cfg->rank; c->px.seq = c->xseq;
   }
   ALLOC(c->gflat, static_cast<size_t>(c->P) + 4);
-  ALLOC(c->block_ss, static_cast<size_t>(c->opt_blocks));
+  ALLOC(c->block_ss, static_cast<size_t>(c->sm_count));
   ALLOC(c->head_part, static_cast<size_t>(c->tiles64) * c->head_stride);
   ALLOC(c->gnorms, static_cast<size_t>(EM));
   ALLOC(c->losses_scratch, 4);

@@ -108,10 +108,11 @@ struct OptLeaf {
                                  // and of the dX GEMMs as K-major), or null
   uint8_t* img_w2;               // output-head kernels: 16 KB bf16 hi / lo image of kernel^T in the fused kernel's
                                  // shared-memory layout (fused_step.cuh FS_W2T), or null
-  int late;                      // 1: partials are written by the dW GEMM of the same launch (hidden kernels)
+  int late;                      // 1: partials are written by the dW GEMM (hidden kernels), summed in 16-byte units
   int size;                      // elements of this leaf (host-computed: the kernels never walk the table serially)
   int ap;                        // img_w2: padded head width of the image (16 or 32 rows per hi / lo half)
-  // late leaves in dwopt.cuh: the completion counters of the dW GEMM tiles that write this leaf's partials
+  // late leaves in dwopt.cuh: the completion counters of the dW GEMM tiles that write this leaf's partials (all 0 when the
+  // GEMM ran as a launch of its own)
   int tile0;                     // counter of the layer's first tile (column group 0, m-tile 0); tiles run m-tile fastest
   int tile_n;                    // tiles of the layer (column groups x 128-row m-tiles)
   int tile_split;                // hidden kernels: columns of column group 0; 0 (biases): an element needs every tile
@@ -120,7 +121,7 @@ struct OptArgs {
   OptLeaf leaf[MINPPO_MAX_LEAVES];
   int nleaves, P, A;
   int n_early;                   // elements of the leaves with late == 0
-  int do_reduce, do_apply;
+  int do_apply;
   float* gflat;                  // [P + 4] reduced gradient (minppo_ctx_read buffer 3 returns the last one), then the loss sums
   const float* loss_src;         // loss partial sums (2 per partial)
   int loss_src_offset, loss_nparts, loss_part_stride;
@@ -136,8 +137,6 @@ struct OptArgs {
   float lr, max_norm, b1, b2, one_minus_b1, one_minus_b2, eps, eps_root;
   float inv_mb, vf_coef, ent_coef, entropy_const;
 };
-int opt_launch(const OptArgs& a, int blocks, cudaStream_t stream, bool pdl = false);
-int opt_max_params(int blocks);
 int weight_images_launch(const OptArgs& a, cudaStream_t stream);
 int obs_image_launch(const float* obs, __nv_bfloat16* img, long long rows, int cols, int ld, cudaStream_t stream);
 

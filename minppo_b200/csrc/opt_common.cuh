@@ -1,27 +1,10 @@
-// minppo_b200 -- device helpers shared by the optimizer kernels (adam.cu, dwopt.cuh).
+// minppo_b200 -- device helpers of the optimizer (dwopt.cuh) and of the weight-image kernel (adam.cu).
 #pragma once
 
 #include "common.cuh"
 #include "minppo_internal.h"
 
 namespace minppo {
-
-constexpr int OPT_THREADS = 512;                 // 512 x <= 42 regs: co-resident with a fused-step CTA under PDL
-
-
-template <int NTHREADS = 512>
-MINPPO_DEVINL float block_sum(float v, float* scratch /*[32]*/) {
-  v = warp_sum(v);
-  if ((threadIdx.x & 31) == 0) scratch[threadIdx.x >> 5] = v;
-  __syncthreads();
-  float s = 0.f;
-  if (threadIdx.x < 32) {
-    s = threadIdx.x < (NTHREADS / 32) ? scratch[threadIdx.x] : 0.f;
-    s = warp_sum(s);
-  }
-  __syncthreads();
-  return s;                                   // valid in warp 0
-}
 
 // Sense-free grid barrier on a monotonically increasing 64-bit counter.  All blocks of the
 // grid are co-resident (grid <= #SMs, one block per SM).  Arrive = atom.add.release.gpu, wait =
@@ -44,28 +27,6 @@ MINPPO_DEVINL void grid_barrier(unsigned long long* counter, int* err_flag) {
   }
   __syncthreads();
 }
-
-// fixed-order sum of `nparts` partials, 8 loads in flight
-MINPPO_DEVINL float sum_partials(const float* __restrict__ src, int nparts, size_t stride) {
-  float acc = 0.f;
-  int p = 0;
-  for (; p + 8 <= nparts; p += 8) {
-    float v[8];
-#pragma unroll
-    for (int u = 0; u < 8; ++u) v[u] = __ldcg(src + static_cast<size_t>(p + u) * stride);
-#pragma unroll
-    for (int u = 0; u < 8; ++u) acc += v[u];
-  }
-  for (; p < nparts; ++p) acc += __ldcg(src + static_cast<size_t>(p) * stride);
-  return acc;
-}
-
-MINPPO_DEVINL int find_leaf_idx(const OptArgs& a, int i) {
-  int l = 0;
-  while (l + 1 < a.nleaves && i >= a.leaf[l + 1].offset) ++l;
-  return l;
-}
-
 
 // One Adam step on one element (optax.scale_by_adam + scale(-lr), train.py:116-124), after the
 // global-norm clip (optax.clip_by_global_norm: g unchanged if gnorm < max_norm, else g / gnorm * max_norm).
@@ -189,7 +150,7 @@ MINPPO_DEVINL float4 sum_partials16_v4(const float* __restrict__ src, int nparts
 // Gradient reduction of one class of leaves -> gflat; returns this thread's sum of squares.
 //   LATE == false: leaves whose partials the fused step kernel wrote (biases of the output heads, head
 //                  kernels, log_std, ...): one element per job, then the two loss sums.
-//   LATE == true : leaves whose partials the dW GEMM of the SAME launch writes (hidden kernels): four
+//   LATE == true : leaves whose partials the dW GEMM writes (hidden kernels): four
 //                  elements per job (sizes and partial strides are multiples of 4, partial buffers 16-byte
 //                  aligned; gflat itself is only 4-byte aligned at a leaf offset).
 // Jobs are dealt round-robin (job = first + k * stride); the leaf walk is monotonic in k.

@@ -50,7 +50,7 @@ CASES = {
     "h512_d1000_a64": _case(32, 8, 1000, 64, H=512, expect=dict(fused=False, maxu=4, fast=False, head_amax=64)),
     "maxu2_d415_a20": _case(32, 16, 415, 20, expect=dict(fused=True, maxu=2, fast=True, two_launch=False)),
     "maxu4_d1000": _case(32, 16, 1000, 10, expect=dict(fused=True, maxu=4, fast=True, two_launch=False)),
-    # the two-launch sequence (stand-alone dW GEMM, then opt_kernel): 4 (fused) / 8 (layer-wise) splits of a
+    # the two-launch sequence (stand-alone dW GEMM, then dwopt without GEMM CTAs): 4 (fused) / 8 (layer-wise) splits of a
     # D = 1000 network do not fit one CTA per SM
     "two_launch_fused": _case(32, 16, 1000, 10, cfg=dict(dw_splits=4), expect=dict(fused=True, S=4, two_launch=True)),
     "two_launch_layerwise": _case(32, 16, 1000, 10, cfg=dict(dw_splits=8, fused=False),

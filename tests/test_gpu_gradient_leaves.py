@@ -179,7 +179,7 @@ OPT_PATHS = {
     "dwopt4_nonfast": dict(hp=dict(num_envs=8, num_steps=4, hidden_size=512), D=1000, A=64, cfg={},
                            expect=dict(two_launch=False, maxu=4, fast=False)),
     # 4 splits need 4 k-blocks: 256 rows
-    "opt_kernel": dict(hp=dict(num_envs=32, num_steps=8, hidden_size=256), D=1000, A=10, cfg=dict(dw_splits=4),
+    "two_launch": dict(hp=dict(num_envs=32, num_steps=8, hidden_size=256), D=1000, A=10, cfg=dict(dw_splits=4),
                        expect=dict(two_launch=True)),
 }
 

@@ -69,7 +69,7 @@ CASES = {
     # 16 k-blocks of D, P = 646k: four register-resident units per optimizer thread
     "d1000": dict(hp=dict(num_envs=32, num_steps=16, num_minibatches=2, update_epochs=1, anneal_lr=False), D=1000, A=10),
     # the same with 4 dW splits: 4 x 40 GEMM CTAs do not fit one CTA per SM (148), so every step takes the two-launch
-    # sequence (stand-alone dW GEMM, then opt_kernel) instead of the merged dwopt launch
+    # sequence (stand-alone dW GEMM, then dwopt without GEMM CTAs) instead of the merged dwopt launch
     "d1000_two_launch": dict(hp=dict(num_envs=32, num_steps=16, num_minibatches=2, update_epochs=1, anneal_lr=False),
                              D=1000, A=10, cfg=dict(dw_splits=4)),
 }
