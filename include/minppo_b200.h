@@ -146,6 +146,23 @@ int minppo_update(minppo_ctx* ctx, float* params, float* mu, float* nu, int32_t*
                   const uint8_t* done, const float* last_val, const uint32_t* key_in, uint32_t* key_out,
                   float* losses_out, int32_t use_graph, void* stream);
 
+/* minppo_update plus per-minibatch PPO diagnostics (minppo_update is this call with stats_out == NULL).
+ * stats_out: f32 [E, M, 4], may be NULL.  Row s = e * M + k describes minibatch step s over the rows of the GLOBAL
+ * minibatch (all ranks, live rows only), evaluated in the forward pass of that step's loss, i.e. with the parameters
+ * BEFORE that step's Adam update; r = exp(logp_new - logp_old) is the loss's probability ratio:
+ *   [0] approx_kl            mean(expm1(log r) - log r)        (the "(r - 1) - log r" estimator)
+ *   [1] clip_fraction        mean(|r - 1| > clip_eps)
+ *   [2] value_clip_fraction  mean(|v - v_old| > clip_eps)
+ *   [3] grad_norm            global gradient norm before clipping (clip_by_global_norm), bit-identical to
+ *                            minppo_ctx_read buffer 4
+ * The sums are always computed; stats_out only selects whether they are written.  Everything else the update computes
+ * is bit-identical with and without stats_out.  stats_out is part of the graph cache's pointer set.  A device-side
+ * failure turns all four columns of the remaining steps into NaN, as it does the losses. */
+int minppo_update_with_stats(minppo_ctx* ctx, float* params, float* mu, float* nu, int32_t* count, const float* obs,
+                             const float* action, const float* value, const float* reward, const float* log_prob,
+                             const uint8_t* done, const float* last_val, const uint32_t* key_in, uint32_t* key_out,
+                             float* losses_out, float* stats_out, int32_t use_graph, void* stream);
+
 /* ---- (5) policy / value inference for the rollout: replaces train.py:157-160 and 182-183 ------------
  * One env step's network evaluation on this rank's Nl = N / world_size envs, forward only, on the same bf16 weight
  * images and with the same rounding points as the learner's forward pass:

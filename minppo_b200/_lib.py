@@ -24,7 +24,7 @@ SYMBOLS = (
     "minppo_nccl_unique_id", "minppo_ctx_create", "minppo_ctx_destroy", "minppo_update",
     "minppo_ctx_check", "minppo_update_launch_count", "minppo_ctx_read", "minppo_debug_gemm",
     "minppo_ctx_profile", "minppo_ctx_profile_read", "minppo_ctx_ipc_handle", "minppo_ctx_set_peers",
-    "minppo_policy_step",
+    "minppo_policy_step", "minppo_update_with_stats",
 )
 POLICY_WEIGHTS_CURRENT = 1
 PROFILE_CLASSES = ("gae", "perm_sort", "rows_and_adv_stats", "obs_image", "weight_images", "fwd_gemm", "head_loss",
@@ -91,6 +91,8 @@ def load() -> C.CDLL:
     lib.minppo_ctx_destroy.argtypes = [vp]
     lib.minppo_update.restype = C.c_int
     lib.minppo_update.argtypes = [vp] + [vp] * 14 + [i32, vp]
+    lib.minppo_update_with_stats.restype = C.c_int
+    lib.minppo_update_with_stats.argtypes = [vp] + [vp] * 15 + [i32, vp]
     lib.minppo_ctx_check.restype = C.c_int
     lib.minppo_ctx_check.argtypes = [vp, vp]
     lib.minppo_update_launch_count.restype = i64

@@ -44,7 +44,7 @@ constexpr int DWOPT_THREADS = 512;
 // Exchange allocation of one rank (exported by CUDA IPC):
 //   stage [2][W][np] f32   slot (n & 1, q): rank q's local gradient of exchange n (all words start as the sentinel).
 //                          Inside a slot: the 4-element units of the late leaves (16-byte aligned), then the early
-//                          elements and the two loss sums (dwopt job numbering).  The element -> (CTA, thread)
+//                          elements and the LOSS_SUMS loss sums (dwopt job numbering).  The element -> (CTA, thread)
 //                          mapping is the same on every rank: a thread only ever waits for its own unit.
 //   (pad)  [W][256] u32    unused (was: the arrival flags of the earlier release/acquire protocol).
 //   result [2][np] f32     two-phase variant: the reduced gradient of exchange n, pushed by the owners of its units.
@@ -335,7 +335,7 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
     const int n_late4 = 4 * n_units;
     // early element (or loss sum) of this thread: same job numbering as apply_adam_class<false>
     int eidx = -1;
-    if (gtid < T.n_early + 2) {
+    if (gtid < T.n_early + LOSS_SUMS) {
       if (gtid >= T.n_early) eidx = P + (gtid - T.n_early);
       else {
         int x = gtid, l = 0;
@@ -581,6 +581,15 @@ __global__ void __launch_bounds__(DWOPT_THREADS, 1) dwopt_kernel(const __grid_co
       losses_out[2] = actor_loss + poison;
       losses_out[3] = ent + poison;
       if (gnorm_out) *gnorm_out = sc.gnorm;
+      if (a.stats_out) {
+        // gflat[P+2] = value-clip count, gflat[P+3] = approx-KL sum, gflat[P+4] = ratio-clip count (LOSS_SUMS).  The
+        // address is formed here, from the kernel parameters: a pointer live across the kernel adds to dwopt_kernel<4>'s spills
+        float* stats_out = a.stats_out + static_cast<size_t>(p.step) * 4;
+        stats_out[0] = __ldcg(a.gflat + P + 3) * a.inv_mb + poison;
+        stats_out[1] = __ldcg(a.gflat + P + 4) * a.inv_mb + poison;
+        stats_out[2] = __ldcg(a.gflat + P + 2) * a.inv_mb + poison;
+        stats_out[3] = sc.gnorm + poison;
+      }
     }
   }
 }

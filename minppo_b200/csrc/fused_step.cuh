@@ -89,6 +89,7 @@ struct alignas(64) FusedNet {
   int act;                       // ACT_*
   int aout;                      // A (actor) or 1 (critic)
   int po_w2, po_b2, po_loss;     // offsets of this net's fields inside a per-tile partial
+  int po_stat;                   // ... this net's statistics sums (LOSS_SUMS): actor 2 (KL, ratio clips), critic 1 (value clips)
   int po_db0, po_db1;            // ... hidden bias gradients (column sums of dZ1 / dZ2), H floats each
 };
 
@@ -371,6 +372,7 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
     if (static_cast<int>(threadIdx.x) < G.aout) part[G.po_b2 + threadIdx.x] = 0.f;
     if (net == 0 && static_cast<int>(threadIdx.x) < G.aout) part[p.po_logstd + threadIdx.x] = 0.f;
     if (threadIdx.x == 0) part[G.po_loss] = 0.f;
+    if (static_cast<int>(threadIdx.x) < (net == 0 ? 2 : 1)) part[G.po_stat + threadIdx.x] = 0.f;
     return;
   }
   __syncthreads();
@@ -732,6 +734,8 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
     mbar_wait(headf, 0);
     tc_fence_after();
     if (wt == 0) FS_STAMP(6);
+    // inputs of the statistics sums (LOSS_SUMS), reduced after g^T is published: actor log r and r, critic v - v_old
+    float st_a = 0.f, st_b = 1.f;
     {
       const uint32_t th = acc_head + (static_cast<uint32_t>(q * 32) << 16);
       const float inv_n = p.inv_mb;
@@ -770,7 +774,8 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
         float s_loss = 0.f, g_logp = 0.f;
         if (live) {
           const float logp = quad - hb[3 * AP];
-          const float ratio = expf(logp - in0);
+          const float logr = logp - in0;
+          const float ratio = expf(logr);
           const float adv_mean = adv_sum * inv_n;
           const float adv_std = sqrtf(adv_sq * inv_n);
           const float adv = (in1 - adv_mean) / (adv_std + 1e-8f);                 // train.py:235
@@ -781,6 +786,7 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
           const float w1 = l1 < l2 ? 1.f : (l1 == l2 ? 0.5f : 0.f);
           const float dmin = (w1 + (1.f - w1) * dclip_f(ratio, lo, hi)) * adv;
           g_logp = -inv_n * dmin * ratio;
+          st_a = logr; st_b = ratio;
         }
         // tile sums of dlog_std and of the head-bias gradient g through a 2 CW x 32 transpose-reduce
         float v[2 * CW];
@@ -814,6 +820,7 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
           s_loss = fmaxf(vl, vlc);
           const float wa = vl > vlc ? 1.f : (vl == vlc ? 0.5f : 0.f);
           g0 = p.vf_coef * 0.5f * inv_n * (wa * 2.f * e1 + (1.f - wa) * 2.f * e2 * dclip_f(dvv, -p.clip_eps, p.clip_eps));
+          st_a = dvv;
         }
         put_g(0, g0);
         const float gs = warp_sum(g0);
@@ -826,13 +833,29 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
     tc_fence_before();
     __syncwarp();
     if (lane == 0) mbar_arrive(gr);
+    // statistics sums, off the path to the dA2 / dW2 MMAs that g^T starts: red[q][2 AP + 1, 2 AP + 3) (po_stat).  Actor:
+    // approx-KL term (r - 1) - log r as expm1 (no cancellation at small log r) and |r - 1| > clip_eps; critic:
+    // |v - v_old| > clip_eps.  The four warps of an actor lane quadrant hold the same rows: warp sub == 0 sums them.
+    if (sub == 0) {
+      float* rw = red + q * RS + 2 * AP + 1;
+      if (net == 0) {
+        const float kl = live ? expm1f(st_a) - st_a : 0.f;
+        const float clipped = live && fabsf(st_b - 1.f) > p.clip_eps ? 1.f : 0.f;
+        const float s_kl = warp_sum(kl), s_clip = warp_sum(clipped);
+        if (lane == 0) { rw[0] = s_kl; rw[1] = s_clip; }
+      } else {
+        const float s_vclip = warp_sum(live && fabsf(st_a) > p.clip_eps ? 1.f : 0.f);
+        if (lane == 0) rw[0] = s_vclip;
+      }
+    }
     worker_bar();
     if (wt == 0) FS_STAMP(7);
     float* part = p.part + static_cast<size_t>(tile) * p.part_stride;
-    if (wt <= 2 * AP) {
+    if (wt < 2 * AP + (net == 0 ? 3 : 2)) {
       float s = 0.f;
       for (int w = 0; w < 4; ++w) s += red[w * RS + wt];         // fixed order: the four loss warps
-      if (wt == 2 * AP) part[G.po_loss] = s;
+      if (wt > 2 * AP) part[G.po_stat + wt - 2 * AP - 1] = s;
+      else if (wt == 2 * AP) part[G.po_loss] = s;
       else if (wt >= AP) { if (wt - AP < aout) part[G.po_b2 + wt - AP] = s; }
       else if (net == 0 && wt < aout) part[p.po_logstd + wt] = s;
     }

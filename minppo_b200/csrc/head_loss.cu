@@ -7,7 +7,7 @@
 //   logp, ratio, clipped surrogate, clipped value loss              (train.py:223-239)
 //   g_mean = dL/dmean, g_v = dL/dv, dL/dlog_std                      (hand-derived; oracle/ppo_numpy.py)
 //   dZ_a = (g_mean W3a^T) * f'(h_a), dZ_c = (g_v W3c^T) * f'(h_c)   -> bf16, feeds the tcgen05 GEMMs
-//   per-tile partial sums of dW3, db3, dlog_std and the loss terms
+//   per-tile partial sums of dW3, db3, dlog_std, the loss terms and the statistics sums (LOSS_SUMS)
 // Partials are written per tile (no atomics) and reduced in fixed order by the optimizer kernel.
 //
 // Rows >= count (padding of the last 128-row GEMM tile, or rows another GPU owns) produce
@@ -52,7 +52,7 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
   float* w3c = w3a + (CHUNKED ? HL_KCHUNK : H) * (AMAX + 1);       // [H]
   float* gm = w3c + H;                                            // [64][AMAX]  g_mean
   float* gv = gm + HL_ROWS * AMAX;                                // [64]
-  float* red = gv + HL_ROWS;                                      // [8][AMAX + 4] warp partials
+  float* red = gv + HL_ROWS;                                      // [8][AMAX + 8] warp partials: dlog_std, then LOSS_SUMS
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int tile = blockIdx.x;
@@ -130,7 +130,7 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
 
   // ---- phase 2: loss and gradient seeds, one thread per row (part == 0) -------------------
   float dls[AMAX];                       // this row's contribution to d/dlog_std
-  float s_val = 0.f, s_act = 0.f;
+  float s_val = 0.f, s_act = 0.f, s_vclip = 0.f, s_kl = 0.f, s_clip = 0.f;   // the LOSS_SUMS terms of this row
 #pragma unroll
   for (int j = 0; j < AMAX; ++j) dls[j] = 0.f;
   const int grow = row0 + r;
@@ -158,7 +158,8 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
         } else { z[j] = 0.f; inv_s[j] = 0.f; }
       }
       const float logp = quad - logdet;
-      const float ratio = expf(logp - a.logp_old[src]);                          // train.py:234
+      const float logr = logp - a.logp_old[src];
+      const float ratio = expf(logr);                                            // train.py:234
       const float adv_mean = (*a.adv_sum) * inv_n;
       const float adv_std = sqrtf((*a.adv_sq) * inv_n);
       const float adv = (a.adv[src] - adv_mean) / (adv_std + 1e-8f);             // train.py:235
@@ -169,6 +170,8 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
       const float w1 = l1 < l2 ? 1.f : (l1 == l2 ? 0.5f : 0.f);
       const float dmin = (w1 + (1.f - w1) * dclip(ratio, lo, hi)) * adv;
       const float g_logp = -inv_n * dmin * ratio;
+      s_kl = expm1f(logr) - logr;                                                // (r - 1) - log r without the cancellation
+      s_clip = fabsf(ratio - 1.f) > a.clip_eps ? 1.f : 0.f;
 #pragma unroll
       for (int j = 0; j < AMAX; ++j) {
         g_mean[j] = g_logp * (z[j] * inv_s[j]);
@@ -184,6 +187,7 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
       s_val = fmaxf(vl, vlc);
       const float wa = vl > vlc ? 1.f : (vl == vlc ? 0.5f : 0.f);
       g_v = a.vf_coef * 0.5f * inv_n * (wa * 2.f * e1 + (1.f - wa) * 2.f * e2 * dclip(dvv, -a.clip_eps, a.clip_eps));
+      s_vclip = fabsf(dvv) > a.clip_eps ? 1.f : 0.f;
     }
 #pragma unroll
     for (int j = 0; j < AMAX; ++j) gm[r * AMAX + j] = g_mean[j];
@@ -192,23 +196,21 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
   // reduce loss sums and dlog_std over the tile (fixed order: lanes, then warps)
 #pragma unroll
   for (int j = 0; j < AMAX; ++j) dls[j] = warp_sum(dls[j]);
-  s_val = warp_sum(s_val);
-  s_act = warp_sum(s_act);
+  const float sums[LOSS_SUMS] = {warp_sum(s_val), warp_sum(s_act), warp_sum(s_vclip), warp_sum(s_kl), warp_sum(s_clip)};
   if (lane == 0) {
 #pragma unroll
-    for (int j = 0; j < AMAX; ++j) red[warp * (AMAX + 4) + j] = dls[j];
-    red[warp * (AMAX + 4) + AMAX] = s_val;
-    red[warp * (AMAX + 4) + AMAX + 1] = s_act;
+    for (int j = 0; j < AMAX; ++j) red[warp * (AMAX + 8) + j] = dls[j];
+#pragma unroll
+    for (int j = 0; j < LOSS_SUMS; ++j) red[warp * (AMAX + 8) + AMAX + j] = sums[j];
   }
   __syncthreads();
 
   float* part_out = a.partials + static_cast<size_t>(tile) * a.partial_stride;
-  if (tid < AMAX + 2) {
+  if (tid < AMAX + LOSS_SUMS) {
     float s = 0.f;
-    for (int w = 0; w < HL_THREADS / 32; ++w) s += red[w * (AMAX + 4) + tid];
+    for (int w = 0; w < HL_THREADS / 32; ++w) s += red[w * (AMAX + 8) + tid];
     if (tid < A) part_out[a.po_logstd + tid] = s;
-    else if (tid == AMAX) part_out[a.po_loss + 0] = s;
-    else if (tid == AMAX + 1) part_out[a.po_loss + 1] = s;
+    else if (tid >= AMAX) part_out[a.po_loss + tid - AMAX] = s;
   }
   // head bias grads: db3a[j] = sum_r g_mean[r][j], db3c = sum_r g_v[r]
   if (tid < A + 1) {
@@ -258,9 +260,10 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
 constexpr size_t head_loss_smem_bytes(int H, int amax) {
   return static_cast<size_t>(2) * HL_ROWS * (H + 8) * 2 +
          static_cast<size_t>(amax > 32 ? HL_KCHUNK : H) * (amax + 1) * 4 + H * 4 +
-         HL_ROWS * amax * 4 + HL_ROWS * 4 + 8 * (amax + 4) * 4 + 64;
+         HL_ROWS * amax * 4 + HL_ROWS * 4 + 8 * (amax + 8) * 4 + 64;
 }
-// H = 512: 212,416 bytes with the 32-wide template, 220,608 with the 64-wide one (its W3a staged in 256-row chunks):
+static_assert(LOSS_SUMS <= 8, "head_loss_kernel: the loss sums share the 8 spare floats of a warp's row of red");
+// H = 512: 212,544 bytes with the 32-wide template, 220,736 with the 64-wide one (its W3a staged in 256-row chunks):
 // above 200 KB, within the 227 KB a block may opt in to
 constexpr int HL_SMEM_OPTIN = 227 * 1024;
 static_assert(head_loss_smem_bytes(MAX_HIDDEN, 32) <= HL_SMEM_OPTIN, "head_loss_kernel<32> shared memory at H = 512");

@@ -240,6 +240,7 @@ struct UpdatePtrs {
   const uint32_t* key_in;
   uint32_t* key_out;
   float* losses_out;
+  float* stats_out;
   bool operator==(const UpdatePtrs& o) const { return memcmp(this, &o, sizeof(*this)) == 0; }
 };
 
@@ -477,6 +478,7 @@ static void fill_fused_params(minppo_ctx* c, const UpdatePtrs& u, FusedParams* p
     g.po_w2 = net == 0 ? c->po_w3a : c->po_w3c;
     g.po_b2 = net == 0 ? c->po_b3a : c->po_b3c;
     g.po_loss = c->po_loss + (net == 0 ? 1 : 0);          // [0] = sum max(vl, vlc), [1] = sum min(l1, l2)
+    g.po_stat = c->po_loss + (net == 0 ? 3 : 2);          // [2] value-clip count; [3] approx-KL sum, [4] ratio-clip count
     g.po_db0 = c->po_db[net][0]; g.po_db1 = c->po_db[net][1];
   }
   p.rowidx = c->rowidx; p.obs_img = c->obs_img; p.count = c->counts; p.step = 0;
@@ -544,6 +546,7 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
   dp.opt.losses_out = u.losses_out ? u.losses_out : c->losses_scratch;
   dp.losses_stride = u.losses_out ? 4 : 0;
   dp.opt.gnorm_out = c->gnorms;
+  dp.opt.stats_out = u.stats_out;
   dp.ridx_base = c->rowidx; dp.counts = c->counts; dp.cap = c->cap; dp.EM = c->E * c->M;
   dp.padded = c->padded ? 1 : 0;
   dp.part_rows = c->fused ? 128 : 64;
@@ -553,7 +556,7 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
 }
 
 // The NCCL fallback's second dwopt launch, which only applies the all-reduced gradient: gflat holds it (P floats, then the
-// two loss sums), and it becomes the single partial of every leaf and of the loss sums.  The reduction phase then copies
+// LOSS_SUMS loss sums), and it becomes the single partial of every leaf and of the loss sums.  The reduction phase then copies
 // gflat onto itself and forms the global norm; phase 3 runs clip + Adam and writes the weight images as usual.  Every leaf
 // is "early": the late path issues 16-byte loads, and gflat + a leaf offset is only 4-byte aligned.  grad_bias is 0
 // because rank 0 added -ent_coef to the log_std gradient before the all-reduce, and padded is 0 because the live-tile
@@ -722,7 +725,7 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
   }
   RET(launch_dwopt());
   if (nccl) {
-    { PROF(PC_ALLREDUCE); RET(nccl_allreduce(c, c->gflat, static_cast<size_t>(c->P) + 2, stream)); }
+    { PROF(PC_ALLREDUCE); RET(nccl_allreduce(c, c->gflat, static_cast<size_t>(c->P) + LOSS_SUMS, stream)); }
     c->launches++;
     fill_apply_only(c, &dp);
     RET(launch_dwopt());
@@ -995,7 +998,7 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
     c->po_logstd = o; o += A;
     for (int net = 0; net < 2; ++net)
       for (int l = 0; l < 2; ++l) { c->po_db[net][l] = o; o += H; }
-    c->po_loss = o; o += 2;
+    c->po_loss = o; o += LOSS_SUMS;
     c->head_stride = (o + 3) / 4 * 4;
   }
   const int EM = c->E * c->M;
@@ -1007,7 +1010,7 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   if (cfg->world_size > 1) {
     // the local gradient buffer lives inside the exchange allocation so that peers can read it (own cudaMalloc:
     // CUDA IPC exports whole allocations)
-    const int np = static_cast<int>((c->P + 2 + 3) / 4 * 4);
+    const int np = static_cast<int>((c->P + LOSS_SUMS + 3) / 4 * 4);
     const size_t floats = 2 * static_cast<size_t>(cfg->world_size) * np + static_cast<size_t>(cfg->world_size) * 256 + 2 * static_cast<size_t>(np);
     ALLOC(c->xchg, floats);
     // staging / result words start as the "not yet written" sentinel -0.0f of the Lamport-style exchange (dwopt.cuh)
@@ -1015,7 +1018,7 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
     ALLOC(c->xseq, 1);
     c->px.np = np; c->px.world = 0; c->px.rank = cfg->rank; c->px.seq = c->xseq;
   }
-  ALLOC(c->gflat, static_cast<size_t>(c->P) + 4);
+  ALLOC(c->gflat, static_cast<size_t>(c->P) + 8);
   ALLOC(c->block_ss, static_cast<size_t>(c->sm_count));
   ALLOC(c->head_part, static_cast<size_t>(c->tiles64) * c->head_stride);
   ALLOC(c->gnorms, static_cast<size_t>(EM));
@@ -1108,10 +1111,10 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   return 0;
 }
 
-int minppo_update(minppo_ctx* c, float* params, float* mu, float* nu, int32_t* count, const float* obs,
-                  const float* action, const float* value, const float* reward, const float* log_prob,
-                  const uint8_t* done, const float* last_val, const uint32_t* key_in, uint32_t* key_out,
-                  float* losses_out, int32_t use_graph, void* stream_v) {
+int minppo_update_with_stats(minppo_ctx* c, float* params, float* mu, float* nu, int32_t* count, const float* obs,
+                             const float* action, const float* value, const float* reward, const float* log_prob,
+                             const uint8_t* done, const float* last_val, const uint32_t* key_in, uint32_t* key_out,
+                             float* losses_out, float* stats_out, int32_t use_graph, void* stream_v) {
   if (!c || !params || !mu || !nu || !count || !obs || !action || !value || !reward || !log_prob || !done ||
       !last_val || !key_in) {
     set_error("minppo_update: null pointer");
@@ -1122,7 +1125,7 @@ int minppo_update(minppo_ctx* c, float* params, float* mu, float* nu, int32_t* c
   memset(&u, 0, sizeof(u));
   u.params = params; u.mu = mu; u.nu = nu; u.count = count; u.obs = obs; u.action = action; u.value = value;
   u.reward = reward; u.log_prob = log_prob; u.done = done; u.last_val = last_val; u.key_in = key_in;
-  u.key_out = key_out; u.losses_out = losses_out;
+  u.key_out = key_out; u.losses_out = losses_out; u.stats_out = stats_out;
   if (!use_graph) return enqueue_update(c, u, stream);
   const bool was_profiling = c->profiling;
   c->profiling = false;                         // event records are not captured; profile in eager mode
@@ -1155,6 +1158,14 @@ int minppo_update(minppo_ctx* c, float* params, float* mu, float* nu, int32_t* c
   c->launches = c->graphs.back().launches;
   CK(cudaGraphLaunch(c->graphs.back().exec, stream));
   return 0;
+}
+
+int minppo_update(minppo_ctx* c, float* params, float* mu, float* nu, int32_t* count, const float* obs,
+                  const float* action, const float* value, const float* reward, const float* log_prob,
+                  const uint8_t* done, const float* last_val, const uint32_t* key_in, uint32_t* key_out,
+                  float* losses_out, int32_t use_graph, void* stream_v) {
+  return minppo_update_with_stats(c, params, mu, nu, count, obs, action, value, reward, log_prob, done, last_val, key_in,
+                                  key_out, losses_out, nullptr, use_graph, stream_v);
 }
 
 int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, const uint32_t* key_in, uint32_t* key_out,

@@ -17,6 +17,13 @@ constexpr int MAX_HIDDEN = 512;
 // widest act_dim: above 32 (FS_MAX_AP) the heads run on the layer-wise kernels' 64-wide templates
 constexpr int MAX_ACT_DIM = 64;
 
+// Per-minibatch sums the loss kernels hand to the optimizer kernel: a block of LOSS_SUMS floats in every per-tile partial
+// (at po_loss), reduced in fixed order into gflat[P + i] and, on env-sharded ranks, all-reduced with the gradient:
+//   [0] sum max(vl, vlc)   [1] sum min(l1, l2)   [2] value-clip count |v - v_old| > clip_eps
+//   [3] approx-KL sum of expm1(log r) - log r    [4] ratio-clip count |r - 1| > clip_eps
+// [0], [1] are the loss sums; [2..4] exist only for the per-step statistics (minppo_update_with_stats) and feed nothing else.
+constexpr int LOSS_SUMS = 5;
+
 // ---- gae.cu ------------------------------------------------------------------------------
 void gae_plan(int T, long long N, int sm_count, int* vec, int* chunks, int* seg_len);
 int gae_launch(const float* reward, const float* value, const uint8_t* done, const float* last_val, float* adv,
@@ -122,8 +129,8 @@ struct OptArgs {
   int nleaves, P, A;
   int n_early;                   // elements of the leaves with late == 0
   int do_apply;
-  float* gflat;                  // [P + 4] reduced gradient (minppo_ctx_read buffer 3 returns the last one), then the loss sums
-  const float* loss_src;         // loss partial sums (2 per partial)
+  float* gflat;                  // [P + 8] reduced gradient (minppo_ctx_read buffer 3 returns the last one), then the LOSS_SUMS sums
+  const float* loss_src;         // loss partial sums (LOSS_SUMS per partial)
   int loss_src_offset, loss_nparts, loss_part_stride;
   float* params; float* mu; float* nu;
   int32_t* count;
@@ -131,6 +138,7 @@ struct OptArgs {
   unsigned long long* barrier;
   int* err_flag;
   float* losses_out;             // [4] or null
+  float* stats_out;              // [E * M][4] per-step statistics (approx_kl, clip_fraction, value_clip_fraction, grad_norm) or null
   float* gnorm_out;              // [1] or null
   int off_logstd;
   int anneal, anneal_div, num_updates;

@@ -149,7 +149,7 @@ MINPPO_DEVINL float4 sum_partials16_v4(const float* __restrict__ src, int nparts
 
 // Gradient reduction of one class of leaves -> gflat; returns this thread's sum of squares.
 //   LATE == false: leaves whose partials the fused step kernel wrote (biases of the output heads, head
-//                  kernels, log_std, ...): one element per job, then the two loss sums.
+//                  kernels, log_std, ...): one element per job, then the LOSS_SUMS loss sums.
 //   LATE == true : leaves whose partials the dW GEMM writes (hidden kernels): four
 //                  elements per job (sizes and partial strides are multiples of 4, partial buffers 16-byte
 //                  aligned; gflat itself is only 4-byte aligned at a leaf offset).
@@ -171,7 +171,7 @@ MINPPO_DEVINL float reduce_leaves(const OptArgs& a, const LeafTab& T, int first,
       if (l < nl) n = LATE ? (T.size[l] >> 2) : T.size[l];
     }
     if (l >= nl) {
-      if (!LATE && j - base < 2)          // the loss sums ride behind the early leaves
+      if (!LATE && j - base < LOSS_SUMS)  // the loss sums ride behind the early leaves
         a.gflat[a.P + (j - base)] = sum_partials16(a.loss_src + a.loss_src_offset + (j - base), min(a.loss_nparts, max_parts), a.loss_part_stride);
       break;
     }

@@ -54,6 +54,10 @@ class TrainState:
         return TrainState(p, torch.zeros_like(p), torch.zeros_like(p), torch.zeros(1, dtype=torch.int32, device=device))
 
 
+# columns of the per-minibatch statistics ``Learner.update(..., stats=...)`` writes (include/minppo_b200.h)
+STATS_COLUMNS = ("approx_kl", "clip_fraction", "value_clip_fraction", "grad_norm")
+
+
 def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
 
@@ -213,9 +217,16 @@ class Learner:
 
     # -- the update -----------------------------------------------------------------------
     def update(self, train_state: TrainState, mem_batch: Memory, last_val: torch.Tensor, rng: torch.Tensor,
-               losses: Optional[torch.Tensor] = None, rng_out: Optional[torch.Tensor] = None):
+               losses: Optional[torch.Tensor] = None, rng_out: Optional[torch.Tensor] = None,
+               stats: Optional[torch.Tensor] = None):
         """train.py:185-281.  In place on ``train_state``; returns (train_state, rng', losses[E, M, 4])
         with losses columns (total, value_loss, actor_loss, entropy).  Nothing synchronises.
+
+        ``stats``: optional caller-owned f32 [E, M, 4] device tensor, filled in place with per-minibatch diagnostics,
+        columns ``STATS_COLUMNS``: approx_kl = mean(expm1(log r) - log r), clip_fraction = mean(|r - 1| > clip_eps),
+        value_clip_fraction = mean(|v - v_old| > clip_eps) over the rows of the global minibatch, evaluated with the
+        parameters before that minibatch's Adam step, and the pre-clip global gradient norm.  Passing it changes
+        nothing else the update computes.
 
         ``rng`` is copied (8 bytes, stream-ordered) into a learner-owned slot; without ``losses`` / ``rng_out`` the
         results land in learner-owned buffers that the NEXT ``update`` overwrites (pass your own to keep them).  With
@@ -240,15 +251,17 @@ class Learner:
             losses = self._losses
         else:
             _check(losses, "losses", torch.float32, (self.E, self.M, 4), dev)
+        if stats is not None:
+            _check(stats, "stats", torch.float32, (self.E, self.M, len(STATS_COLUMNS)), dev)
         if rng_out is None:
             rng_out = self._key_out.view(rng.dtype)
         with torch.cuda.device(dev):
             if rng.data_ptr() != self._key_in.data_ptr():
                 self._key_in.copy_(rng.reshape(2).view(torch.int32), non_blocking=True)
-            _lib.check(self.lib.minppo_update(
+            _lib.check(self.lib.minppo_update_with_stats(
                 self._h, _ptr(train_state.params), _ptr(train_state.mu), _ptr(train_state.nu), _ptr(train_state.step),
                 _ptr(obs), _ptr(action), _ptr(value), _ptr(reward), _ptr(log_prob), _ptr(done), _ptr(last_val),
-                _ptr(self._key_in), _ptr(rng_out), _ptr(losses), int(self.use_graph), _stream_ptr(dev)))
+                _ptr(self._key_in), _ptr(rng_out), _ptr(losses), _ptr(stats), int(self.use_graph), _stream_ptr(dev)))
         return train_state, rng_out, losses
 
     # -- policy / value inference for the rollout -------------------------------------------
