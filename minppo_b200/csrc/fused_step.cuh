@@ -37,6 +37,7 @@
 
 #include "common.cuh"
 #include "minppo_internal.h"
+#include "ppo_math.cuh"
 #include "umma_gemm.cuh"
 
 namespace minppo {
@@ -97,22 +98,13 @@ struct alignas(64) FusedParams {
   FusedNet net[2];
   CUtensorMap tm_xg;             // gathered observation rows [M_pad][Dp], box {64, 128}: TMA store by the critic CTAs,
                                  // the A operand of both nets' first-layer weight-gradient GEMM
-  const int32_t* rowidx;         // [E*M][cap] row lists of ALL minibatch steps of the update
+  // (obs_img ahead of loss keeps the pointer pairs the compiler fetches with one 16-byte constant load, and the kernel's code)
   const __nv_bfloat16* obs_img;  // [Bl][Dp]
-  const int32_t* count;          // [E*M]
-  const float* adv_sum;          // [E*M]
-  const float* adv_sq;           // [E*M]
-  const float* action;
-  const float* v_old;
-  const float* logp_old;
-  const float* adv;
-  const float* tgt;
+  LossOperands loss;             // its row lists also gather the observation rows
   const float* log_std;          // arena pointer
   float* part;                   // per-tile partials [m_tiles][part_stride]
   int part_stride, po_logstd;
-  int H, A, Dp, m_tiles, cap;
-  int step;                      // minibatch step e * M + k of this launch
-  float inv_mb, clip_eps, vf_coef;
+  int H, A, Dp, m_tiles;
   long long* trace;              // debug: [ctas][32] clock64 stamps (null = off)
 };
 
@@ -195,9 +187,6 @@ MINPPO_DEVINL float act_apply(float x) {
 }
 template <int ACT>
 MINPPO_DEVINL float act_deriv_t(float h) { return ACT == ACT_RELU ? (h > 0.f ? 1.f : 0.f) : (1.f - h * h); }
-MINPPO_DEVINL float dclip_f(float x, float lo, float hi) {
-  return (x > lo && x < hi) ? 1.f : ((x == lo || x == hi) ? 0.5f : 0.f);
-}
 // The four epilogues walk `nchunks` 16-column chunks of an accumulator, chunk i at column col0 + i * cstride, and (bars != null)
 // publish chunk i on bars[i] as soon as it is in shared memory.  The TMEM read of chunk i + 1 is issued before chunk i is
 // processed (one tcgen05.ld outstanding at every tcgen05.wait::ld): with four warps per scheduler the read latency is
@@ -346,8 +335,9 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
   uint64_t* dz2r = bars + 45;           // [4] dZ2 columns [64 b, 64 b + 64) in R1 (k-block b of the dH1 GEMM)
   uint64_t* dz1r = bars + 49;           // [4] dZ1 columns [64 b, 64 b + 64) in R1
   uint64_t* x_stored = bars + 53;       // [4] the TMA store of the X k-block in slot s (for the dW GEMM) has read the slot
-  const int32_t* rowidx_s = p.rowidx + static_cast<size_t>(step) * p.cap;     // this step's row list
-  const int32_t* count_s = p.count + step;
+  const LossOperands& L = p.loss;
+  const int32_t* rowidx_s = L.rowidx + static_cast<size_t>(step) * L.cap;   // this step's row list
+  const int32_t* count_s = L.count + step;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   // CTA order: (tile, net) with net fastest, so that the LIVE tiles of both nets are the lowest block indices and fit the
@@ -364,7 +354,7 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
 
   // Env-sharded ranks size the row lists for the worst case (learner.cu: 1.5 x the mean + 256 rows); the tiles
   // beyond this minibatch's actual row count have nothing to do except zeroing their partial sums.
-  if (tile * 128 >= min(*count_s, p.cap)) {
+  if (tile * 128 >= min(*count_s, L.cap)) {
     griddep_wait();                                     // the previous optimizer step may still be reading the partials
     float* part = p.part + static_cast<size_t>(tile) * p.part_stride;
     for (int i = threadIdx.x; i < H * G.aout; i += FS_THREADS) part[G.po_w2 + i] = 0.f;
@@ -592,7 +582,7 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
     for (int g = 0; g < 2; ++g) src_g[g] = rowidx_s[tile * 128 + grow0 + 64 * g];
     const int lrow = tile * 128 + erow;                          // loss row of this thread (actor: the four warps of a lane
                                                                  // quadrant share a row, AP / 4 head columns each; critic: sub == 0)
-    const int count = min(*count_s, p.cap);
+    const int count = min(*count_s, L.cap);
     const bool live = (sub == 0 || net == 0) && (lrow < count);
     const int src_l = live ? rowidx_s[lrow] : 0;
     // one warp instruction copies 4 rows x 128 contiguous bytes (4 L1 wavefronts; a lane-per-row mapping needed 32)
@@ -608,7 +598,7 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
     const int nb0 = nk0 < FS_XSLOTS ? nk0 : FS_XSLOTS;
     for (int kb = 0; kb < nb0; ++kb) gather_block(kb);
     if (wt == 0) FS_STAMP(26);
-    const float adv_sum = p.adv_sum[step], adv_sq = p.adv_sq[step];
+    const float adv_sum = L.adv_sum[step], adv_sq = L.adv_sq[step];
     // per-row loss inputs (update-static: old log-prob / value, advantage / target, action), requested BEFORE the dependency
     // wait: under PDL this part of the kernel runs while the previous optimizer step drains, so the loads -- each touches 32
     // distinct lines -- are off the critical path.  Measured (configs[1], ms per update): here 5.48; after the X rows are
@@ -621,8 +611,8 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
     for (int j = 0; j < CW; ++j) zz[j] = 0.f;
     if (live) {
       if (net == 0) {
-        in0 = p.logp_old[src_l]; in1 = p.adv[src_l];
-        const float* ap = p.action + static_cast<size_t>(src_l) * aout + j0;
+        in0 = L.logp_old[src_l]; in1 = L.adv[src_l];
+        const float* ap = L.action + static_cast<size_t>(src_l) * aout + j0;
         if ((aout & 1) == 0) {                                     // rows are 8-byte aligned: half the load wavefronts
 #pragma unroll
           for (int j = 0; j < CW; j += 2)
@@ -632,7 +622,7 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
           for (int j = 0; j < CW; ++j) if (j0 + j < aout) zz[j] = ap[j];
         }
       } else {
-        in0 = p.v_old[src_l]; in1 = p.tgt[src_l];
+        in0 = L.v_old[src_l]; in1 = L.tgt[src_l];
       }
     }
 
@@ -738,7 +728,6 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
     float st_a = 0.f, st_b = 1.f;
     {
       const uint32_t th = acc_head + (static_cast<uint32_t>(q * 32) << 16);
-      const float inv_n = p.inv_mb;
       // g^T as bf16 hi/lo, [2AP j][128 rows] SW128 (the MN-major A of dA2 and the K-major B of dW2)
       const uint32_t gcol = GT + (erow >> 6) * PG + ((erow & 7) << 1);
       const int gch = (erow & 63) >> 3;
@@ -762,7 +751,7 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
           const float mean = (ohi[jj] + olo[jj]) + hb[j];                   // W2_hi and W2_lo contributions
           const float z = j < aout ? (zz[jj] - mean) * hb[2 * AP + j] : 0.f;
           zz[jj] = z;
-          if (j < aout) quad += -0.5f * z * z - 0.91893853320467274178f;
+          if (j < aout) quad += gauss_logp_term(z);
         }
         // qp aliases the hidden biases, last read in epilogue 2.  Every warp's reads precede its h2r arrivals, which precede
         // the head MMAs, headf and this point -- an mbarrier / tcgen05.commit chain that compute-sanitizer's racecheck does not
@@ -773,20 +762,8 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
         quad = ((qp[erow] + qp[128 + erow]) + qp[256 + erow]) + qp[384 + erow];   // fixed order: column groups 0..3
         float s_loss = 0.f, g_logp = 0.f;
         if (live) {
-          const float logp = quad - hb[3 * AP];
-          const float logr = logp - in0;
-          const float ratio = expf(logr);
-          const float adv_mean = adv_sum * inv_n;
-          const float adv_std = sqrtf(adv_sq * inv_n);
-          const float adv = (in1 - adv_mean) / (adv_std + 1e-8f);                 // train.py:235
-          const float lo = 1.f - p.clip_eps, hi = 1.f + p.clip_eps;
-          const float l1 = ratio * adv;
-          const float l2 = fminf(fmaxf(ratio, lo), hi) * adv;
-          s_loss = fminf(l1, l2);
-          const float w1 = l1 < l2 ? 1.f : (l1 == l2 ? 0.5f : 0.f);
-          const float dmin = (w1 + (1.f - w1) * dclip_f(ratio, lo, hi)) * adv;
-          g_logp = -inv_n * dmin * ratio;
-          st_a = logr; st_b = ratio;
+          const PpoActorRow ar = ppo_actor_row(quad - hb[3 * AP], in0, in1, adv_sum, adv_sq, L.inv_mb, L.clip_eps);
+          s_loss = ar.loss; g_logp = ar.g_logp; st_a = ar.logr; st_b = ar.ratio;
         }
         // tile sums of dlog_std and of the head-bias gradient g through a 2 CW x 32 transpose-reduce
         float v[2 * CW];
@@ -811,16 +788,8 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
         tmem_ld_wait();
         float s_loss = 0.f, g0 = 0.f;
         if (live) {
-          // clipped value loss, train.py:226-231
-          const float v = (ohi + olo) + hb[0];
-          const float dvv = v - in0;
-          const float v_clip = in0 + fminf(fmaxf(dvv, -p.clip_eps), p.clip_eps);
-          const float e1 = v - in1, e2 = v_clip - in1;
-          const float vl = e1 * e1, vlc = e2 * e2;
-          s_loss = fmaxf(vl, vlc);
-          const float wa = vl > vlc ? 1.f : (vl == vlc ? 0.5f : 0.f);
-          g0 = p.vf_coef * 0.5f * inv_n * (wa * 2.f * e1 + (1.f - wa) * 2.f * e2 * dclip_f(dvv, -p.clip_eps, p.clip_eps));
-          st_a = dvv;
+          const PpoValueRow vr = ppo_value_row((ohi + olo) + hb[0], in0, in1, L.inv_mb, L.clip_eps, L.vf_coef);
+          s_loss = vr.loss; g0 = vr.g_v; st_a = vr.dv;
         }
         put_g(0, g0);
         const float gs = warp_sum(g0);
@@ -833,18 +802,17 @@ MINPPO_DEVINL void fused_tile(const FusedParams& p, int unit, int step, uint8_t*
     tc_fence_before();
     __syncwarp();
     if (lane == 0) mbar_arrive(gr);
-    // statistics sums, off the path to the dA2 / dW2 MMAs that g^T starts: red[q][2 AP + 1, 2 AP + 3) (po_stat).  Actor:
-    // approx-KL term (r - 1) - log r as expm1 (no cancellation at small log r) and |r - 1| > clip_eps; critic:
-    // |v - v_old| > clip_eps.  The four warps of an actor lane quadrant hold the same rows: warp sub == 0 sums them.
+    // statistics sums, off the path to the dA2 / dW2 MMAs that g^T starts: red[q][2 AP + 1, 2 AP + 3) (po_stat).  The four
+    // warps of an actor lane quadrant hold the same rows: warp sub == 0 sums them.
     if (sub == 0) {
       float* rw = red + q * RS + 2 * AP + 1;
       if (net == 0) {
-        const float kl = live ? expm1f(st_a) - st_a : 0.f;
-        const float clipped = live && fabsf(st_b - 1.f) > p.clip_eps ? 1.f : 0.f;
+        const float kl = live ? approx_kl_term(st_a) : 0.f;
+        const float clipped = live ? ratio_clipped(st_b, L.clip_eps) : 0.f;
         const float s_kl = warp_sum(kl), s_clip = warp_sum(clipped);
         if (lane == 0) { rw[0] = s_kl; rw[1] = s_clip; }
       } else {
-        const float s_vclip = warp_sum(live && fabsf(st_a) > p.clip_eps ? 1.f : 0.f);
+        const float s_vclip = warp_sum(live ? value_clipped(st_a, L.clip_eps) : 0.f);
         if (lane == 0) rw[0] = s_vclip;
       }
     }
@@ -954,7 +922,7 @@ __global__ void __launch_bounds__(FS_THREADS, 1) fused_step_kernel(const __grid_
   uint8_t* sm = smem_raw + (base - raw);
   const int warp = threadIdx.x >> 5;
   const int unit = static_cast<int>(blockIdx.x);
-  if ((unit >> 1) * 128 < min(p.count[p.step], p.cap)) {          // live tile: needs the tensor memory
+  if ((unit >> 1) * 128 < min(p.loss.count[p.loss.step], p.loss.cap)) {   // live tile: needs the tensor memory
     if (warp == FS_MMA_WARP) {
       tmem_alloc(&tmem_slot, 512);
       tmem_relinquish();
@@ -963,10 +931,10 @@ __global__ void __launch_bounds__(FS_THREADS, 1) fused_step_kernel(const __grid_
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = tmem_slot;
-    fused_tile<AP>(p, unit, p.step, sm, base, tmem_base);
+    fused_tile<AP>(p, unit, p.loss.step, sm, base, tmem_base);
     if (warp == FS_MMA_WARP) tmem_dealloc(tmem_base, 512);
   } else {
-    fused_tile<AP>(p, unit, p.step, sm, base, 0u);                // dead tile: zeroes its partials and returns
+    fused_tile<AP>(p, unit, p.loss.step, sm, base, 0u);                      // dead tile: zeroes its partials and returns
   }
 }
 

@@ -18,6 +18,7 @@
 // arena.  Every thread accumulates the same terms in the same order as with the whole kernel resident.
 #include "common.cuh"
 #include "minppo_internal.h"
+#include "ppo_math.cuh"
 
 namespace minppo {
 
@@ -25,11 +26,6 @@ constexpr int HL_ROWS = 64;
 constexpr int HL_THREADS = 256;
 constexpr int HL_KCHUNK = 256;          // rows of W3a per phase-1 stage (AMAX > 32)
 static_assert(HL_KCHUNK % 8 == 0, "phase 1 steps k by 8 across a quad");
-
-MINPPO_DEVINL float dclip(float x, float lo, float hi) {
-  // d/dx min(max(x, lo), hi) with the 0.5/0.5 tie split of jnp.minimum / jnp.maximum
-  return (x > lo && x < hi) ? 1.f : ((x == lo || x == hi) ? 0.5f : 0.f);
-}
 
 // rows [k0, k0 + rows) of the head kernel W3a -> w3a[rows][AMAX + 1], columns >= A zero
 template <int AMAX>
@@ -57,7 +53,9 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int tile = blockIdx.x;
   const int row0 = tile * HL_ROWS;
-  const int count = min(*a.count, a.cap);
+  const LossOperands& L = a.loss;
+  const int32_t* rowidx_s = L.rowidx + static_cast<size_t>(L.step) * L.cap;   // this step's row list
+  const int count = min(L.count[L.step], L.cap);
   const float* P = a.params;
 
   // ---- stage weights and the two activation tiles --------------------------------------
@@ -141,9 +139,7 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
 #pragma unroll
     for (int j = 0; j < AMAX; ++j) g_mean[j] = 0.f;
     if (live) {
-      const int src = a.rowidx[grow];
-      const float inv_n = a.inv_mb;
-      // distrax: z = (a - loc) * (1/scale); log_prob = sum(-z^2/2 - log(2pi)/2) - sum(log|scale|)
+      const int src = rowidx_s[grow];
       float z[AMAX], inv_s[AMAX];
       float quad = 0.f, logdet = 0.f;
 #pragma unroll
@@ -152,42 +148,21 @@ __global__ void __launch_bounds__(HL_THREADS) head_loss_kernel(const HeadLossArg
           const float scale = expf(P[a.off.logstd + j]);
           inv_s[j] = 1.f / scale;
           const float mean = acc[j] + P[a.off.b3a + j];
-          z[j] = (a.action[static_cast<size_t>(src) * A + j] - mean) * inv_s[j];
-          quad += -0.5f * z[j] * z[j] - 0.91893853320467274178f;
+          z[j] = (L.action[static_cast<size_t>(src) * A + j] - mean) * inv_s[j];
+          quad += gauss_logp_term(z[j]);
           logdet += logf(fabsf(scale));
         } else { z[j] = 0.f; inv_s[j] = 0.f; }
       }
-      const float logp = quad - logdet;
-      const float logr = logp - a.logp_old[src];
-      const float ratio = expf(logr);                                            // train.py:234
-      const float adv_mean = (*a.adv_sum) * inv_n;
-      const float adv_std = sqrtf((*a.adv_sq) * inv_n);
-      const float adv = (a.adv[src] - adv_mean) / (adv_std + 1e-8f);             // train.py:235
-      const float lo = 1.f - a.clip_eps, hi = 1.f + a.clip_eps;
-      const float l1 = ratio * adv;
-      const float l2 = fminf(fmaxf(ratio, lo), hi) * adv;                        // train.py:237
-      s_act = fminf(l1, l2);                                                     // train.py:238
-      const float w1 = l1 < l2 ? 1.f : (l1 == l2 ? 0.5f : 0.f);
-      const float dmin = (w1 + (1.f - w1) * dclip(ratio, lo, hi)) * adv;
-      const float g_logp = -inv_n * dmin * ratio;
-      s_kl = expm1f(logr) - logr;                                                // (r - 1) - log r without the cancellation
-      s_clip = fabsf(ratio - 1.f) > a.clip_eps ? 1.f : 0.f;
+      const PpoActorRow ar = ppo_actor_row(quad - logdet, L.logp_old[src], L.adv[src], L.adv_sum[L.step], L.adv_sq[L.step],
+                                           L.inv_mb, L.clip_eps);
+      s_act = ar.loss; s_kl = approx_kl_term(ar.logr); s_clip = ratio_clipped(ar.ratio, L.clip_eps);
 #pragma unroll
       for (int j = 0; j < AMAX; ++j) {
-        g_mean[j] = g_logp * (z[j] * inv_s[j]);
-        dls[j] = g_logp * (z[j] * z[j] - 1.f);
+        g_mean[j] = ar.g_logp * (z[j] * inv_s[j]);
+        dls[j] = ar.g_logp * (z[j] * z[j] - 1.f);
       }
-      // value loss, train.py:226-231
-      const float v = accv + P[a.off.b3c];
-      const float v_old = a.v_old[src], tgt = a.tgt[src];
-      const float dvv = v - v_old;
-      const float v_clip = v_old + fminf(fmaxf(dvv, -a.clip_eps), a.clip_eps);
-      const float e1 = v - tgt, e2 = v_clip - tgt;
-      const float vl = e1 * e1, vlc = e2 * e2;
-      s_val = fmaxf(vl, vlc);
-      const float wa = vl > vlc ? 1.f : (vl == vlc ? 0.5f : 0.f);
-      g_v = a.vf_coef * 0.5f * inv_n * (wa * 2.f * e1 + (1.f - wa) * 2.f * e2 * dclip(dvv, -a.clip_eps, a.clip_eps));
-      s_vclip = fabsf(dvv) > a.clip_eps ? 1.f : 0.f;
+      const PpoValueRow vr = ppo_value_row(accv + P[a.off.b3c], L.v_old[src], L.tgt[src], L.inv_mb, L.clip_eps, L.vf_coef);
+      s_val = vr.loss; s_vclip = value_clipped(vr.dv, L.clip_eps); g_v = vr.g_v;
     }
 #pragma unroll
     for (int j = 0; j < AMAX; ++j) gm[r * AMAX + j] = g_mean[j];

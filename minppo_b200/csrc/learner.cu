@@ -460,7 +460,15 @@ static int nccl_allreduce(minppo_ctx* c, float* buf, size_t n, cudaStream_t stre
 }
 
 // ---- parameter blocks of the per-minibatch kernels ----
-static void fill_fused_params(minppo_ctx* c, const UpdatePtrs& u, FusedParams* pp) {
+static void fill_loss_operands(const minppo_ctx* c, const UpdatePtrs& u, int s, LossOperands* lo) {
+  lo->rowidx = c->rowidx; lo->count = c->counts; lo->cap = c->cap; lo->step = s;
+  lo->adv_sum = c->stats; lo->adv_sq = c->stats + c->E * c->M;
+  lo->action = u.action; lo->v_old = u.value; lo->logp_old = u.log_prob; lo->adv = c->adv; lo->tgt = c->tgt;
+  lo->inv_mb = static_cast<float>(1.0 / c->mb);
+  lo->clip_eps = static_cast<float>(c->cfg.clip_eps); lo->vf_coef = static_cast<float>(c->cfg.vf_coef);
+}
+
+static void fill_fused_params(minppo_ctx* c, const UpdatePtrs& u, int s, FusedParams* pp) {
   FusedParams& p = *pp;
   memset(&p, 0, sizeof(p));
   const int H = c->H;
@@ -481,15 +489,11 @@ static void fill_fused_params(minppo_ctx* c, const UpdatePtrs& u, FusedParams* p
     g.po_stat = c->po_loss + (net == 0 ? 3 : 2);          // [2] value-clip count; [3] approx-KL sum, [4] ratio-clip count
     g.po_db0 = c->po_db[net][0]; g.po_db1 = c->po_db[net][1];
   }
-  p.rowidx = c->rowidx; p.obs_img = c->obs_img; p.count = c->counts; p.step = 0;
-  p.tm_xg = c->m_xg_k;
-  p.adv_sum = c->stats; p.adv_sq = c->stats + c->E * c->M;
-  p.action = u.action; p.v_old = u.value; p.logp_old = u.log_prob; p.adv = c->adv; p.tgt = c->tgt;
+  fill_loss_operands(c, u, s, &p.loss);
+  p.obs_img = c->obs_img; p.tm_xg = c->m_xg_k;
   p.log_std = u.params + c->head.logstd;
   p.part = c->head_part; p.part_stride = c->head_stride; p.po_logstd = c->po_logstd;
-  p.H = H; p.A = c->A; p.Dp = c->Dp; p.m_tiles = c->m_tiles; p.cap = c->cap;
-  p.inv_mb = static_cast<float>(1.0 / c->mb);
-  p.clip_eps = static_cast<float>(c->cfg.clip_eps); p.vf_coef = static_cast<float>(c->cfg.vf_coef);
+  p.H = H; p.A = c->A; p.Dp = c->Dp; p.m_tiles = c->m_tiles;
   p.trace = c->trace_on ? c->trace : nullptr;
 }
 
@@ -626,8 +630,7 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
   if (c->fused) {
     // forward + heads + loss + backward-to-dZ of both nets in one launch (fused_step.cuh)
     FusedParams p;
-    fill_fused_params(c, u, &p);
-    p.step = s;
+    fill_fused_params(c, u, s, &p);
     PROF(PC_FWD_GEMM);
     const cudaError_t e = c->ap == 16
         ? launch_kernel(fused_step_kernel<16>, 2 * c->m_tiles, FS_THREADS, FsLayout<16>::BYTES, stream, pdl, p)
@@ -652,17 +655,14 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
     memset(&a, 0, sizeof(a));
     a.h_a = c->net[0].act[L]; a.h_c = c->net[1].act[L];
     a.dz_a = c->net[0].dz[L]; a.dz_c = c->net[1].dz[L];
-    a.params = u.params; a.rowidx = ridx; a.count = c->counts + s;
-    a.adv_sum = c->stats + s; a.adv_sq = c->stats + c->E * c->M + s;
-    a.action = u.action; a.v_old = u.value; a.logp_old = u.log_prob; a.adv = c->adv; a.tgt = c->tgt;
+    a.params = u.params;
+    fill_loss_operands(c, u, s, &a.loss);
     a.partials = c->head_part; a.partial_stride = c->head_stride;
     a.po_w3a = c->po_w3a; a.po_b3a = c->po_b3a; a.po_w3c = c->po_w3c; a.po_b3c = c->po_b3c;
     a.po_logstd = c->po_logstd; a.po_loss = c->po_loss;
     a.off = c->head;
-    a.H = H; a.A = c->A; a.ldh = H; a.cap = c->cap;
+    a.H = H; a.A = c->A; a.ldh = H;
     a.act_a = act_kind(c, 0) == ACT_RELU ? ACTK_RELU : ACTK_TANH; a.act_c = ACTK_RELU;
-    a.inv_mb = static_cast<float>(1.0 / c->mb);
-    a.clip_eps = static_cast<float>(c->cfg.clip_eps); a.vf_coef = static_cast<float>(c->cfg.vf_coef);
     PROF(PC_HEAD_LOSS);
     RET(head_loss_launch(a, c->tiles64, stream));
     c->launches++;

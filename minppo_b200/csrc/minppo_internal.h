@@ -54,6 +54,23 @@ struct HeadOffsets {
   int w3a, b3a, w3c, b3c, logstd;
 };
 
+// Inputs of the PPO loss of one minibatch step (ppo_math.cuh), read by the fused step kernel and head_loss_kernel.  The row
+// lists and sums cover every step of the update; a kernel reads those of minibatch step `step`.
+struct LossOperands {
+  const int32_t* rowidx;         // [E*M][cap] local flat transition index per minibatch row
+  const int32_t* count;          // [E*M] rows owned by this rank in each minibatch
+  const float* adv_sum;          // [E*M] sum adv over the GLOBAL minibatch
+  const float* adv_sq;           // [E*M] sum (adv - mean)^2 over the GLOBAL minibatch
+  const float* action;           // [Bl][A]
+  const float* v_old;            // [Bl]   Memory.value
+  const float* logp_old;         // [Bl]   Memory.log_prob
+  const float* adv;              // [Bl]
+  const float* tgt;              // [Bl]
+  int cap;                       // row-list stride
+  int step;                      // minibatch step e * M + k of this launch
+  float inv_mb, clip_eps, vf_coef;
+};
+
 // ---- head_loss.cu ------------------------------------------------------------------------
 struct HeadLossArgs {
   const __nv_bfloat16* h_a;      // last hidden activation, actor  [M_pad][ldh]
@@ -61,22 +78,13 @@ struct HeadLossArgs {
   __nv_bfloat16* dz_a;           // out: dL/dz of the last hidden layer (actor)
   __nv_bfloat16* dz_c;
   const float* params;           // fp32 arena
-  const int32_t* rowidx;         // [cap] local flat transition index per minibatch row
-  const int32_t* count;          // [1] rows owned by this rank in this minibatch
-  const float* adv_sum;          // [1] sum adv over the GLOBAL minibatch
-  const float* adv_sq;           // [1] sum (adv - mean)^2 over the GLOBAL minibatch
-  const float* action;           // [Bl][A]
-  const float* v_old;            // [Bl]   Memory.value
-  const float* logp_old;         // [Bl]   Memory.log_prob
-  const float* adv;              // [Bl]
-  const float* tgt;              // [Bl]
+  LossOperands loss;
   float* partials;               // [tiles][partial_stride]
   int partial_stride;
   int po_w3a, po_b3a, po_w3c, po_b3c, po_logstd, po_loss;   // offsets inside a partial
   HeadOffsets off;                                            // offsets inside the arena
-  int H, A, ldh, cap;
+  int H, A, ldh;
   int act_a, act_c;              // ACTK_* of the hidden layers
-  float inv_mb, clip_eps, vf_coef;
 };
 int head_loss_init();
 int head_loss_launch(const HeadLossArgs& a, int tiles, cudaStream_t stream);

@@ -17,6 +17,7 @@
 #include "minppo_internal.h"
 #include "threefry.cuh"
 #include "policy_math.cuh"
+#include "ppo_math.cuh"
 
 namespace minppo {
 
@@ -109,7 +110,7 @@ __global__ void __launch_bounds__(PH_THREADS) policy_head_kernel(const PolicyHea
       }
       if (a.action) a.action[static_cast<size_t>(row) * A + j] = act;
       const float z = (act - mean) * (1.f / scale);
-      quad += -0.5f * z * z - 0.91893853320467274178f;
+      quad += gauss_logp_term(z);
       logdet += logf(fabsf(scale));
     }
   }

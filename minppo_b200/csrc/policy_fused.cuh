@@ -14,6 +14,7 @@
 
 #include "fused_step.cuh"
 #include "policy_math.cuh"
+#include "ppo_math.cuh"
 
 namespace minppo {
 
@@ -274,7 +275,7 @@ __global__ void __launch_bounds__(FS_THREADS, 1) policy_fused_kernel(const __gri
                 }
                 if (p.action) p.action[static_cast<size_t>(row) * p.A + j] = a;
                 const float z = (a - mean) * (1.f / scale);
-                quad += -0.5f * z * z - 0.91893853320467274178f;
+                quad += gauss_logp_term(z);
                 logdet += logf(fabsf(scale));
               }
             }
