@@ -110,6 +110,28 @@ int minppo_permutation(const uint32_t* key_in, uint32_t* key_out, int32_t prng_m
 int64_t minppo_param_layout(const minppo_config* cfg, int32_t* nleaves, int64_t* offsets, int64_t* rows,
                             int64_t* cols);
 
+/* ---- kernel path ---------------------------------------------------------------------------
+ * The kernels minppo_ctx_create and minppo_update pick for a config on a device with `sm_count` SMs (minppo_ctx_create
+ * uses the device's).  Host only, no CUDA call: it answers without a GPU.  A config the context refuses is refused here
+ * with the same code and message.  Named like `struct stat` / stat(): declare the result as `struct minppo_plan`.
+ *   num_params     P
+ *   fused          fused step kernel (num_layers == 2, hidden_size <= 256, act_dim <= 32, not disabled)
+ *   ap, head_amax  head width of the fused step kernel (16 or 32) and template of the layer-wise heads (8, 16, 32, 64)
+ *   hsplit         column groups of the forward, dX and policy GEMMs (2: hidden_size > 256)
+ *   dw_nsplit, S   column groups per (net, layer) and split-K factor of the weight-gradient GEMM
+ *   dw_gemm_ctas   CTAs of that GEMM; two_launch = dw_gemm_ctas > sm_count: it runs as a launch of its own
+ *   maxu           4-element units per thread of the optimizer's register-resident path (1, 2 or 4); dwopt_fast: that
+ *                  path holds the weight-gradient GEMM's leaves
+ *   padded         row lists sized for a worst-case row count (world_size > 1), row counts read on the device
+ *   row_cap        rows per minibatch row list (a multiple of 128)
+ *   peer_exchange  world_size > 1: the peer-memory gradient exchange may replace NCCL once peers are set */
+struct minppo_plan {
+  int64_t num_params;
+  int32_t fused, ap, head_amax, hsplit, dw_nsplit, S, dw_gemm_ctas, two_launch;
+  int32_t maxu, dwopt_fast, padded, row_cap, peer_exchange;
+};
+int minppo_plan(const minppo_config* cfg, int32_t sm_count, struct minppo_plan* out);
+
 /* ---- (3) context -----------------------------------------------------------------------
  * Owns workspace, TMA descriptors, weight images and (world_size > 1) a NCCL communicator
  * built from `nccl_unique_id_host` (128 bytes from minppo_nccl_unique_id on rank 0, broadcast

@@ -24,7 +24,7 @@ SYMBOLS = (
     "minppo_nccl_unique_id", "minppo_ctx_create", "minppo_ctx_destroy", "minppo_update",
     "minppo_ctx_check", "minppo_update_launch_count", "minppo_ctx_read", "minppo_debug_gemm",
     "minppo_ctx_profile", "minppo_ctx_profile_read", "minppo_ctx_ipc_handle", "minppo_ctx_set_peers",
-    "minppo_policy_step", "minppo_update_with_stats",
+    "minppo_policy_step", "minppo_update_with_stats", "minppo_plan",
 )
 POLICY_WEIGHTS_CURRENT = 1
 PROFILE_CLASSES = ("gae", "perm_sort", "rows_and_adv_stats", "obs_image", "weight_images", "fwd_gemm", "head_loss",
@@ -45,6 +45,13 @@ class MinppoConfig(C.Structure):
         ("ent_coef", C.c_double), ("vf_coef", C.c_double),
         ("adam_b1", C.c_double), ("adam_b2", C.c_double), ("adam_eps", C.c_double), ("adam_eps_root", C.c_double),
     ]
+
+
+class MinppoPlan(C.Structure):
+    """``struct minppo_plan`` -- field order and types must match the header."""
+    _fields_ = [("num_params", C.c_int64)] + [(n, C.c_int32) for n in (
+        "fused", "ap", "head_amax", "hsplit", "dw_nsplit", "S", "dw_gemm_ctas", "two_launch",
+        "maxu", "dwopt_fast", "padded", "row_cap", "peer_exchange")]
 
 
 class MinppoError(RuntimeError):
@@ -85,6 +92,8 @@ def load() -> C.CDLL:
                                         C.POINTER(i64)]
     lib.minppo_nccl_unique_id.restype = C.c_int
     lib.minppo_nccl_unique_id.argtypes = [vp]
+    lib.minppo_plan.restype = C.c_int
+    lib.minppo_plan.argtypes = [C.POINTER(MinppoConfig), i32, C.POINTER(MinppoPlan)]
     lib.minppo_ctx_create.restype = C.c_int
     lib.minppo_ctx_create.argtypes = [C.POINTER(MinppoConfig), vp, C.POINTER(vp)]
     lib.minppo_ctx_destroy.restype = C.c_int

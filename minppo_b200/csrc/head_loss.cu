@@ -257,7 +257,7 @@ int head_loss_init() {
 
 int head_loss_launch(const HeadLossArgs& a, int tiles, cudaStream_t stream) {
   if (a.A > MAX_ACT_DIM) return MINPPO_ERR_ARG;
-  const int amax = a.A <= 8 ? 8 : (a.A <= 16 ? 16 : (a.A <= 32 ? 32 : 64));
+  const int amax = head_amax(a.A);
   const size_t smem = head_loss_smem_bytes(a.H, amax);
   if (amax == 8) head_loss_kernel<8><<<tiles, HL_THREADS, smem, stream>>>(a);
   else if (amax == 16) head_loss_kernel<16><<<tiles, HL_THREADS, smem, stream>>>(a);

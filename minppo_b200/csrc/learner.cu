@@ -249,14 +249,8 @@ struct minppo_ctx {
   int device, sm_count;
   int T, N, Nl, n0, M, E, L, H, D, Dp, A;
   long long B, Bl, P;
-  int mb, cap, M_pad, m_tiles, tiles64, S;
-  int dw_nsplit;              // dW GEMM groups per (net, layer): 1 (128 x H tiles) or 2 (column groups of col_group: half the
-                              // split-K factor -- half the partial bytes stored and re-read per step; H % 128 == 0 on the
-                              // fused path, always when H > GEMM_MAXN)
-  int hsplit;                 // column groups of the forward, dX and policy GEMMs: 1, or 2 when H > GEMM_MAXN (col_group)
-  int maxu;                   // dwopt fast path: 4-element units of the hidden kernels per thread (1, 2 or 4)
-  bool fused;                 // fused step kernel (L == 2; any obs_dim, act_dim <= FS_MAX_AP, hidden_size <= 256)
-  int head_parts;             // head partials per minibatch: m_tiles (fused) or tiles64
+  int mb, m_tiles, tiles64;   // 128- and 64-row tiles of plan.row_cap
+  struct minppo_plan plan;    // kernel path (minppo_plan)
   std::vector<LeafInfo> leaves;
   // device buffers
   std::vector<void*> allocs;
@@ -266,8 +260,6 @@ struct minppo_ctx {
   bool trace_on;
   int32_t *perms, *rowidx, *counts;
   int32_t* perm_tmp;          // world_size > 1: the epochs THIS rank sorts ([ceil(E / W)][B]); broadcast into perms
-  bool padded;                // row lists sized for a worst-case row count (world_size > 1): device-side row counts bound
-                              // the per-minibatch work
   void* perm_ws;
   size_t perm_ws_bytes;
   __nv_bfloat16* obs_img;
@@ -279,7 +271,6 @@ struct minppo_ctx {
   NetBufs net[2];
   int head_stride, po_w3a, po_b3a, po_w3c, po_b3c, po_logstd, po_loss;
   int po_db[2][2];            // fused path: [net][layer] hidden-bias gradient partials (column sums of dZ), H floats each
-  int ap;                     // padded head width of the fused step kernel: 16 (A <= 16) or 32
   HeadOffsets head;           // arena offsets of the output-head leaves
   // graph cache
   cudaStream_t cap_stream;
@@ -402,26 +393,27 @@ static void fill_opt_args(const minppo_ctx* c, const UpdatePtrs& u, OptArgs* o) 
   memset(o, 0, sizeof(*o));
   const minppo_config& cfg = c->cfg;
   const int L = c->L, H = c->H;
+  const int head_parts = c->plan.fused ? c->m_tiles : c->tiles64;   // head partials per minibatch
   int n = 0;
   for (const auto& lf : c->leaves) {
     OptLeaf& ol = o->leaf[n++];
     ol.offset = static_cast<int>(lf.offset);
     ol.cols = static_cast<int>(lf.cols);
     if (lf.net == 2) {                         // log_std
-      ol.grad_src = c->head_part; ol.src_offset = c->po_logstd; ol.nparts = c->head_parts; ol.part_stride = c->head_stride;
+      ol.grad_src = c->head_part; ol.src_offset = c->po_logstd; ol.nparts = head_parts; ol.part_stride = c->head_stride;
       ol.grad_bias = cfg.rank == 0 ? -static_cast<float>(cfg.ent_coef) : 0.f;
     } else if (lf.layer == L) {                // output heads
-      ol.grad_src = c->head_part; ol.nparts = c->head_parts; ol.part_stride = c->head_stride;
-      if (lf.is_kernel) { ol.src_offset = lf.net == 0 ? c->po_w3a : c->po_w3c; ol.img_w2 = c->fused ? c->net[lf.net].w2img : nullptr; ol.ap = c->ap; }
+      ol.grad_src = c->head_part; ol.nparts = head_parts; ol.part_stride = c->head_stride;
+      if (lf.is_kernel) { ol.src_offset = lf.net == 0 ? c->po_w3a : c->po_w3c; ol.img_w2 = c->plan.fused ? c->net[lf.net].w2img : nullptr; ol.ap = c->plan.ap; }
       else ol.src_offset = lf.net == 0 ? c->po_b3a : c->po_b3c;
     } else if (lf.is_kernel) {                 // hidden kernels: split-K partials of the dW GEMM
       const int in_l = lf.layer == 0 ? c->D : H;
-      ol.grad_src = c->net[lf.net].dw_part[lf.layer]; ol.src_offset = 0; ol.nparts = c->S; ol.part_stride = in_l * H; ol.late = 1;
+      ol.grad_src = c->net[lf.net].dw_part[lf.layer]; ol.src_offset = 0; ol.nparts = c->plan.S; ol.part_stride = in_l * H; ol.late = 1;
       ol.img_n = c->net[lf.net].wn[lf.layer];
-    } else if (c->fused) {                     // hidden biases, fused path: per-tile column sums of dz[l+1] from the fused step kernel
-      ol.grad_src = c->head_part; ol.src_offset = c->po_db[lf.net][lf.layer]; ol.nparts = c->head_parts; ol.part_stride = c->head_stride;
+    } else if (c->plan.fused) {                // hidden biases, fused path: per-tile column sums of dz[l+1] from the fused step kernel
+      ol.grad_src = c->head_part; ol.src_offset = c->po_db[lf.net][lf.layer]; ol.nparts = head_parts; ol.part_stride = c->head_stride;
     } else {                                   // hidden biases: column sums of dz[l+1], computed by the dW GEMM (ones x dz)
-      ol.grad_src = c->net[lf.net].dbias[lf.layer]; ol.src_offset = 0; ol.nparts = c->S;
+      ol.grad_src = c->net[lf.net].dbias[lf.layer]; ol.src_offset = 0; ol.nparts = c->plan.S;
       ol.part_stride = H; ol.late = 1;
     }
   }
@@ -434,7 +426,7 @@ static void fill_opt_args(const minppo_ctx* c, const UpdatePtrs& u, OptArgs* o) 
   o->P = static_cast<int>(c->P);
   o->A = c->A;
   o->gflat = c->gflat;
-  o->loss_src = c->head_part; o->loss_src_offset = c->po_loss; o->loss_nparts = c->head_parts; o->loss_part_stride = c->head_stride;
+  o->loss_src = c->head_part; o->loss_src_offset = c->po_loss; o->loss_nparts = head_parts; o->loss_part_stride = c->head_stride;
   o->params = u.params; o->mu = u.mu; o->nu = u.nu; o->count = u.count;
   o->block_ss = c->block_ss; o->barrier = c->barrier; o->err_flag = c->err_flag;
   o->off_logstd = c->head.logstd;
@@ -461,7 +453,7 @@ static int nccl_allreduce(minppo_ctx* c, float* buf, size_t n, cudaStream_t stre
 
 // ---- parameter blocks of the per-minibatch kernels ----
 static void fill_loss_operands(const minppo_ctx* c, const UpdatePtrs& u, int s, LossOperands* lo) {
-  lo->rowidx = c->rowidx; lo->count = c->counts; lo->cap = c->cap; lo->step = s;
+  lo->rowidx = c->rowidx; lo->count = c->counts; lo->cap = c->plan.row_cap; lo->step = s;
   lo->adv_sum = c->stats; lo->adv_sq = c->stats + c->E * c->M;
   lo->action = u.action; lo->v_old = u.value; lo->logp_old = u.log_prob; lo->adv = c->adv; lo->tgt = c->tgt;
   lo->inv_mb = static_cast<float>(1.0 / c->mb);
@@ -497,8 +489,8 @@ static void fill_fused_params(minppo_ctx* c, const UpdatePtrs& u, int s, FusedPa
   p.trace = c->trace_on ? c->trace : nullptr;
 }
 
-// weight-gradient GEMM groups + optimizer block + per-update arrays; returns the number of GEMM CTAs
-static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dpp) {
+// weight-gradient GEMM groups + optimizer block + per-update arrays
+static void fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dpp) {
   DwOptParams& dp = *dpp;
   memset(&dp, 0, sizeof(dp));
   const int L = c->L, H = c->H;
@@ -508,24 +500,24 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
   for (int net = 0; net < 2; ++net) {
     NetBufs& nb = c->net[net];
     for (int l = 0; l < L; ++l) {
-      tile_first[net][l] = cta / c->S;
+      tile_first[net][l] = cta / c->plan.S;
       tile_count[net][l] = 0;
-      for (int nh = 0; nh < c->dw_nsplit; ++nh) {
+      for (int nh = 0; nh < c->plan.dw_nsplit; ++nh) {
       GemmGroup& g = p.g[ng++];
       g.cta_begin = cta;
       const int in_l = l == 0 ? c->D : H;
       const int in_pad = l == 0 ? c->Dp : H;
-      if (l == 0 && c->fused) { g.amode = A_TMA_MN; g.tmA = c->m_xg_mn; }   // rows gathered by the fused kernel
+      if (l == 0 && c->plan.fused) { g.amode = A_TMA_MN; g.tmA = c->m_xg_mn; }   // rows gathered by the fused kernel
       else if (l == 0) { g.amode = A_GATHER_MN; g.rowidx = c->rowidx; g.gimage = c->obs_img; g.ldg = c->Dp; }      // row list: per step
       else { g.amode = A_TMA_MN; g.tmA = nb.m_act_mn[l]; }
       g.bmode = B_TMA_MN; g.tmB = nb.m_dz_mn[l + 1];
-      g.kb_total = c->M_pad / 64;
+      g.kb_total = c->plan.row_cap / 64;
       g.k_count = nullptr;                                    // per step (counts[] below)
       g.tmC = nb.m_dw[l];
-      g.colsum_out = c->fused ? nullptr : nb.dbias[l];      // fused path: the bias gradients come from the fused step kernel
-      col_group(H, c->dw_nsplit, nh, &g.n_off, &g.N);
+      g.colsum_out = c->plan.fused ? nullptr : nb.dbias[l]; // fused path: the bias gradients come from the fused step kernel
+      col_group(H, c->plan.dw_nsplit, nh, &g.n_off, &g.N);
       g.ldc = H;
-      g.m_tiles = (in_pad + 127) / 128; g.splits = c->S; g.m_store = in_l;
+      g.m_tiles = (in_pad + 127) / 128; g.splits = c->plan.S; g.m_store = in_l;
       cta += g.m_tiles * g.splits;
       tile_count[net][l] += g.m_tiles;
       if (nh == 0) tile_split[net][l] = g.N;
@@ -537,7 +529,7 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
   fill_opt_args(c, u, &dp.opt);
   // A GEMM grid past one CTA per SM runs as a launch of its own in front of dwopt (enqueue_step): dwopt then has no GEMM
   // CTAs, and its late leaves wait for no counter (tile fields 0), since their partials are complete when it starts.
-  dp.gemm_ctas = cta <= c->sm_count ? cta : 0;
+  dp.gemm_ctas = c->plan.two_launch ? 0 : c->plan.dw_gemm_ctas;
   for (size_t i = 0; i < c->leaves.size() && dp.gemm_ctas; ++i) {
     OptLeaf& ol = dp.opt.leaf[i];
     const LeafInfo& lf = c->leaves[i];
@@ -551,12 +543,11 @@ static int fill_dwopt_params(minppo_ctx* c, const UpdatePtrs& u, DwOptParams* dp
   dp.losses_stride = u.losses_out ? 4 : 0;
   dp.opt.gnorm_out = c->gnorms;
   dp.opt.stats_out = u.stats_out;
-  dp.ridx_base = c->rowidx; dp.counts = c->counts; dp.cap = c->cap; dp.EM = c->E * c->M;
-  dp.padded = c->padded ? 1 : 0;
-  dp.part_rows = c->fused ? 128 : 64;
+  dp.ridx_base = c->rowidx; dp.counts = c->counts; dp.cap = c->plan.row_cap; dp.EM = c->E * c->M;
+  dp.padded = c->plan.padded;
+  dp.part_rows = c->plan.fused ? 128 : 64;
   dp.obs_img = c->obs_img; dp.obs_ld = c->Dp;
   dp.trace = c->trace_on ? c->trace2 : nullptr;
-  return cta;
 }
 
 // The NCCL fallback's second dwopt launch, which only applies the all-reduced gradient: gflat holds it (P floats, then the
@@ -593,11 +584,11 @@ static void fill_forward_gemm(const minppo_ctx* c, int l, const float* params, i
   memset(&p, 0, sizeof(p));
   const int H = c->H;
   int ng = 0;
-  for (int i = first_net * c->hsplit; i < 2 * c->hsplit; ++i, ++ng) {
-    const int net = i / c->hsplit;
+  for (int i = first_net * c->plan.hsplit; i < 2 * c->plan.hsplit; ++i, ++ng) {
+    const int net = i / c->plan.hsplit;
     GemmGroup& g = p.g[ng];
     g.cta_begin = ng * m_tiles;
-    col_group(H, c->hsplit, i % c->hsplit, &g.n_off, &g.N);
+    col_group(H, c->plan.hsplit, i % c->plan.hsplit, &g.n_off, &g.N);
     g.bmode = B_TMA_MN;                   // kernel image as stored [in = k][out = n]
     g.tmB = c->net[net].m_wn_mn[l];
     if (op[net].rowidx) { g.amode = A_GATHER_K; g.rowidx = op[net].rowidx; g.gimage = c->obs_img; g.ldg = c->Dp; }
@@ -624,15 +615,15 @@ static int enqueue_weight_images(const minppo_ctx* c, const float* params, cudaS
 // ---- one minibatch step --------------------------------------------------------------------
 static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t stream) {
   const int L = c->L, H = c->H;
-  const int32_t* ridx = c->rowidx + static_cast<size_t>(s) * c->cap;
+  const int32_t* ridx = c->rowidx + static_cast<size_t>(s) * c->plan.row_cap;
   // programmatic dependent launch between the per-minibatch kernels (fused path only; common.cuh)
-  const bool pdl = c->fused && !c->profiling;
-  if (c->fused) {
+  const bool pdl = c->plan.fused && !c->profiling;
+  if (c->plan.fused) {
     // forward + heads + loss + backward-to-dZ of both nets in one launch (fused_step.cuh)
     FusedParams p;
     fill_fused_params(c, u, s, &p);
     PROF(PC_FWD_GEMM);
-    const cudaError_t e = c->ap == 16
+    const cudaError_t e = c->plan.ap == 16
         ? launch_kernel(fused_step_kernel<16>, 2 * c->m_tiles, FS_THREADS, FsLayout<16>::BYTES, stream, pdl, p)
         : launch_kernel(fused_step_kernel<32>, 2 * c->m_tiles, FS_THREADS, FsLayout<32>::BYTES, stream, pdl, p);
     if (e != cudaSuccess) { set_error("fused_step launch failed: %s", cudaGetErrorString(e)); return MINPPO_ERR_CUDA; }
@@ -671,20 +662,20 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
   for (int l = L - 1; l >= 1; --l) {
     GemmParams p;
     memset(&p, 0, sizeof(p));
-    p.ngroups = 2 * c->hsplit;
+    p.ngroups = 2 * c->plan.hsplit;
     for (int i = 0; i < p.ngroups; ++i) {
-      const int net = i / c->hsplit, j = i % c->hsplit;
+      const int net = i / c->plan.hsplit, j = i % c->plan.hsplit;
       GemmGroup& g = p.g[i];
       NetBufs& nb = c->net[net];
       g.cta_begin = i * c->m_tiles;
-      col_group(H, c->hsplit, j, &g.n_off, &g.N);
+      col_group(H, c->plan.hsplit, j, &g.n_off, &g.N);
       g.amode = A_TMA_K; g.tmA = nb.m_dz_k[l + 1];
       g.bmode = B_TMA_K; g.tmB = nb.m_wn[2 * l + j];
       g.kb_total = H / 64;
       g.out = nb.dz[l]; g.ldo = H;
       g.hprev = nb.act[l]; g.ldh = H;
       g.act = act_kind(c, net);
-      g.m_tiles = c->m_tiles; g.splits = 1; g.m_store = c->M_pad;
+      g.m_tiles = c->m_tiles; g.splits = 1; g.m_store = c->plan.row_cap;
     }
     PROF(PC_BWD_GEMM);
     RET(launch_gemm<EPI_DACT>(p, p.ngroups * c->m_tiles, stream));
@@ -696,31 +687,28 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
   // CTAs.  Env-sharded ranks without the peer-memory exchange then all-reduce the gradient sums over NCCL and apply them
   // with a second dwopt launch.
   DwOptParams dp;
-  const int cta = fill_dwopt_params(c, u, &dp);
+  fill_dwopt_params(c, u, &dp);
   dp.step = s;
-  const bool two_launch = cta > c->sm_count;
   const bool sharded = c->cfg.world_size > 1;
-  // all-reduce fused into the dwopt launch (peer memory); needs the register-resident fast path of the kernel, and the
-  // GEMM in the same launch
-  const bool px_on = sharded && c->peers_set && c->P <= dwopt_fast_capacity(c->sm_count, c->maxu) && !two_launch;
+  const bool px_on = sharded && c->peers_set && c->plan.peer_exchange;   // all-reduce fused into the dwopt launch
   const bool nccl = sharded && !px_on;
   if (px_on) dp.px = c->px;
   dp.opt.do_apply = nccl ? 0 : 1;
   auto launch_dwopt = [&]() -> int {
     PROF(dp.gemm_ctas ? PC_DW_GEMM : PC_OPT);
-    const cudaError_t e = dwopt_launch(dp, c->sm_count, stream, pdl, c->maxu);
+    const cudaError_t e = dwopt_launch(dp, c->sm_count, stream, pdl, c->plan.maxu);
     if (e != cudaSuccess) { set_error("dwopt launch failed: %s", cudaGetErrorString(e)); return MINPPO_ERR_CUDA; }
     c->launches++;
     return 0;
   };
-  if (two_launch) {
+  if (c->plan.two_launch) {
     GemmParams p = dp.gemm;                                  // this step's row list and row count go into the groups
     for (int i = 0; i < p.ngroups; ++i) {
       if (p.g[i].rowidx) p.g[i].rowidx = ridx;
-      p.g[i].k_count = c->padded ? c->counts + s : nullptr;
+      p.g[i].k_count = c->plan.padded ? c->counts + s : nullptr;
     }
     PROF(PC_DW_GEMM);
-    RET(launch_gemm<EPI_PARTIAL>(p, cta, stream, pdl));
+    RET(launch_gemm<EPI_PARTIAL>(p, c->plan.dw_gemm_ctas, stream, pdl));
     c->launches++;
   }
   RET(launch_dwopt());
@@ -785,10 +773,10 @@ static int enqueue_update(minppo_ctx* c, const UpdatePtrs& u, cudaStream_t strea
   const int EM = c->E * c->M;
   {
     PROF(PC_PREP);
-    RET(compact_rows_launch(c->perms, c->rowidx, c->counts, c->E, c->M, c->B, c->mb, c->cap, c->N, c->n0, c->Nl, c->err_flag, stream));
-    RET(adv_stats_launch(c->adv, c->rowidx, c->counts, c->stats, EM, c->cap, c->mb, 0, stream));
+    RET(compact_rows_launch(c->perms, c->rowidx, c->counts, c->E, c->M, c->B, c->mb, c->plan.row_cap, c->N, c->n0, c->Nl, c->err_flag, stream));
+    RET(adv_stats_launch(c->adv, c->rowidx, c->counts, c->stats, EM, c->plan.row_cap, c->mb, 0, stream));
     if (cfg.world_size > 1) RET(nccl_allreduce(c, c->stats, EM, stream));
-    RET(adv_stats_launch(c->adv, c->rowidx, c->counts, c->stats, EM, c->cap, c->mb, 1, stream));
+    RET(adv_stats_launch(c->adv, c->rowidx, c->counts, c->stats, EM, c->plan.row_cap, c->mb, 1, stream));
     if (cfg.world_size > 1) RET(nccl_allreduce(c, c->stats + EM, EM, stream));
     c->launches += 3 + (cfg.world_size > 1 ? 2 : 0);
   }
@@ -880,6 +868,72 @@ int minppo_nccl_unique_id(void* id128_host) {
   return 0;
 }
 
+// Every choice of the kernel path (include/minppo_b200.h); minppo_ctx_create keeps the result as c->plan.
+int minppo_plan(const minppo_config* cfg, int32_t sm_count, struct minppo_plan* out) {
+  if (!cfg || !out || sm_count < 1) { set_error("minppo_plan: null argument or sm_count %d", sm_count); return MINPPO_ERR_ARG; }
+  RET(validate_config(*cfg));
+  const minppo_config& c = *cfg;
+  const int L = c.num_layers, H = c.hidden_size, A = c.act_dim, Dp = (c.obs_dim + 63) / 64 * 64;
+  const long long Bl = static_cast<long long>(c.num_steps) * (c.num_envs / c.world_size);   // this rank's transitions
+  const int mb = static_cast<int>(static_cast<long long>(c.num_steps) * c.num_envs / c.num_minibatches);
+  struct minppo_plan p = {};
+  p.num_params = build_layout(c, nullptr);
+  // row lists: the whole minibatch, or on env-sharded ranks 1.5 x the mean share + 256 rows
+  p.padded = c.world_size > 1;
+  int cap = mb;
+  if (p.padded) cap = static_cast<int>(std::min<long long>({(3LL * mb / c.world_size + 1) / 2 + 256, mb, Bl}));
+  // test hook (tests/test_gpu_update.py): an undersized row list, to exercise the overflow path on one GPU
+  const int force_cap = getenv("MINPPO_FORCE_CAP") ? atoi(getenv("MINPPO_FORCE_CAP")) : 0;
+  if (force_cap > 0) { p.padded = 1; cap = force_cap; }
+  p.row_cap = (cap + 127) / 128 * 128;                 // row lists are padded to whole GEMM tiles
+  // wider hidden layers or heads than the fused step kernel holds run layer-wise, whatever learner.fused says
+  p.fused = !c.disable_fused && L == 2 && H <= GEMM_MAXN && A <= FS_MAX_AP;
+  p.ap = A <= 16 ? 16 : 32;
+  p.head_amax = head_amax(A);
+  p.hsplit = H > GEMM_MAXN ? 2 : 1;
+  const long long P = p.num_params;
+  p.maxu = P <= dwopt_fast_capacity(sm_count, 1) ? 1 : (P <= dwopt_fast_capacity(sm_count, 2) ? 2 : 4);
+  // split-K of the dW GEMMs: fill the SMs once
+  // N-halved dW tiles (fused path, H a multiple of 128): half the split-K factor for the same number of GEMM CTAs
+  // (only with TMA-fed A operands: groups that gather their rows by index would gather every row twice).
+  // H > GEMM_MAXN needs the two column groups of col_group whatever the path; there the first layer's groups gather
+  // their observation rows by index (A_GATHER_MN), so every row is gathered once per column group: twice the
+  // observation-image reads of that layer's A operand.
+  p.dw_nsplit = H > GEMM_MAXN ? 2 : (p.fused && H % 128 == 0 && 2 * 2 * L <= GEMM_MAX_GROUPS) ? 2 : 1;
+  int per_split = 0;
+  for (int l = 0; l < L; ++l) per_split += 2 * p.dw_nsplit * (((l == 0 ? Dp : H) + 127) / 128);
+  // leave ~16 of the one-CTA-per-SM grid as spare CTAs: they sum the per-tile partials of the small leaves while the GEMM
+  // runs (D = 415 / A = 20 with 4 spare CTAs: 6,441 elements x 64 partials on 2,048 threads outlasted the GEMM itself)
+  const int gemm_budget = sm_count > 48 ? sm_count - 16 : sm_count;
+  int S = c.dw_splits > 0 ? c.dw_splits : (gemm_budget / (per_split > 0 ? per_split : 1));
+  // k-blocks (64 minibatch rows each) the splits share.  Padded row lists (env-sharded ranks): size the split for the
+  // rows a minibatch is EXPECTED to have on this rank (mean + 3 sigma of the hypergeometric count), not for the
+  // worst-case capacity -- the kernel splits the live k-blocks at run time, an over-sized S only removes spare CTAs.
+  int kb_total = p.row_cap / 64;
+  if (p.padded) {
+    const double mean = static_cast<double>(mb) / c.world_size;
+    const long long rows = static_cast<long long>(mean + 3.0 * sqrt(mean)) + 1;
+    kb_total = std::max(1, static_cast<int>(std::min<long long>(p.row_cap, rows + 63) / 64));
+  }
+  S = std::max(1, std::min({S, kb_total, 32}));
+  // no empty splits: ceil(kb_total / S) * (S - 1) < kb_total
+  while (S > 1 && ((kb_total + S - 1) / S) * (S - 1) >= kb_total) --S;
+  p.S = S;
+  p.dw_gemm_ctas = per_split * S;
+  // a GEMM grid past one CTA per SM runs as a launch of its own in front of dwopt
+  p.two_launch = p.dw_gemm_ctas > sm_count;
+  // dwopt_kernel decides its register-resident path on the device from the leaf table, `n_units <= G * NT * MAXU`
+  // (dwopt.cuh), n_units = the 4-element units of the late leaves that fill_opt_args marks: the hidden kernels and, on
+  // the layer-wise path, the hidden biases whose column sums the dW GEMM computes.  The same condition on the host:
+  long long late_units = 0;                            // both nets: hidden kernel (+ bias)
+  for (int l = 0; l < L; ++l) late_units += 2 * ((l == 0 ? c.obs_dim : H) * (H / 4LL) + (p.fused ? 0 : H / 4));
+  p.dwopt_fast = 4 * late_units <= dwopt_fast_capacity(sm_count, p.maxu);
+  // the all-reduce fused into the dwopt launch needs the kernel's register-resident path and the GEMM in the same launch
+  p.peer_exchange = P <= dwopt_fast_capacity(sm_count, p.maxu) && !p.two_launch;
+  *out = p;
+  return 0;
+}
+
 static void drop_graphs(minppo_ctx* c) {
   for (auto& g : c->graphs) { cudaGraphExecDestroy(g.exec); cudaGraphDestroy(g.graph); }
   c->graphs.clear();
@@ -925,67 +979,15 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   c->D = cfg->obs_dim; c->Dp = (c->D + 63) / 64 * 64; c->A = cfg->act_dim;
   c->B = static_cast<long long>(c->T) * c->N; c->Bl = static_cast<long long>(c->T) * c->Nl;
   c->mb = static_cast<int>(c->B / c->M);
-  c->padded = cfg->world_size > 1;
-  if (!c->padded) c->cap = c->mb;
-  else {
-    long long cap = (3LL * c->mb / cfg->world_size + 1) / 2 + 256;    // 1.5 x mean + 256 rows
-    if (cap > c->mb) cap = c->mb;
-    if (cap > c->Bl) cap = c->Bl;
-    c->cap = static_cast<int>(cap);
-  }
-  if (getenv("MINPPO_FORCE_CAP") && atoi(getenv("MINPPO_FORCE_CAP")) > 0) {
-    // test hook (tests/test_gpu_update.py): an undersized row list, to exercise the overflow path on one GPU
-    c->padded = true;
-    c->cap = atoi(getenv("MINPPO_FORCE_CAP"));
-  }
-  c->M_pad = (c->cap + 127) / 128 * 128;
-  c->cap = c->M_pad;                                  // row lists are padded to whole GEMM tiles
-  c->m_tiles = c->M_pad / 128;
-  c->tiles64 = c->M_pad / 64;
-  // wider hidden layers or heads than the fused step kernel holds run layer-wise, whatever learner.fused says
-  c->fused = !cfg->disable_fused && c->L == 2 && c->H <= GEMM_MAXN && c->A <= FS_MAX_AP;
-  c->hsplit = c->H > GEMM_MAXN ? 2 : 1;
-  c->ap = c->A <= 16 ? 16 : 32;
-  c->head_parts = c->fused ? c->m_tiles : c->tiles64;
+  if ((rc = minppo_plan(cfg, c->sm_count, &c->plan))) return fail(rc);
+  c->m_tiles = c->plan.row_cap / 128;
+  c->tiles64 = c->plan.row_cap / 64;
   c->P = build_layout(*cfg, &c->leaves);
   c->head.w3a = static_cast<int>(find_leaf(c, 0, c->L, 1).offset);
   c->head.b3a = static_cast<int>(find_leaf(c, 0, c->L, 0).offset);
   c->head.w3c = static_cast<int>(find_leaf(c, 1, c->L, 1).offset);
   c->head.b3c = static_cast<int>(find_leaf(c, 1, c->L, 0).offset);
   c->head.logstd = static_cast<int>(c->leaves.back().offset);
-  c->maxu = c->P <= dwopt_fast_capacity(c->sm_count, 1) ? 1 : (c->P <= dwopt_fast_capacity(c->sm_count, 2) ? 2 : 4);
-  // split-K of the dW GEMMs: fill the SMs once
-  {
-    // N-halved dW tiles (fused path, H a multiple of 128): half the split-K factor for the same number of GEMM CTAs
-    // (only with TMA-fed A operands: groups that gather their rows by index would gather every row twice).
-    // H > GEMM_MAXN needs the two column groups of col_group whatever the path; there the first layer's groups gather
-    // their observation rows by index (A_GATHER_MN), so every row is gathered once per column group: twice the
-    // observation-image reads of that layer's A operand.
-    c->dw_nsplit = c->H > GEMM_MAXN ? 2
-                 : (c->fused && c->H % 128 == 0 && 2 * 2 * c->L <= GEMM_MAX_GROUPS) ? 2 : 1;
-    int per_split = 0;
-    for (int l = 0; l < c->L; ++l) per_split += 2 * c->dw_nsplit * (((l == 0 ? c->Dp : c->H) + 127) / 128);
-    // leave ~16 of the one-CTA-per-SM grid as spare CTAs: they sum the per-tile partials of the small leaves while the GEMM
-    // runs (D = 415 / A = 20 with 4 spare CTAs: 6,441 elements x 64 partials on 2,048 threads outlasted the GEMM itself)
-    const int gemm_budget = c->sm_count > 48 ? c->sm_count - 16 : c->sm_count;
-    int S = cfg->dw_splits > 0 ? cfg->dw_splits : (gemm_budget / (per_split > 0 ? per_split : 1));
-    // k-blocks (64 minibatch rows each) the splits share.  Padded row lists (env-sharded ranks): size the split for the
-    // rows a minibatch is EXPECTED to have on this rank (mean + 3 sigma of the hypergeometric count), not for the
-    // worst-case capacity -- the kernel splits the live k-blocks at run time, an over-sized S only removes spare CTAs.
-    int kb_total = c->M_pad / 64;
-    if (c->padded) {
-      const double mean = static_cast<double>(c->mb) / cfg->world_size;
-      const long long rows = static_cast<long long>(mean + 3.0 * sqrt(mean)) + 1;
-      kb_total = static_cast<int>(std::min<long long>(c->M_pad, rows + 63) / 64);
-      if (kb_total < 1) kb_total = 1;
-    }
-    if (S > kb_total) S = kb_total;
-    if (S > 32) S = 32;
-    if (S < 1) S = 1;
-    // no empty splits: ceil(kb_total / S) * (S - 1) < kb_total
-    while (S > 1 && ((kb_total + S - 1) / S) * (S - 1) >= kb_total) --S;
-    c->S = S;
-  }
   const int H = c->H, L = c->L, A = c->A;
   // head partial layout
   {
@@ -1029,14 +1031,14 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   ALLOC(c->perms, static_cast<size_t>(c->E) * c->B);
   c->perm_tmp = nullptr;
   if (cfg->world_size > 1) ALLOC(c->perm_tmp, static_cast<size_t>((c->E + cfg->world_size - 1) / cfg->world_size) * c->B);
-  ALLOC(c->rowidx, static_cast<size_t>(EM) * c->cap);
+  ALLOC(c->rowidx, static_cast<size_t>(EM) * c->plan.row_cap);
   ALLOC(c->counts, static_cast<size_t>(EM));
   c->perm_ws_bytes = perm_workspace_bytes(c->E, c->B);
   { uint8_t* p; ALLOC(p, c->perm_ws_bytes); c->perm_ws = p; }
   ALLOC(c->obs_img, static_cast<size_t>(c->Bl) * c->Dp + 256);   // slack: MN gather may read one chunk past Dp
-  ALLOC(c->xg, static_cast<size_t>(c->M_pad) * c->Dp);
-  if ((rc = make_tmap(&c->m_xg_k, c->xg, c->Dp, c->M_pad, c->Dp, 64, 128))) return fail(rc);
-  if ((rc = make_tmap(&c->m_xg_mn, c->xg, c->Dp, c->M_pad, c->Dp, 64, 64))) return fail(rc);
+  ALLOC(c->xg, static_cast<size_t>(c->plan.row_cap) * c->Dp);
+  if ((rc = make_tmap(&c->m_xg_k, c->xg, c->Dp, c->plan.row_cap, c->Dp, 64, 128))) return fail(rc);
+  if ((rc = make_tmap(&c->m_xg_mn, c->xg, c->Dp, c->plan.row_cap, c->Dp, 64, 64))) return fail(rc);
   ALLOC(c->barrier, 1);
   ALLOC(c->dw_done, static_cast<size_t>(c->sm_count + 2) * DWOPT_DONE_STRIDE);   // zeroed: dwopt_kernel expects 0 at launch
   ALLOC(c->err_flag, 1);
@@ -1048,12 +1050,12 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
     nb.m_act_k.resize(L + 1); nb.m_act_mn.resize(L + 1); nb.m_dz_k.resize(L + 1); nb.m_dz_mn.resize(L + 1);
     nb.m_wn_mn.resize(L); nb.m_wn.resize(2 * L); nb.m_dw.resize(L); nb.m_wn_h.resize(L);
     for (int l = 1; l <= L; ++l) {
-      ALLOC(nb.act[l], static_cast<size_t>(c->M_pad) * H);
-      ALLOC(nb.dz[l], static_cast<size_t>(c->M_pad) * H);
-      if ((rc = make_tmap(&nb.m_act_k[l], nb.act[l], H, c->M_pad, H, 64, 128))) return fail(rc);
-      if ((rc = make_tmap(&nb.m_act_mn[l], nb.act[l], H, c->M_pad, H, 64, 64))) return fail(rc);
-      if ((rc = make_tmap(&nb.m_dz_k[l], nb.dz[l], H, c->M_pad, H, 64, 128))) return fail(rc);
-      if ((rc = make_tmap(&nb.m_dz_mn[l], nb.dz[l], H, c->M_pad, H, 64, 64))) return fail(rc);
+      ALLOC(nb.act[l], static_cast<size_t>(c->plan.row_cap) * H);
+      ALLOC(nb.dz[l], static_cast<size_t>(c->plan.row_cap) * H);
+      if ((rc = make_tmap(&nb.m_act_k[l], nb.act[l], H, c->plan.row_cap, H, 64, 128))) return fail(rc);
+      if ((rc = make_tmap(&nb.m_act_mn[l], nb.act[l], H, c->plan.row_cap, H, 64, 64))) return fail(rc);
+      if ((rc = make_tmap(&nb.m_dz_k[l], nb.dz[l], H, c->plan.row_cap, H, 64, 128))) return fail(rc);
+      if ((rc = make_tmap(&nb.m_dz_mn[l], nb.dz[l], H, c->plan.row_cap, H, 64, 64))) return fail(rc);
     }
     for (int l = 0; l < L; ++l) {
       const int kp = l == 0 ? c->Dp : H;
@@ -1063,15 +1065,15 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
       if ((rc = make_tmap(&nb.m_wn_h[l], nb.wn[l], H, kp, H, 64, 32))) return fail(rc);
       if (l == 1 && (rc = make_tmap(&nb.m_w1k_h, nb.wn[l], H, H, H, 64, H / 2))) return fail(rc);
       if (l >= 1) {
-        for (int j = 0; j < c->hsplit; ++j) {
+        for (int j = 0; j < c->plan.hsplit; ++j) {
           int n_off, n;
-          col_group(H, c->hsplit, j, &n_off, &n);
+          col_group(H, c->plan.hsplit, j, &n_off, &n);
           if ((rc = make_tmap(&nb.m_wn[2 * l + j], nb.wn[l], H, H, H, 64, n))) return fail(rc);
         }
       }
-      ALLOC(nb.dw_part[l], static_cast<size_t>(c->S) * in_l * H);
-      ALLOC(nb.dbias[l], static_cast<size_t>(c->S) * H);
-      if ((rc = make_tmap_f32_3d(&nb.m_dw[l], nb.dw_part[l], H, in_l, c->S))) return fail(rc);
+      ALLOC(nb.dw_part[l], static_cast<size_t>(c->plan.S) * in_l * H);
+      ALLOC(nb.dbias[l], static_cast<size_t>(c->plan.S) * H);
+      if ((rc = make_tmap_f32_3d(&nb.m_dw[l], nb.dw_part[l], H, in_l, c->plan.S))) return fail(rc);
     }
   }
   c->pol_tiles = (c->Nl + 127) / 128;
@@ -1177,7 +1179,7 @@ int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, con
   cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
   const int L = c->L, H = c->H;
   if (!(flags & MINPPO_POLICY_WEIGHTS_CURRENT)) RET(enqueue_weight_images(c, params, stream));
-  if (c->fused) {
+  if (c->plan.fused) {
     // 2-hidden-layer nets: ONE launch (policy_fused.cuh) -- observation conversion, both hidden layers, heads, sampler
     PolicyParams pp;
     memset(&pp, 0, sizeof(pp));
@@ -1198,7 +1200,7 @@ int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, con
     pp.n0 = c->n0; pp.n_total = static_cast<long long>(c->N) * c->A;
     pp.rows = c->Nl; pp.D = c->D; pp.Dp = c->Dp; pp.H = H; pp.A = c->A; pp.mode = c->cfg.prng_mode;
     pp.net_first = actor ? 0 : 1;
-    const cudaError_t e = policy_fused_launch(pp, c->pol_tiles, stream, c->ap);
+    const cudaError_t e = policy_fused_launch(pp, c->pol_tiles, stream, c->plan.ap);
     if (e != cudaSuccess) { set_error("policy_fused launch failed: %s", cudaGetErrorString(e)); return MINPPO_ERR_CUDA; }
     return 0;
   }
@@ -1270,7 +1272,7 @@ int minppo_ctx_check(minppo_ctx* c, void* stream_v) {
   std::vector<int32_t> counts(EM);
   CK(cudaMemcpy(counts.data(), c->counts, EM * sizeof(int32_t), cudaMemcpyDeviceToHost));
   for (int s = 0; s < EM; ++s)
-    if (counts[s] > c->cap) { set_error("minibatch %d: %d local rows exceed capacity %d", s, counts[s], c->cap); return MINPPO_ERR_WORKSPACE; }
+    if (counts[s] > c->plan.row_cap) { set_error("minibatch %d: %d local rows exceed capacity %d", s, counts[s], c->plan.row_cap); return MINPPO_ERR_WORKSPACE; }
   std::vector<float> gn(EM);
   CK(cudaMemcpy(gn.data(), c->gnorms, EM * sizeof(float), cudaMemcpyDeviceToHost));
   for (int s = 0; s < EM; ++s)

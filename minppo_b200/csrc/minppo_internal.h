@@ -16,6 +16,8 @@ enum : int { ACTK_TANH = 0, ACTK_RELU = 1, ACTK_TANH_FAST = 2 };   // == ACT_* i
 constexpr int MAX_HIDDEN = 512;
 // widest act_dim: above 32 (FS_MAX_AP) the heads run on the layer-wise kernels' 64-wide templates
 constexpr int MAX_ACT_DIM = 64;
+// head template width of the layer-wise kernels (head_loss_kernel, policy_head_kernel) for act_dim A
+inline int head_amax(int A) { return A <= 8 ? 8 : (A <= 16 ? 16 : (A <= 32 ? 32 : 64)); }
 
 // Per-minibatch sums the loss kernels hand to the optimizer kernel: a block of LOSS_SUMS floats in every per-tile partial
 // (at po_loss), reduced in fixed order into gflat[P + i] and, on env-sharded ranks, all-reduced with the gradient:

@@ -132,7 +132,7 @@ int policy_head_init() {
 
 int policy_head_launch(const PolicyHeadArgs& a, cudaStream_t stream) {
   if (a.A > MAX_ACT_DIM || a.H % 8 != 0 || a.rows <= 0) { set_error("policy head: unsupported shape"); return MINPPO_ERR_ARG; }
-  const int amax = a.A <= 8 ? 8 : (a.A <= 16 ? 16 : (a.A <= 32 ? 32 : 64));
+  const int amax = head_amax(a.A);
   const size_t smem = policy_head_smem(a.H, amax);
   const int blocks = (a.rows + PH_ROWS - 1) / PH_ROWS;
   if (amax == 8) policy_head_kernel<8><<<blocks, PH_THREADS, smem, stream>>>(a);

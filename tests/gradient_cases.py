@@ -1,26 +1,27 @@
-"""Shapes of the per-leaf gradient tests and the learner's path selection restated in Python.
+"""Shapes of the per-leaf gradient tests and the learner path each of them must reach.
 
 ``CASES`` is shared by tests/test_gpu_gradient_leaves.py (the GPU against the oracle) and
 tests/test_gradient_check_host.py (the oracle against itself, no device).  Every case runs one
 minibatch step (E = M = 1), so the minibatch is the whole batch: mb = num_envs * num_steps.
 
-``learner_path`` repeats the host-side choices of minppo_ctx_create / enqueue_step
-(minppo_b200/csrc/learner.cu, dwopt.cuh, head_loss.cu) from the shapes and the SM count, so that
-each case can assert the path it is meant to reach: a heuristic change that moves a case to another
-path then fails the case instead of silently testing something else.  ``launches`` is observable
-(``Learner.launches_per_update``) and ties the restatement to the library.
+``learner_path`` asks the library (minppo_plan, the host-only path decision of minppo_ctx_create)
+which kernels a shape reaches at an SM count, so that each case can assert the path it is meant to
+reach: a heuristic change that moves a case to another path then fails the case instead of silently
+testing something else.  ``launches`` counts the launches of one update on that path; the GPU tests
+compare it with the count the library issued (``Learner.launches_per_update``).
 """
 from __future__ import annotations
 
+import ctypes as C
 import math
+import os
+from unittest import mock
 
+from minppo_b200 import _lib
+from minppo_b200.config import to_c_config
 from oracle import ppo_numpy as P
 from oracle import threefry
-
-DWOPT_THREADS = 512          # dwopt.cuh
-GEMM_MAXN = 256              # umma_gemm.cuh: widest tcgen05 tile; wider hidden layers run as two column groups
-GEMM_MAX_GROUPS = 8
-FS_MAX_AP = 32               # fused_step.cuh: widest padded head of the fused step kernel
+from tests.helpers import hyper_to_config
 
 
 def _case(N, T, D, A, H=256, L=2, cfg=None, expect=None, force_cap=None, **hp):
@@ -75,58 +76,21 @@ for _s in (1, 2, 3, 4, 8):
                                            expect=dict(fused=False, S=_s, two_launch=False))
 
 
-def param_count(D: int, A: int, H: int, L: int) -> int:
-    n = 0
-    for out in (A, 1):
-        fan_in = D
-        for i in range(L + 1):
-            o = H if i < L else out
-            n += o + fan_in * o
-            fan_in = o
-    return n + A
-
-
 def perm_launch_count(B: int) -> int:          # prng_sort.cu
     return math.ceil(3.0 * math.log(max(B, 1)) / math.log(4294967295.0)) * 4 * 3
 
 
 def learner_path(hp: dict, D: int, A: int, sm_count: int, cfg: dict | None = None, force_cap: int | None = None) -> dict:
-    """The single-GPU path minppo_ctx_create picks for a shape (learner.cu), and the launch count of one update."""
-    cfg = cfg or {}
+    """The single-GPU path the library plans for a shape (minppo_plan), and the launch count of one update.
+    ``cfg``: keyword arguments of tests.helpers.hyper_to_config; ``force_cap``: MINPPO_FORCE_CAP for the call."""
     h = P.Hyper(**hp)
-    H, L, E, M, B = h.hidden_size, h.num_layers, h.update_epochs, h.num_minibatches, h.batch_size
-    mb = B // M
-    padded = force_cap is not None
-    cap = force_cap if padded else mb
-    M_pad = (cap + 127) // 128 * 128
-    Dp = (D + 63) // 64 * 64
-    fused = cfg.get("fused", True) and L == 2 and H <= GEMM_MAXN and A <= FS_MAX_AP
-    n_params = param_count(D, A, H, L)
-    cap1 = 4 * sm_count * DWOPT_THREADS
-    maxu = 1 if n_params <= cap1 else (2 if n_params <= 2 * cap1 else 4)
-    dw_nsplit = 2 if H > GEMM_MAXN else (2 if fused and H % 128 == 0 and 2 * 2 * L <= GEMM_MAX_GROUPS else 1)
-    per_split = sum(2 * dw_nsplit * (((Dp if l == 0 else H) + 127) // 128) for l in range(L))
-    budget = sm_count - 16 if sm_count > 48 else sm_count
-    S = cfg.get("dw_splits", 0) or budget // max(per_split, 1)
-    kb_total = M_pad // 64
-    if padded:
-        kb_total = max(min(M_pad, int(mb + 3.0 * math.sqrt(mb)) + 1 + 63) // 64, 1)
-    S = max(min(S, kb_total, 32), 1)
-    while S > 1 and -(-kb_total // S) * (S - 1) >= kb_total:
-        S -= 1
-    gemm_ctas = per_split * S
-    two_launch = gemm_ctas > sm_count
-    # register-resident (fast) dwopt path: the 4-element units of the "late" leaves (hidden kernels; layer-wise also the
-    # hidden biases, whose column sums the dW GEMM computes) fit MAXU per thread of the one-CTA-per-SM grid
-    late = 0
-    fan_in = D
-    for _ in range(L):
-        late += fan_in * H + (0 if fused else H)
-        fan_in = H
-    late *= 2
-    fast = late // 4 <= sm_count * DWOPT_THREADS * maxu
-    per_step = (1 if fused else 2 * L) + (2 if two_launch else 1)
-    launches = 2 + 1 + perm_launch_count(B) + 1 + 3 + E * M * per_step
-    return dict(fused=fused, P=n_params, maxu=maxu, fast=fast, dw_nsplit=dw_nsplit, hsplit=2 if H > GEMM_MAXN else 1,
-                ap=16 if A <= 16 else 32, head_amax=8 if A <= 8 else (16 if A <= 16 else (32 if A <= 32 else 64)),
-                S=S, gemm_ctas=gemm_ctas, two_launch=two_launch, padded=padded, cap=M_pad, launches=launches)
+    c = to_c_config(hyper_to_config(h, **(cfg or {})), D, A)
+    plan = _lib.MinppoPlan()
+    with mock.patch.dict(os.environ, {} if force_cap is None else {"MINPPO_FORCE_CAP": str(force_cap)}):
+        _lib.check(_lib.load().minppo_plan(C.byref(c), sm_count, C.byref(plan)))
+    fused, two_launch = bool(plan.fused), bool(plan.two_launch)
+    per_step = (1 if fused else 2 * h.num_layers) + (2 if two_launch else 1)
+    launches = 2 + 1 + perm_launch_count(h.batch_size) + 1 + 3 + h.update_epochs * h.num_minibatches * per_step
+    return dict(fused=fused, P=plan.num_params, maxu=plan.maxu, fast=bool(plan.dwopt_fast), dw_nsplit=plan.dw_nsplit,
+                hsplit=plan.hsplit, ap=plan.ap, head_amax=plan.head_amax, S=plan.S, gemm_ctas=plan.dw_gemm_ctas,
+                two_launch=two_launch, padded=bool(plan.padded), cap=plan.row_cap, launches=launches)

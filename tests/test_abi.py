@@ -9,6 +9,8 @@ import pytest
 
 from minppo_b200 import _lib, config
 from minppo_b200.params import leaf_paths, leaf_shapes, param_count
+from oracle import ppo_numpy as P
+from tests.helpers import hyper_to_config
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -40,19 +42,32 @@ def test_version_and_error_string(lib):
     assert isinstance(lib.minppo_last_error(), bytes)
 
 
-def test_struct_layout_matches_header():
-    """Field order of the ctypes mirror == field order of struct minppo_config in the header."""
+def _header_fields(begin, end):
     text = open(os.path.join(ROOT, "include", "minppo_b200.h")).read()
-    body = text[text.index("typedef struct minppo_config {"):text.index("} minppo_config;")]
-    body = re.sub(r"/\*.*?\*/", "", body, flags=re.S)
-    names = []
-    for decl in body.split("{", 1)[1].split(";"):
-        decl = decl.strip()
-        if not decl:
-            continue
-        names += [n.strip() for n in decl.split(None, 1)[1].split(",")]
+    start = text.index(begin)
+    body = re.sub(r"/\*.*?\*/", "", text[start:text.index(end, start)], flags=re.S)
+    decls = [d.strip() for d in body.split("{", 1)[1].split(";") if d.strip()]
+    return [n.strip() for d in decls for n in d.split(None, 1)[1].split(",")]
+
+
+def test_struct_layout_matches_header():
+    """Field order of the ctypes mirrors == field order of struct minppo_config and struct minppo_plan in the header."""
+    names = _header_fields("typedef struct minppo_config {", "} minppo_config;")
     assert names == [f[0] for f in _lib.MinppoConfig._fields_]
     assert C.sizeof(_lib.MinppoConfig) == 4 * 4 + 8 + 12 * 4 + 12 * 8            # 4 i32, i64, 12 i32, 12 f64
+    assert _header_fields("struct minppo_plan {", "};") == [f[0] for f in _lib.MinppoPlan._fields_]
+    assert C.sizeof(_lib.MinppoPlan) == 8 + 14 * 4                                # i64, 14 i32
+
+
+@pytest.mark.parametrize("H,L,A,limit", [(576, 2, 2, "<= 512"), (384, 3, 2, "num_layers <= 2"), (256, 2, 65, "<= 64")])
+def test_plan_refuses_what_the_context_refuses(lib, H, L, A, limit):
+    """minppo_plan runs the config check of minppo_ctx_create: the shapes test_wide_hidden_refusals and
+    test_wide_action_refusal hand to a context are refused here with the same code and message, without a device."""
+    hp = P.Hyper(num_envs=16, num_steps=4, num_minibatches=4, hidden_size=H, num_layers=L)
+    cc = config.to_c_config(hyper_to_config(hp), 8, A)
+    plan = _lib.MinppoPlan()
+    assert lib.minppo_plan(C.byref(cc), 148, C.byref(plan)) == _lib.ERR_UNSUPPORTED
+    assert limit in lib.minppo_last_error().decode()
 
 
 @pytest.mark.parametrize("D,A,H,L", [(225, 10, 256, 2), (37, 3, 128, 1), (256, 16, 192, 3)])
@@ -82,3 +97,6 @@ def test_host_side_argument_validation(lib):
     assert lib.minppo_permutation_workspace_size(4, 262144) >= 3 * 4 * 262144 * 4
     with pytest.raises(_lib.MinppoError):
         _lib.check(rc)
+    assert lib.minppo_plan(None, 148, None) == _lib.ERR_ARG
+    cc = config.to_c_config(config.load_config(), 225, 10)
+    assert lib.minppo_plan(C.byref(cc), 0, C.byref(_lib.MinppoPlan())) == _lib.ERR_ARG

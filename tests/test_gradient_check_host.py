@@ -10,9 +10,10 @@
 import numpy as np
 import pytest
 
+from minppo_b200.params import param_count
 from oracle import ppo_numpy as P
 from oracle import synth
-from tests.gradient_cases import CASES, learner_path, param_count
+from tests.gradient_cases import CASES, learner_path
 from tests.helpers import (LEAF_BOUND_BF16, LEAF_BOUND_FP64, clip_adam_flat, compare_leaves, flat_grads, fp64_leaf_bounds,
                            leaf_errors, leaves_over, perturb_policy, rel_err, single_step_oracle_grads)
 
@@ -100,8 +101,8 @@ def test_emulated_oracle_meets_the_fp64_leaf_bound(name):
 
 @pytest.mark.parametrize("name", list(CASES))
 def test_cases_reach_their_paths_on_a_b200(name):
-    """At the B200's 148 SMs every case reaches the path it names (the GPU test asserts the same with the device's own
-    SM count and the library's launch count)."""
+    """At the B200's 148 SMs the library plans for every case the path it names (the GPU test asserts the same with the
+    device's own SM count and the library's launch count)."""
     case = CASES[name]
     path = learner_path(case["hp"], case["D"], case["A"], 148, case["cfg"], case.get("force_cap"))
     for k, v in case["expect"].items():
