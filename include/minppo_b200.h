@@ -185,6 +185,41 @@ int minppo_update_with_stats(minppo_ctx* ctx, float* params, float* mu, float* n
                              const uint8_t* done, const float* last_val, const uint32_t* key_in, uint32_t* key_out,
                              float* losses_out, float* stats_out, int32_t use_graph, void* stream);
 
+/* ---- running observation normalization (optional; minppo_update_normalized, minppo_policy_step_normalized) --------
+ * State: caller-owned device buffers, like the train state -- mean f32 [D], var f32 [D] (population variance), count f64
+ * [1]; the initial state is mean = 0, var = 1, count = 0.  eps (usually 1e-8) and clip (usually 10; <= 0: no clip) are
+ * host scalars.  Every observation the networks see is, in fp32 with IEEE round-to-nearest,
+ *   s_j = 1 / sqrtf(var_j + (float)eps),  y = clamp((x - mean_j) * s_j, -clip, clip)
+ * and then rounded to bf16 like an unnormalized observation (NumPy float32 reproduces y bit for bit:
+ * oracle/ppo_numpy.py normalize_obs).
+ * Contract: rollout k runs the policy step with S_k, which it only reads.  The update of that trajectory normalizes every
+ * row with S_k as well (the statistics the trajectory's log_prob and value were computed with; Brax updates first, this
+ * does not) and, stream-ordered after its last minibatch step, folds its GLOBAL batch (T * N rows, every rank) into the
+ * buffers in place, leaving S_k+1.  The fold is Chan's parallel merge in fp64 of the running (n, mean, var) with the batch
+ * moments (n_b, mean_b, M2_b), d = mean_b - mean:
+ *   n' = n + n_b;  mean' = mean + d n_b / n';  var' = (var n + M2_b + d^2 n n_b / n') / n'
+ * stored as f32 mean / var and f64 count.  The batch moments are per-column Welford sums in fp64 in a fixed order; with
+ * world_size > 1 every rank all-gathers the per-rank moments and merges them in rank order.  The statistics are therefore
+ * bit-identical run to run and on every rank.  The update and the fold support obs_dim <= 1024. */
+typedef struct minppo_obs_norm {
+  float* mean; float* var; double* count;   /* device: f32 [D], f32 [D], f64 [1] */
+  double eps, clip;                          /* clip <= 0: no clip */
+} minppo_obs_norm;
+
+/* minppo_update_with_stats with observation normalization (norm_host == NULL: exactly minppo_update_with_stats).  The
+ * three buffers and eps / clip are part of the graph cache's pointer set.  One update enqueues 2 more launches (1-rank)
+ * or 3 (world_size > 1: the all-gather), timed as class 3 (observation image) by the profiler. */
+int minppo_update_normalized(minppo_ctx* ctx, float* params, float* mu, float* nu, int32_t* count, const float* obs,
+                             const float* action, const float* value, const float* reward, const float* log_prob,
+                             const uint8_t* done, const float* last_val, const uint32_t* key_in, uint32_t* key_out,
+                             float* losses_out, float* stats_out, const minppo_obs_norm* norm_host, int32_t use_graph,
+                             void* stream);
+
+/* Folds `rows` observations obs f32 [rows, D] into the statistics, exactly as an update over the same rows does
+ * (bit-identical on one process), without a context: for warming the statistics up from a random-policy rollout before
+ * training.  Single process; stream-ordered; uses stream-ordered scratch memory (cudaMallocAsync). */
+int minppo_obs_norm_fold(const float* obs, int64_t rows, int32_t D, const minppo_obs_norm* norm_host, void* stream);
+
 /* ---- (5) policy / value inference for the rollout: replaces train.py:157-160 and 182-183 ------------
  * One env step's network evaluation on this rank's Nl = N / world_size envs, forward only, on the same bf16 weight
  * images and with the same rounding points as the learner's forward pass:
@@ -204,6 +239,11 @@ int minppo_update_with_stats(minppo_ctx* ctx, float* params, float* mu, float* n
 int minppo_policy_step(minppo_ctx* ctx, const float* params, const float* obs, const uint32_t* key_in,
                        uint32_t* key_out, float* action, float* log_prob, float* value, float* mean,
                        int32_t flags, void* stream);
+/* minppo_policy_step on normalized observations (norm_host == NULL: exactly minppo_policy_step).  The statistics are
+ * only read; norm_host->count may be NULL. */
+int minppo_policy_step_normalized(minppo_ctx* ctx, const float* params, const float* obs, const uint32_t* key_in,
+                                  uint32_t* key_out, float* action, float* log_prob, float* value, float* mean,
+                                  const minppo_obs_norm* norm_host, int32_t flags, void* stream);
 
 /* Device-side error flag of the last update (0 = ok); synchronises `stream`. */
 int minppo_ctx_check(minppo_ctx* ctx, void* stream);

@@ -6,6 +6,7 @@ Public surface:
   minppo_b200.config   -- mirror of the rl.* / training.* / opt.* / model.* config keys
   minppo_b200.params   -- checkpoint pickle layout <-> flat fp32 arena
   minppo_b200.learner  -- Learner.update (the seam of _update_step), Learner.policy_step, calculate_gae, permutations
+  minppo_b200.obs_norm -- ObsNormalizer: running observation statistics for the update, the policy step and checkpoints
   minppo_b200.infer    -- InferencePolicy: checkpoint pickle -> deterministic / sampled actions (infer.py:17-27)
   minppo_b200._lib     -- ctypes binding of the C ABI (include/minppo_b200.h)
 """
@@ -21,4 +22,9 @@ def __getattr__(name):
 
         mod = importlib.import_module(".learner", __name__)
         return mod if name == "learner" else getattr(mod, name)
+    if name in ("obs_norm", "ObsNormalizer"):
+        import importlib
+
+        mod = importlib.import_module(".obs_norm", __name__)
+        return mod if name == "obs_norm" else mod.ObsNormalizer
     raise AttributeError(name)

@@ -25,6 +25,7 @@ SYMBOLS = (
     "minppo_ctx_check", "minppo_update_launch_count", "minppo_ctx_read", "minppo_debug_gemm",
     "minppo_ctx_profile", "minppo_ctx_profile_read", "minppo_ctx_ipc_handle", "minppo_ctx_set_peers",
     "minppo_policy_step", "minppo_update_with_stats", "minppo_plan",
+    "minppo_update_normalized", "minppo_policy_step_normalized", "minppo_obs_norm_fold",
 )
 POLICY_WEIGHTS_CURRENT = 1
 PROFILE_CLASSES = ("gae", "perm_sort", "rows_and_adv_stats", "obs_image", "weight_images", "fwd_gemm", "head_loss",
@@ -52,6 +53,11 @@ class MinppoPlan(C.Structure):
     _fields_ = [("num_params", C.c_int64)] + [(n, C.c_int32) for n in (
         "fused", "ap", "head_amax", "hsplit", "dw_nsplit", "S", "dw_gemm_ctas", "two_launch",
         "maxu", "dwopt_fast", "padded", "row_cap", "peer_exchange")]
+
+
+class MinppoObsNorm(C.Structure):
+    """``struct minppo_obs_norm`` -- field order and types must match the header."""
+    _fields_ = [("mean", C.c_void_p), ("var", C.c_void_p), ("count", C.c_void_p), ("eps", C.c_double), ("clip", C.c_double)]
 
 
 class MinppoError(RuntimeError):
@@ -102,6 +108,11 @@ def load() -> C.CDLL:
     lib.minppo_update.argtypes = [vp] + [vp] * 14 + [i32, vp]
     lib.minppo_update_with_stats.restype = C.c_int
     lib.minppo_update_with_stats.argtypes = [vp] + [vp] * 15 + [i32, vp]
+    norm = C.POINTER(MinppoObsNorm)
+    lib.minppo_update_normalized.restype = C.c_int
+    lib.minppo_update_normalized.argtypes = [vp] + [vp] * 15 + [norm, i32, vp]
+    lib.minppo_obs_norm_fold.restype = C.c_int
+    lib.minppo_obs_norm_fold.argtypes = [vp, i64, i32, norm, vp]
     lib.minppo_ctx_check.restype = C.c_int
     lib.minppo_ctx_check.argtypes = [vp, vp]
     lib.minppo_update_launch_count.restype = i64
@@ -118,6 +129,8 @@ def load() -> C.CDLL:
     lib.minppo_ctx_set_peers.argtypes = [vp, vp]
     lib.minppo_policy_step.restype = C.c_int
     lib.minppo_policy_step.argtypes = [vp] * 9 + [i32, vp]
+    lib.minppo_policy_step_normalized.restype = C.c_int
+    lib.minppo_policy_step_normalized.argtypes = [vp] * 9 + [norm, i32, vp]
     lib.minppo_debug_gemm.restype = C.c_int
     lib.minppo_debug_gemm.argtypes = [i32, vp, vp, vp, vp, i32, i32, i32, i32, i32, vp]
     _lib = lib

@@ -112,6 +112,7 @@ struct NcclApi {
   ncclResult_t (*CommInitRank)(ncclComm_t*, int, ncclUniqueId, int);
   ncclResult_t (*AllReduce)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t);
   ncclResult_t (*Broadcast)(const void*, void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t);
+  ncclResult_t (*AllGather)(const void*, void*, size_t, ncclDataType_t, ncclComm_t, cudaStream_t);
   ncclResult_t (*GroupStart)();
   ncclResult_t (*GroupEnd)();
   ncclResult_t (*CommDestroy)(ncclComm_t);
@@ -130,11 +131,12 @@ static NcclApi* nccl_api() {
       api.CommInitRank = reinterpret_cast<decltype(api.CommInitRank)>(dlsym(h, "ncclCommInitRank"));
       api.AllReduce = reinterpret_cast<decltype(api.AllReduce)>(dlsym(h, "ncclAllReduce"));
       api.Broadcast = reinterpret_cast<decltype(api.Broadcast)>(dlsym(h, "ncclBroadcast"));
+      api.AllGather = reinterpret_cast<decltype(api.AllGather)>(dlsym(h, "ncclAllGather"));
       api.GroupStart = reinterpret_cast<decltype(api.GroupStart)>(dlsym(h, "ncclGroupStart"));
       api.GroupEnd = reinterpret_cast<decltype(api.GroupEnd)>(dlsym(h, "ncclGroupEnd"));
       api.CommDestroy = reinterpret_cast<decltype(api.CommDestroy)>(dlsym(h, "ncclCommDestroy"));
       api.GetErrorString = reinterpret_cast<decltype(api.GetErrorString)>(dlsym(h, "ncclGetErrorString"));
-      api.ok = api.GetUniqueId && api.CommInitRank && api.AllReduce && api.Broadcast && api.GroupStart && api.GroupEnd &&
+      api.ok = api.GetUniqueId && api.CommInitRank && api.AllReduce && api.Broadcast && api.AllGather && api.GroupStart && api.GroupEnd &&
                api.CommDestroy && api.GetErrorString;
     }
   }
@@ -241,6 +243,9 @@ struct UpdatePtrs {
   uint32_t* key_out;
   float* losses_out;
   float* stats_out;
+  float *norm_mean, *norm_var;  // running observation statistics (minppo_update_normalized), or null
+  double* norm_count;
+  double norm_eps, norm_clip;
   bool operator==(const UpdatePtrs& o) const { return memcmp(this, &o, sizeof(*this)) == 0; }
 };
 
@@ -263,6 +268,9 @@ struct minppo_ctx {
   void* perm_ws;
   size_t perm_ws_bytes;
   __nv_bfloat16* obs_img;
+  double* obs_part;           // observation normalization (Dp <= OBS_NORM_MAX_D): block moments of the image kernel
+  double* obs_mom;            //   [world_size][obs_mom_stride] per-rank batch moments [n, mean[D], M2[D]] (all-gathered)
+  int obs_mom_stride;
   __nv_bfloat16* xg;           // gathered observation rows of the current minibatch [M_pad][Dp] (fused path)
   CUtensorMap m_xg_k, m_xg_mn;
   unsigned long long* barrier;
@@ -721,6 +729,21 @@ static int enqueue_step(minppo_ctx* c, const UpdatePtrs& u, int s, cudaStream_t 
   return 0;
 }
 
+// The bf16 observation image of the update; with normalization also this rank's batch moments (two launches).
+static int enqueue_obs_image(minppo_ctx* c, const UpdatePtrs& u, cudaStream_t stream) {
+  if (!u.norm_mean) {
+    RET(obs_image_launch(u.obs, c->obs_img, c->Bl, c->D, c->Dp, stream));
+    c->launches++;
+    return 0;
+  }
+  const ObsNormArgs na = {u.norm_mean, u.norm_var, static_cast<float>(u.norm_eps), static_cast<float>(u.norm_clip), c->obs_part};
+  double* mine = c->obs_mom + static_cast<size_t>(c->cfg.rank) * c->obs_mom_stride;
+  RET(obs_norm_image_launch(u.obs, c->obs_img, c->Bl, c->D, c->Dp, na, stream));
+  RET(obs_moments_finalize_launch(c->obs_part, c->Bl, c->D, c->Dp, mine, stream));
+  c->launches += 2;
+  return 0;
+}
+
 static int enqueue_update(minppo_ctx* c, const UpdatePtrs& u, cudaStream_t stream) {
   const minppo_config& cfg = c->cfg;
   c->launches = 0;
@@ -736,10 +759,10 @@ static int enqueue_update(minppo_ctx* c, const UpdatePtrs& u, cudaStream_t strea
   if (fork) {
     CK(cudaEventRecord(c->ev_fork, stream));
     CK(cudaStreamWaitEvent(c->side_stream, c->ev_fork, 0));
-    RET(obs_image_launch(u.obs, c->obs_img, c->Bl, c->D, c->Dp, c->side_stream));
+    RET(enqueue_obs_image(c, u, c->side_stream));
     RET(enqueue_weight_images(c, u.params, c->side_stream));
     CK(cudaEventRecord(c->ev_join, c->side_stream));
-    c->launches += 2;
+    c->launches += 1;
   }
   {
     PROF(PC_GAE);
@@ -785,8 +808,7 @@ static int enqueue_update(minppo_ctx* c, const UpdatePtrs& u, cudaStream_t strea
   } else {
     {
       PROF(PC_OBS_IMAGE);
-      RET(obs_image_launch(u.obs, c->obs_img, c->Bl, c->D, c->Dp, stream));
-      c->launches++;
+      RET(enqueue_obs_image(c, u, stream));
     }
     // the weight images must match the caller's params at entry (they may have been replaced)
     {
@@ -796,6 +818,22 @@ static int enqueue_update(minppo_ctx* c, const UpdatePtrs& u, cudaStream_t strea
     }
   }
   for (int s = 0; s < EM; ++s) RET(enqueue_step(c, u, s, stream));
+  if (u.norm_mean) {
+    // Fold this update's batch into the running statistics.  After the last step rather than at the join: the image kernel
+    // has long finished reading the entry statistics, and the merge stays off the first step's critical path.  NCCL stays
+    // on this stream (one stream per communicator); the rank-order merge gives every rank the same bits.
+    PROF(PC_OBS_IMAGE);
+    const int W = cfg.world_size;
+    if (W > 1) {
+      NcclApi* api = nccl_api();
+      const size_t n = static_cast<size_t>(c->obs_mom_stride);
+      const ncclResult_t r = api->AllGather(c->obs_mom + cfg.rank * n, c->obs_mom, n, ncclFloat64, c->comm, stream);
+      if (r != ncclSuccess) { set_error("ncclAllGather (observation moments) failed: %s", api->GetErrorString(r)); return MINPPO_ERR_NCCL; }
+      c->launches++;
+    }
+    RET(obs_norm_merge_launch(c->obs_mom, W, c->obs_mom_stride, c->D, u.norm_mean, u.norm_var, u.norm_count, stream));
+    c->launches++;
+  }
   return 0;
 }
 
@@ -1037,6 +1075,12 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   { uint8_t* p; ALLOC(p, c->perm_ws_bytes); c->perm_ws = p; }
   ALLOC(c->obs_img, static_cast<size_t>(c->Bl) * c->Dp + 256);   // slack: MN gather may read one chunk past Dp
   ALLOC(c->xg, static_cast<size_t>(c->plan.row_cap) * c->Dp);
+  c->obs_part = c->obs_mom = nullptr;
+  c->obs_mom_stride = (1 + 2 * c->D + 1) / 2 * 2;
+  if (c->Dp <= OBS_NORM_MAX_D) {
+    ALLOC(c->obs_part, static_cast<size_t>(obs_norm_blocks(c->Bl, c->Dp)) * 2 * c->Dp);
+    ALLOC(c->obs_mom, static_cast<size_t>(cfg->world_size) * c->obs_mom_stride);
+  }
   if ((rc = make_tmap(&c->m_xg_k, c->xg, c->Dp, c->plan.row_cap, c->Dp, 64, 128))) return fail(rc);
   if ((rc = make_tmap(&c->m_xg_mn, c->xg, c->Dp, c->plan.row_cap, c->Dp, 64, 64))) return fail(rc);
   ALLOC(c->barrier, 1);
@@ -1113,14 +1157,32 @@ int minppo_ctx_create(const minppo_config* cfg, const void* nccl_unique_id_host,
   return 0;
 }
 
-int minppo_update_with_stats(minppo_ctx* c, float* params, float* mu, float* nu, int32_t* count, const float* obs,
+// The host half of a minppo_obs_norm: buffers present, eps and clip finite, eps >= 0.
+static int check_obs_norm(const minppo_obs_norm* n, bool need_count, const char* who) {
+  if (!n->mean || !n->var || (need_count && !n->count)) { set_error("%s: null pointer in minppo_obs_norm", who); return MINPPO_ERR_ARG; }
+  if (!(n->eps >= 0.0) || !isfinite(n->eps) || !isfinite(n->clip)) {
+    set_error("%s: minppo_obs_norm needs a finite eps >= 0 and a finite clip (got eps=%g clip=%g)", who, n->eps, n->clip);
+    return MINPPO_ERR_ARG;
+  }
+  return 0;
+}
+
+int minppo_update_normalized(minppo_ctx* c, float* params, float* mu, float* nu, int32_t* count, const float* obs,
                              const float* action, const float* value, const float* reward, const float* log_prob,
                              const uint8_t* done, const float* last_val, const uint32_t* key_in, uint32_t* key_out,
-                             float* losses_out, float* stats_out, int32_t use_graph, void* stream_v) {
+                             float* losses_out, float* stats_out, const minppo_obs_norm* norm_host, int32_t use_graph,
+                             void* stream_v) {
   if (!c || !params || !mu || !nu || !count || !obs || !action || !value || !reward || !log_prob || !done ||
       !last_val || !key_in) {
     set_error("minppo_update: null pointer");
     return MINPPO_ERR_ARG;
+  }
+  if (norm_host) {
+    RET(check_obs_norm(norm_host, true, "minppo_update_normalized"));
+    if (!c->obs_part) {
+      set_error("minppo_update_normalized: obs_dim=%d unsupported with observation normalization (<= %d)", c->D, OBS_NORM_MAX_D);
+      return MINPPO_ERR_UNSUPPORTED;
+    }
   }
   cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
   UpdatePtrs u;
@@ -1128,6 +1190,10 @@ int minppo_update_with_stats(minppo_ctx* c, float* params, float* mu, float* nu,
   u.params = params; u.mu = mu; u.nu = nu; u.count = count; u.obs = obs; u.action = action; u.value = value;
   u.reward = reward; u.log_prob = log_prob; u.done = done; u.last_val = last_val; u.key_in = key_in;
   u.key_out = key_out; u.losses_out = losses_out; u.stats_out = stats_out;
+  if (norm_host) {
+    u.norm_mean = norm_host->mean; u.norm_var = norm_host->var; u.norm_count = norm_host->count;
+    u.norm_eps = norm_host->eps; u.norm_clip = norm_host->clip;
+  }
   if (!use_graph) return enqueue_update(c, u, stream);
   const bool was_profiling = c->profiling;
   c->profiling = false;                         // event records are not captured; profile in eager mode
@@ -1162,6 +1228,14 @@ int minppo_update_with_stats(minppo_ctx* c, float* params, float* mu, float* nu,
   return 0;
 }
 
+int minppo_update_with_stats(minppo_ctx* c, float* params, float* mu, float* nu, int32_t* count, const float* obs,
+                             const float* action, const float* value, const float* reward, const float* log_prob,
+                             const uint8_t* done, const float* last_val, const uint32_t* key_in, uint32_t* key_out,
+                             float* losses_out, float* stats_out, int32_t use_graph, void* stream_v) {
+  return minppo_update_normalized(c, params, mu, nu, count, obs, action, value, reward, log_prob, done, last_val, key_in,
+                                  key_out, losses_out, stats_out, nullptr, use_graph, stream_v);
+}
+
 int minppo_update(minppo_ctx* c, float* params, float* mu, float* nu, int32_t* count, const float* obs,
                   const float* action, const float* value, const float* reward, const float* log_prob,
                   const uint8_t* done, const float* last_val, const uint32_t* key_in, uint32_t* key_out,
@@ -1170,9 +1244,11 @@ int minppo_update(minppo_ctx* c, float* params, float* mu, float* nu, int32_t* c
                                   key_out, losses_out, nullptr, use_graph, stream_v);
 }
 
-int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, const uint32_t* key_in, uint32_t* key_out,
-                       float* action, float* log_prob, float* value, float* mean, int32_t flags, void* stream_v) {
+int minppo_policy_step_normalized(minppo_ctx* c, const float* params, const float* obs, const uint32_t* key_in,
+                                  uint32_t* key_out, float* action, float* log_prob, float* value, float* mean,
+                                  const minppo_obs_norm* norm_host, int32_t flags, void* stream_v) {
   if (!c || !params || !obs) { set_error("minppo_policy_step: null pointer"); return MINPPO_ERR_ARG; }
+  if (norm_host) RET(check_obs_norm(norm_host, false, "minppo_policy_step_normalized"));
   if (key_in && key_out == key_in) { set_error("minppo_policy_step: key_out must not alias key_in"); return MINPPO_ERR_ARG; }
   const bool actor = action || log_prob || mean;
   if (!actor && !value) { set_error("minppo_policy_step: no output requested"); return MINPPO_ERR_ARG; }
@@ -1200,12 +1276,22 @@ int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, con
     pp.n0 = c->n0; pp.n_total = static_cast<long long>(c->N) * c->A;
     pp.rows = c->Nl; pp.D = c->D; pp.Dp = c->Dp; pp.H = H; pp.A = c->A; pp.mode = c->cfg.prng_mode;
     pp.net_first = actor ? 0 : 1;
-    const cudaError_t e = policy_fused_launch(pp, c->pol_tiles, stream, c->plan.ap);
+    if (norm_host) {
+      pp.norm_mean = norm_host->mean; pp.norm_var = norm_host->var;
+      pp.norm_eps = static_cast<float>(norm_host->eps); pp.norm_clip = static_cast<float>(norm_host->clip);
+    }
+    const cudaError_t e = policy_fused_launch(pp, c->pol_tiles, stream, c->plan.ap, norm_host != nullptr);
     if (e != cudaSuccess) { set_error("policy_fused launch failed: %s", cudaGetErrorString(e)); return MINPPO_ERR_CUDA; }
     return 0;
   }
   // bf16 image of last_obs, zero padded to Dp columns (rows >= Nl of the image stay zero from allocation)
-  RET(obs_image_launch(obs, c->pol_img, c->Nl, c->D, c->Dp, stream));
+  if (norm_host) {
+    const ObsNormArgs na = {norm_host->mean, norm_host->var, static_cast<float>(norm_host->eps),
+                            static_cast<float>(norm_host->clip), nullptr};
+    RET(obs_norm_image_launch(obs, c->pol_img, c->Nl, c->D, c->Dp, na, stream));
+  } else {
+    RET(obs_image_launch(obs, c->pol_img, c->Nl, c->D, c->Dp, stream));
+  }
   const int first = actor ? 0 : 1;                        // critic only: the bootstrap value (train.py:182-183)
   for (int l = 0; l < L; ++l) {
     FwdOperands op[2];
@@ -1226,6 +1312,31 @@ int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, con
   a.key_in = actor ? key_in : nullptr; a.key_out = actor ? key_out : nullptr; a.mode = c->cfg.prng_mode;
   a.action = action; a.log_prob = log_prob; a.value = value; a.mean_out = mean;
   return policy_head_launch(a, stream);
+}
+
+int minppo_policy_step(minppo_ctx* c, const float* params, const float* obs, const uint32_t* key_in, uint32_t* key_out,
+                       float* action, float* log_prob, float* value, float* mean, int32_t flags, void* stream_v) {
+  return minppo_policy_step_normalized(c, params, obs, key_in, key_out, action, log_prob, value, mean, nullptr, flags,
+                                       stream_v);
+}
+
+int minppo_obs_norm_fold(const float* obs, int64_t rows, int32_t D, const minppo_obs_norm* norm_host, void* stream_v) {
+  if (!obs || !norm_host || rows <= 0 || D <= 0) { set_error("minppo_obs_norm_fold: null pointer or non-positive size"); return MINPPO_ERR_ARG; }
+  RET(check_obs_norm(norm_host, true, "minppo_obs_norm_fold"));
+  const int ld = (D + 63) / 64 * 64;                    // the update's image row: the same partials, bit for bit
+  if (ld > OBS_NORM_MAX_D) { set_error("minppo_obs_norm_fold: obs_dim=%d unsupported (<= %d)", D, OBS_NORM_MAX_D); return MINPPO_ERR_UNSUPPORTED; }
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_v);
+  const size_t part = static_cast<size_t>(obs_norm_blocks(rows, ld)) * 2 * ld;
+  double* ws = nullptr;
+  CK(cudaMallocAsync(reinterpret_cast<void**>(&ws), (part + 1 + 2 * static_cast<size_t>(D)) * sizeof(double), stream));
+  const ObsNormArgs na = {norm_host->mean, norm_host->var, static_cast<float>(norm_host->eps),
+                          static_cast<float>(norm_host->clip), ws};
+  int r = obs_norm_image_launch(obs, nullptr, rows, D, ld, na, stream);
+  if (!r) r = obs_moments_finalize_launch(ws, rows, D, ld, ws + part, stream);
+  if (!r) r = obs_norm_merge_launch(ws + part, 1, 0, D, norm_host->mean, norm_host->var, norm_host->count, stream);
+  if (r) set_error("minppo_obs_norm_fold: launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+  CK(cudaFreeAsync(ws, stream));
+  return r;
 }
 
 int minppo_ctx_ipc_handle(minppo_ctx* c, void* handle64_host) {

@@ -158,6 +158,26 @@ struct OptArgs {
 int weight_images_launch(const OptArgs& a, cudaStream_t stream);
 int obs_image_launch(const float* obs, __nv_bfloat16* img, long long rows, int cols, int ld, cudaStream_t stream);
 
+// Observation normalization (include/minppo_b200.h, minppo_obs_norm): operands of the normalizing image kernel.
+constexpr int OBS_NORM_MAX_D = 1024;          // widest padded observation row whose moments the image kernel accumulates
+constexpr int OBS_NORM_MAX_BLOCKS = 148 * 3;  // most block partials of one moments pass (obs_norm_blocks)
+struct ObsNormArgs {
+  const float* mean;             // [cols] running statistics at entry (read only)
+  const float* var;              // [cols]
+  float eps, clip;               // clip <= 0: no clamp
+  double* part;                  // null: normalized image only; else the per-block moments [obs_norm_blocks][2][ld]
+};
+int obs_norm_blocks(long long rows, int ld);
+// Normalized observation image (img may be null when na.part is set: moments only), plus the block partials of the raw
+// observations' moments when na.part is set (ld <= OBS_NORM_MAX_D).
+int obs_norm_image_launch(const float* obs, __nv_bfloat16* img, long long rows, int cols, int ld, const ObsNormArgs& na,
+                          cudaStream_t stream);
+// The partials of an obs_norm_image_launch over `rows` rows merged into out = [rows, mean[cols], M2[cols]] (f64).
+int obs_moments_finalize_launch(const double* part, long long rows, int cols, int ld, double* out, cudaStream_t stream);
+// The moments of W ranks ([W][stride], rank order) folded into the running statistics in place.
+int obs_norm_merge_launch(const double* moments, int W, int stride, int D, float* mean, float* var, double* count,
+                          cudaStream_t stream);
+
 // ---- launch helper: optional programmatic-dependent-launch edge to the preceding kernel ------
 template <typename Kern, typename Arg>
 inline cudaError_t launch_kernel(Kern kern, unsigned grid, unsigned block, size_t smem, cudaStream_t stream, bool pdl,

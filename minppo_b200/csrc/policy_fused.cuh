@@ -9,10 +9,12 @@
 // seen by the first PPO epoch with ratio == 1 and v == v_old up to fp32 rounding of the final sums.  The actor CTAs then
 // draw eps = jax.random.normal(action_rng, (N, A)) at the GLOBAL flat index n * A + j (an env-sharded rank generates
 // exactly its rows of the global sample), form the action and its log-prob; the critic CTAs write the value.
-// Same shared-memory layout, warp roles and tensor maps as fused_step.cuh.
+// Same shared-memory layout, warp roles and tensor maps as fused_step.cuh.  The NORM instances normalize every observation
+// with the running statistics (obs_norm.cuh) before its bf16 rounding.
 #pragma once
 
 #include "fused_step.cuh"
+#include "obs_norm.cuh"
 #include "policy_math.cuh"
 #include "ppo_math.cuh"
 
@@ -40,9 +42,13 @@ struct alignas(64) PolicyParams {
   long long n0, n_total;         // first GLOBAL env of this rank; elements of the global normal draw (N * A)
   int rows, D, Dp, H, A, mode;
   int net_first;                 // 0: actor + critic CTAs; 1: critic only (grid = tiles)
+  // NORM instances: running observation statistics (obs_norm.cuh), applied to every observation as it is loaded
+  const float* norm_mean;        // [D]
+  const float* norm_var;         // [D]
+  float norm_eps, norm_clip;
 };
 
-template <int AP>
+template <int AP, bool NORM>
 __global__ void __launch_bounds__(FS_THREADS, 1) policy_fused_kernel(const __grid_constant__ PolicyParams p) {
   using LY = FsLayout<AP>;
   constexpr int NS = LY::NS, NS1 = LY::NS1, PG = LY::PG;
@@ -189,6 +195,23 @@ __global__ void __launch_bounds__(FS_THREADS, 1) policy_fused_kernel(const __gri
       float v[16];
 #pragma unroll
       for (int e = 0; e < 16; ++e) v[e] = (rlive && c0 + e < p.D) ? __ldg(orow + c0 + e) : 0.f;
+      if constexpr (NORM) {
+        // the 8 lanes of a warp that load the same 16 columns (one per row) share the statistics: lane j of them computes
+        // mean and scale of columns 2j and 2j + 1, and hands them to the others by shuffle
+        float hm[2], hs[2];
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          const int c = c0 + 2 * (lane >> 2) + h;
+          hm[h] = c < p.D ? __ldg(p.norm_mean + c) : 0.f;
+          hs[h] = c < p.D ? obs_norm_scale(__ldg(p.norm_var + c), p.norm_eps) : 0.f;
+        }
+#pragma unroll
+        for (int e = 0; e < 16; ++e) {
+          const int src = ((e >> 1) << 2) | (lane & 3);
+          const float m = __shfl_sync(0xffffffffu, hm[e & 1], src), sc = __shfl_sync(0xffffffffu, hs[e & 1], src);
+          if (rlive && c0 + e < p.D) v[e] = obs_norm_apply(v[e], m, sc, p.norm_clip);
+        }
+      }
       const uint32_t dst = R1 + (kb & 3) * 16384 + xrow * 128;
 #pragma unroll
       for (int h = 0; h < 2; ++h) {
@@ -290,14 +313,21 @@ __global__ void __launch_bounds__(FS_THREADS, 1) policy_fused_kernel(const __gri
   if (warp == FS_MMA_WARP) tmem_dealloc(tmem_base, 512);
 }
 
-inline cudaError_t policy_fused_launch(const PolicyParams& p, int tiles, cudaStream_t stream, int ap) {
+// norm: the NORM instance (p.norm_* set), which normalizes the observations as it loads them
+inline cudaError_t policy_fused_launch(const PolicyParams& p, int tiles, cudaStream_t stream, int ap, bool norm) {
   const int grid = p.net_first ? tiles : 2 * tiles;
-  return ap == 16 ? launch_kernel(policy_fused_kernel<16>, grid, FS_THREADS, FsLayout<16>::BYTES, stream, false, p)
-                  : launch_kernel(policy_fused_kernel<32>, grid, FS_THREADS, FsLayout<32>::BYTES, stream, false, p);
+  if (norm)
+    return ap == 16 ? launch_kernel(policy_fused_kernel<16, true>, grid, FS_THREADS, FsLayout<16>::BYTES, stream, false, p)
+                    : launch_kernel(policy_fused_kernel<32, true>, grid, FS_THREADS, FsLayout<32>::BYTES, stream, false, p);
+  return ap == 16 ? launch_kernel(policy_fused_kernel<16, false>, grid, FS_THREADS, FsLayout<16>::BYTES, stream, false, p)
+                  : launch_kernel(policy_fused_kernel<32, false>, grid, FS_THREADS, FsLayout<32>::BYTES, stream, false, p);
 }
 inline cudaError_t policy_fused_init_attrs() {
-  cudaError_t e = cudaFuncSetAttribute(policy_fused_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, FsLayout<16>::BYTES);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_fused_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, FsLayout<32>::BYTES);
+  cudaError_t e = cudaSuccess;
+  for (auto k : {policy_fused_kernel<16, false>, policy_fused_kernel<16, true>})
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, FsLayout<16>::BYTES);
+  for (auto k : {policy_fused_kernel<32, false>, policy_fused_kernel<32, true>})
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, FsLayout<32>::BYTES);
   return e;
 }
 

@@ -4,6 +4,8 @@ forward pass its `main` never got (infer.py:27 raises NotImplementedError).
 The checkpoint is the reference's pickle of the flax variable dict (train.py:86-89); it is flattened into the fp32 arena
 (minppo_b200.params) and evaluated by minppo_policy_step -- the same tensor-core forward pass the rollout uses
 (train.py:157-160).  `act(obs)` returns the mode of pi (deterministic evaluation); with an rng it samples like the rollout.
+A checkpoint with an "obs_normalizer" entry (minppo_b200.params) is evaluated on observations normalized with the stored
+statistics, as during training; without it the observations are used as they are.
 """
 from __future__ import annotations
 
@@ -15,7 +17,8 @@ import torch
 
 from .config import Config
 from .learner import Learner
-from .params import flatten_params, leaf_shapes, load_model
+from .obs_norm import ObsNormalizer
+from .params import OBS_NORMALIZER_KEY, flatten_params, leaf_shapes, load_model
 
 
 class InferencePolicy:
@@ -36,6 +39,11 @@ class InferencePolicy:
         self._learner = Learner(cfg, self.obs_dim, self.act_dim, device)
         self.device = self._learner.device
         self.params = torch.as_tensor(flat).to(self.device)
+        self.obs_norm = None
+        if OBS_NORMALIZER_KEY in params_tree:
+            self.obs_norm = ObsNormalizer.from_tree(params_tree[OBS_NORMALIZER_KEY], self.device)
+            if self.obs_norm.obs_dim != self.obs_dim:
+                raise ValueError(f"obs_normalizer has {self.obs_norm.obs_dim} features, the policy {self.obs_dim}")
         self._first = True
 
     @classmethod
@@ -47,7 +55,8 @@ class InferencePolicy:
         (sampled action, log_prob, value, rng') exactly like one rollout step."""
         cur = not self._first
         self._first = False
-        action, log_prob, value, rng_out, _ = self._learner.policy_step(self.params, obs, rng, weights_current=cur)
+        action, log_prob, value, rng_out, _ = self._learner.policy_step(self.params, obs, rng, weights_current=cur,
+                                                                        obs_norm=self.obs_norm)
         if rng is None:
             return action, value
         return action, log_prob, value, rng_out

@@ -25,6 +25,7 @@ import torch
 
 from . import _lib
 from .config import Config, to_c_config
+from .obs_norm import ObsNormalizer
 from .params import leaf_paths, leaf_shapes, param_count
 
 
@@ -72,6 +73,14 @@ def _as_u8(done: torch.Tensor) -> torch.Tensor:
     if done.dtype != torch.uint8:
         raise TypeError(f"done must be bool or uint8, got {done.dtype}")
     return done
+
+
+def _norm_arg(obs_norm: Optional[ObsNormalizer], obs_dim: int, device: torch.device):
+    """The ``minppo_obs_norm`` argument: None, or a validated struct passed by reference."""
+    if obs_norm is None:
+        return None
+    obs_norm.check(obs_dim, device)
+    return C.byref(obs_norm.c_struct())
 
 
 def _check(t: torch.Tensor, name: str, dtype: torch.dtype, shape, device: torch.device) -> torch.Tensor:
@@ -218,7 +227,7 @@ class Learner:
     # -- the update -----------------------------------------------------------------------
     def update(self, train_state: TrainState, mem_batch: Memory, last_val: torch.Tensor, rng: torch.Tensor,
                losses: Optional[torch.Tensor] = None, rng_out: Optional[torch.Tensor] = None,
-               stats: Optional[torch.Tensor] = None):
+               stats: Optional[torch.Tensor] = None, obs_norm: Optional[ObsNormalizer] = None):
         """train.py:185-281.  In place on ``train_state``; returns (train_state, rng', losses[E, M, 4])
         with losses columns (total, value_loss, actor_loss, entropy).  Nothing synchronises.
 
@@ -227,6 +236,11 @@ class Learner:
         value_clip_fraction = mean(|v - v_old| > clip_eps) over the rows of the global minibatch, evaluated with the
         parameters before that minibatch's Adam step, and the pre-clip global gradient norm.  Passing it changes
         nothing else the update computes.
+
+        ``obs_norm``: optional ``ObsNormalizer`` (minppo_b200.obs_norm).  Every observation is normalized with its
+        statistics at entry -- those the rollout's policy steps used -- and, stream-ordered after the last minibatch
+        step, the update's global batch is folded into them in place.  Its tensors and eps / clip are part of the
+        graph cache's pointer set.
 
         ``rng`` is copied (8 bytes, stream-ordered) into a learner-owned slot; without ``losses`` / ``rng_out`` the
         results land in learner-owned buffers that the NEXT ``update`` overwrites (pass your own to keep them).  With
@@ -255,22 +269,26 @@ class Learner:
             _check(stats, "stats", torch.float32, (self.E, self.M, len(STATS_COLUMNS)), dev)
         if rng_out is None:
             rng_out = self._key_out.view(rng.dtype)
+        norm = _norm_arg(obs_norm, D, dev)
         with torch.cuda.device(dev):
             if rng.data_ptr() != self._key_in.data_ptr():
                 self._key_in.copy_(rng.reshape(2).view(torch.int32), non_blocking=True)
-            _lib.check(self.lib.minppo_update_with_stats(
+            _lib.check(self.lib.minppo_update_normalized(
                 self._h, _ptr(train_state.params), _ptr(train_state.mu), _ptr(train_state.nu), _ptr(train_state.step),
                 _ptr(obs), _ptr(action), _ptr(value), _ptr(reward), _ptr(log_prob), _ptr(done), _ptr(last_val),
-                _ptr(self._key_in), _ptr(rng_out), _ptr(losses), _ptr(stats), int(self.use_graph), _stream_ptr(dev)))
+                _ptr(self._key_in), _ptr(rng_out), _ptr(losses), _ptr(stats), norm, int(self.use_graph),
+                _stream_ptr(dev)))
         return train_state, rng_out, losses
 
     # -- policy / value inference for the rollout -------------------------------------------
     def policy_step(self, params: torch.Tensor, last_obs: torch.Tensor, rng: Optional[torch.Tensor],
-                    weights_current: bool = False, want_mean: bool = False):
+                    weights_current: bool = False, want_mean: bool = False,
+                    obs_norm: Optional[ObsNormalizer] = None):
         """train.py:157-160: ``pi, value = network.apply(params, last_obs); rng, action_rng = split(rng);
         action = pi.sample(seed=action_rng); log_prob = pi.log_prob(action)`` on this rank's ``Nl`` envs.
         Returns (action [Nl, A], log_prob [Nl], value [Nl], rng', mean or None).  ``rng=None``: no sampling
-        (action = the mode of pi, rng' = None).  Nothing synchronises."""
+        (action = the mode of pi, rng' = None).  ``obs_norm``: evaluate on observations normalized with these
+        statistics (read only).  Nothing synchronises."""
         dev = self.device
         obs = _check(last_obs, "last_obs", torch.float32, (self.Nl, self.obs_dim), dev)
         _check(params, "params", torch.float32, (self.P,), dev)
@@ -281,21 +299,25 @@ class Learner:
         value = torch.empty((self.Nl,), dtype=torch.float32, device=dev)
         mean = torch.empty_like(action) if want_mean else None
         rng_out = torch.empty_like(rng) if rng is not None else None
+        norm = _norm_arg(obs_norm, self.obs_dim, dev)
         with torch.cuda.device(dev):
-            _lib.check(self.lib.minppo_policy_step(
+            _lib.check(self.lib.minppo_policy_step_normalized(
                 self._h, _ptr(params), _ptr(obs), _ptr(rng), _ptr(rng_out), _ptr(action), _ptr(log_prob), _ptr(value),
-                _ptr(mean), _lib.POLICY_WEIGHTS_CURRENT if weights_current else 0, _stream_ptr(dev)))
+                _ptr(mean), norm, _lib.POLICY_WEIGHTS_CURRENT if weights_current else 0, _stream_ptr(dev)))
         return action, log_prob, value, rng_out, mean
 
-    def bootstrap_value(self, params: torch.Tensor, last_obs: torch.Tensor, weights_current: bool = False) -> torch.Tensor:
-        """train.py:182-183: ``_, last_val = network.apply(params, last_obs)`` (critic only)."""
+    def bootstrap_value(self, params: torch.Tensor, last_obs: torch.Tensor, weights_current: bool = False,
+                        obs_norm: Optional[ObsNormalizer] = None) -> torch.Tensor:
+        """train.py:182-183: ``_, last_val = network.apply(params, last_obs)`` (critic only), on observations
+        normalized with ``obs_norm`` (read only) when given."""
         dev = self.device
         obs = _check(last_obs, "last_obs", torch.float32, (self.Nl, self.obs_dim), dev)
         _check(params, "params", torch.float32, (self.P,), dev)
         value = torch.empty((self.Nl,), dtype=torch.float32, device=dev)
+        norm = _norm_arg(obs_norm, self.obs_dim, dev)
         with torch.cuda.device(dev):
-            _lib.check(self.lib.minppo_policy_step(
-                self._h, _ptr(params), _ptr(obs), None, None, None, None, _ptr(value), None,
+            _lib.check(self.lib.minppo_policy_step_normalized(
+                self._h, _ptr(params), _ptr(obs), None, None, None, None, _ptr(value), None, norm,
                 _lib.POLICY_WEIGHTS_CURRENT if weights_current else 0, _stream_ptr(dev)))
         return value
 

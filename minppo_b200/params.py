@@ -5,12 +5,16 @@ The reference pickles the flax variable dict ``{'params': {'MLP_0': {'Dense_i': 
 SURVEY.md section 5).  The C ABI sees the same tree flattened in JAX's sorted-key order into
 one contiguous arena (include/minppo_b200.h, minppo_param_layout).  Leaves are NumPy arrays
 here (the reference's are jax.Array; unpickling those needs JAX).
+
+A checkpoint of a policy trained with observation normalization carries the statistics as an optional sibling of
+"params": ``{"params": ..., "obs_normalizer": {"mean", "var", "count", "eps", "clip"}}``
+(minppo_b200.obs_norm.ObsNormalizer.to_tree); everything that reads "params" ignores it.
 """
 from __future__ import annotations
 
 import os
 import pickle
-from typing import Dict, List, Tuple
+from typing import Dict, List, Optional, Tuple
 
 import numpy as np
 
@@ -70,10 +74,20 @@ def unflatten_params(flat: np.ndarray, obs_dim: int, act_dim: int, hidden: int, 
     return tree
 
 
-def save_model(params: Dict, filename: str) -> None:
+OBS_NORMALIZER_KEY = "obs_normalizer"
+OBS_NORMALIZER_FIELDS = ("mean", "var", "count", "eps", "clip")
+
+
+def save_model(params: Dict, filename: str, obs_normalizer: Optional[Dict] = None) -> None:
     """Same pickle as train.py:86-89.  The reference calls os.makedirs(os.path.dirname(f)),
     which raises for a bare filename such as the default 'trained_model.pkl' (SURVEY.md
-    section 5); the empty dirname is guarded here."""
+    section 5); the empty dirname is guarded here.  ``obs_normalizer``: the observation statistics
+    (ObsNormalizer.to_tree()), stored beside "params"."""
+    if obs_normalizer is not None:
+        missing = [k for k in OBS_NORMALIZER_FIELDS if k not in obs_normalizer]
+        if missing:
+            raise ValueError(f"obs_normalizer lacks {missing}")
+        params = {**params, OBS_NORMALIZER_KEY: {k: obs_normalizer[k] for k in OBS_NORMALIZER_FIELDS}}
     d = os.path.dirname(filename)
     if d:
         os.makedirs(d, exist_ok=True)
